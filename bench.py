@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py — audio frames/s of the Pocket-TTS per-frame generation path on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--batch 256] [--kv-len 1500]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--batch 256] [--kv-len 1500] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one batch: FlowLM step -> EOS rule -> LSD head -> Mimi -> 1920 samples, for every
 utterance of the batch (BASELINE.json configs[3]: batch 256, ~40-word paragraphs, KV length ~1.5k; voice prefix padded so the
@@ -23,6 +23,8 @@ no collective on the hot path; NCCL gathers per-rank counts/timings only. Prints
   sustained    >= 2 s of back-to-back steps of the primary mode with the clock record
   cpu_baseline the oracle (CPU restatement of the reference's ggml path) on this box's host cores, bounded samples
   --impl reference : the reference arm on the host cores (oracle/_ref when it was built, else the oracle port)
+  --dump-outputs DIR : after the timed steps, what their last step computed for the primary mode's utterances (the arrays b200_step
+               returns to its caller) as DIR/<name>.npy, so that two builds can be compared output for output (same arguments = same inputs)
 """
 from __future__ import annotations
 
@@ -301,6 +303,8 @@ def run_mode(env: Env, name: str, share: int, kv_f32: int, n_voices: int = 1, pr
     out["value"] = B * env.world * args.steps / (ms_max * 1e-3)
     Lm = L0 + mid_step
     out["kv_len"] = int(Lm.mean())
+    if primary and args.dump_outputs:
+        dump_outputs(args.dump_outputs, eng, B, env.rank, env.world)
 
     # ---- end-to-end through the public C-ABI calls with host buffers ----
     if primary and not args.no_e2e:
@@ -402,6 +406,33 @@ def run_mode(env: Env, name: str, share: int, kv_f32: int, n_voices: int = 1, pr
                             "ms_per_step": round(sus_ms / n_steps, 4), "kv_len_range": [int(L0.max()), int(L0.max()) + chunk], "clocks": s2.stop()}
     ctx.close()
     return out
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir: str, eng, n: int, rank: int, world: int):
+    """Writes what the last timed step computed for slots [0, n) of this rank: the arrays b200_step returns to its caller (PCM frame,
+    produced flag, latent, EOS logit), read back from the engine's output buffers, as float32 .npy files. Above DUMP_BYTES in all, a
+    fixed seeded sample of the slots is written; slots.npy lists which. With world > 1 each rank writes <name>_rank<r>.npy."""
+    import ptts_b200 as P
+    import torch
+    row_bytes = 4 * (P.FRAME + P.LDIM + 2)
+    rows = max(1, min(n, DUMP_BYTES // (row_bytes * world)))
+    slots = np.arange(n) if rows == n else np.sort(np.random.default_rng(0).choice(n, rows, replace=False))
+    ptr = P.lib().b200_device_ptr(eng.h, b"produced")
+
+    class _Produced:                                   # b200_debug_read_f32 reads f32 buffers only: the int32 flags go through torch
+        __cuda_array_interface__ = {"shape": (n,), "typestr": "<i4", "data": (ptr, False), "strides": None, "version": 3}
+    out = {"pcm": eng.debug_read("pcm", 0, n * P.FRAME).reshape(n, P.FRAME),
+           "produced": torch.as_tensor(_Produced(), device="cuda").cpu().numpy().astype(np.float32),
+           "latents": eng.debug_read("latent", 0, n * P.LDIM).reshape(n, P.LDIM),
+           "eos_logit": eng.debug_read("eos", 0, n)}
+    os.makedirs(out_dir, exist_ok=True)
+    suffix = f"_rank{rank}" if world > 1 else ""
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + suffix + ".npy"), np.ascontiguousarray(a[slots], np.float32))
+    np.save(os.path.join(out_dir, "slots" + suffix + ".npy"), slots.astype(np.float64))
 
 
 def verify_against_oracle(args, ctx, model_dir, texts, toks, voice, frames: int = 4):
@@ -527,7 +558,10 @@ def main():
     ap.add_argument("--no-verify", action="store_true")
     ap.add_argument("--only-ragged", action="store_true", help="development: run only the continuous-batching workload")
     ap.add_argument("--verify", action="store_true", help="run the oracle check of the timed context even with --no-extras")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None, help="write what the last timed step computed as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     if args.no_extras:
         args.sustain_s = 0.0
@@ -536,6 +570,9 @@ def main():
     # tokens of a 40-word paragraph ~ 60-75; voice prefix sized so that voice + text + steps/2 ~ kv_len
     args.untimed = max(args.warmup, 100)             # extended warm-up: also gives the clock sampler a loaded window
     args.t_voice = max(16, args.kv_len - 45 - args.untimed - args.steps // 2)
+    # the primary mode runs untimed + timed + e2e (steps + 7) + profiled (steps) steps without a rewind: the cache must hold all of them
+    # behind the voice prefix and the paragraph (< 256 tokens), or utterances reach their cap and a long --steps run times finished slots
+    args.kv_capacity = max(args.kv_capacity, args.t_voice + 256 + args.untimed + 3 * args.steps + 8)
 
     if args.impl == "reference":
         if rank != 0:
@@ -560,8 +597,8 @@ def main():
         dist.init_process_group("nccl", device_id=torch.device("cuda", local))
     import ptts_b200 as P
     from make_assets import default_model_dir, VOICES
-    if rank == 0:                                     # build + synthesise the model directories once, the other ranks wait
-        P.build()
+    if rank == 0:                                     # load the library build() made + synthesise the model directories once, the other ranks wait
+        P.lib()                                       # raises when it has not been built: the benchmark never compiles into the tree
         default_model_dir(eos_mode="never", t_voice=args.t_voice, voices=["cosette"])
         if not args.no_extras:
             default_model_dir(eos_mode="never", t_voice=args.t_voice, voices=VOICES)

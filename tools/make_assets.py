@@ -22,6 +22,7 @@ import os
 import shutil
 import struct
 import sys
+import tempfile
 
 import numpy as np
 
@@ -313,7 +314,8 @@ def make_model_dir(out_dir: str, seed: int = 1234, dtype: str = "BF16", eos_mode
 
 
 def default_model_dir(eos_mode: str = "never", dtype: str = "BF16", t_voice: int = 125, seed: int = 1234, voices=None) -> str:
-    root = os.environ.get("PTTS_B200_ASSETS", "/tmp/ptts_b200_assets")
+    # a cache outside the tree (which may be read-only), one per user: another user's directory on a shared machine is not writable
+    root = os.environ.get("PTTS_B200_ASSETS") or os.path.join(tempfile.gettempdir(), f"ptts_b200_assets_{os.getuid()}")
     name = f"model_s{seed}_{dtype.lower()}_{eos_mode + ('7' if eos_mode == 'late' else '')}_v{t_voice}" + ("" if voices is None else "_" + "-".join(voices))
     return make_model_dir(os.path.join(root, name), seed=seed, dtype=dtype, eos_mode=eos_mode, t_voice=t_voice, voices=voices)
 
