@@ -144,6 +144,33 @@ B200_API int  b200_debug_taps(b200_engine* e, int on);
 B200_API int  b200_debug_tap(b200_engine* e, const char* name, int slot, float* out, int max_elems);
 /* Host-only: tile width (32/64/128) and deterministic split-K factor the GEMM dispatcher would use (cost model of gemm_tc.cuh). */
 B200_API int  b200_debug_gemm_plan(int R, int N, int K, int num_sms, int want_ln, int* bn, int* splits);
+/* Unit-test hooks for the FlowLM attention (tests/test_gpu_attention.py). b200_debug_write_kv writes physical cache rows [pos0, pos0+n)
+ * of a slot from f32 rows [n][1024] (no prefix redirection; rounded to the cache type): the counterpart of b200_read_kv.
+ * b200_debug_set_prefix makes keys [0, pfx_len) of `slot` the rows of `pfx_slot` (0 rows = private cache). */
+B200_API int  b200_debug_write_kv(b200_engine* e, int slot, int layer, int which, int pos0, int n, const float* rows);
+B200_API int  b200_debug_set_prefix(b200_engine* e, int slot, int pfx_slot, int pfx_len);
+/* Per-call overrides of the attention switches; a negative field keeps the engine's value. */
+typedef struct b200_attn_opts {
+    int stream_splits;    /* KV splits of the streaming kernel, 1..16 (0 = automatic; PTTS_B200_AF_SPLITS)          */
+    int tile_prec;        /* operand precision of the decode-side prefix tiles, 0..2 (PTTS_B200_TILE_PREC)           */
+    int prefill_prec;     /* operand precision of the prefill tiles, 0..2 (PTTS_B200_PREFILL_PREC)                   */
+    int fork_tiles;       /* 1 = prefix tiles on a forked stream + merge (PTTS_B200_FORK_TILES)                      */
+    int counted_merge;    /* 1 = last-arriving CTA merges instead of attn_merge_kernel (PTTS_B200_COUNTED_MERGE)     */
+    int tile_min_rows;    /* fewest decode rows that use the prefix tiles (PTTS_B200_TILE_MIN_ROWS)                  */
+} b200_attn_opts;
+/* Runs the attention dispatch of one FlowLM layer eagerly over q [n][1024] f32 and the keys in the cache; out [n][1024] = the bf16
+ * output as f32 (NaN where nothing was written). prefill = 0: row r is slot slot0 + r at position rows_pos[r] (negative = dead row).
+ * prefill = 1: rows (rows_slot[r], rows_pos[r]) slot-major with ascending positions, chunked by max_prefill_rows like a prefill.
+ * Returns the number of tile work items (decode: 1 if the shared-prefix tiles ran, else 0), or a negative error. */
+B200_API int  b200_debug_attention(b200_engine* e, int layer, int prefill, int slot0, int n, const int32_t* rows_slot, const int32_t* rows_pos,
+                                   const float* q, const b200_attn_opts* opts, float* out);
+/* Host-only: the attention work lists. prefill = 0: prefix tiles of decode rows [0, n) whose prefix is (pfx_slot[r], pfx_len[r]) on
+ * num_sms SMs; aux_out[n] receives the tile row list; returns the prefix split count (0: no tiles) or B200_ECAPACITY beyond the work-list
+ * capacity of n slots and max_voices prefixes. prefill = 1: tile items of rows (row_slot[r], row_pos[r]) in chunks of chunk_rows,
+ * pfx_slot / pfx_len indexed by slot; aux_out[chunks + 1] receives the first item of each chunk; returns the chunk count.
+ * items_out[cap][9] = {row0, nrows, a_slot, a_k0, a_k1, b_slot, b_k0, b_k1, out_split}; *n_items = the item count. */
+B200_API int  b200_debug_attn_plan(int prefill, int n, const int32_t* row_slot, const int32_t* row_pos, const int32_t* pfx_slot, const int32_t* pfx_len,
+                                   int num_sms, int chunk_rows, int max_voices, int32_t* items_out, int cap, int32_t* aux_out, int* n_items);
 B200_API const char* b200_build_info(void);
 
 /* ---- extern "C" aliases of the reference's C++ API (include/pocket_tts/pocket_tts.h:18-42) ---- */

@@ -26,6 +26,18 @@ class B200Config(ctypes.Structure):
                 ("prefix_share", ctypes.c_int)]
 
 
+class AttnOpts(ctypes.Structure):
+    """b200_attn_opts: per-call overrides of the attention switches (negative = keep the engine's value)."""
+    _fields_ = [(k, ctypes.c_int) for k in ("stream_splits", "tile_prec", "prefill_prec", "fork_tiles", "counted_merge", "tile_min_rows")]
+
+    def __init__(self, **kw):
+        super().__init__(*([-1] * len(self._fields_)))
+        for k, v in kw.items():
+            if not hasattr(self, k):
+                raise AttributeError(k)
+            setattr(self, k, int(v))
+
+
 class BatchStats(ctypes.Structure):
     _fields_ = [("steps", ctypes.c_longlong), ("frames", ctypes.c_longlong), ("slot_steps", ctypes.c_longlong), ("sentences", ctypes.c_longlong),
                 ("refills", ctypes.c_longlong), ("wall_ms", ctypes.c_double), ("begin_ms", ctypes.c_double), ("submit_ms", ctypes.c_double), ("collect_ms", ctypes.c_double)]
@@ -88,6 +100,10 @@ def lib():
         "b200_device_ptr": (vp, [vp, cp]),
         "b200_launch_count": (ctypes.c_longlong, [vp]),
         "b200_read_kv": (ci, [vp, ci, ci, ci, ci, fp]),
+        "b200_debug_write_kv": (ci, [vp, ci, ci, ci, ci, ci, fp]),
+        "b200_debug_set_prefix": (ci, [vp, ci, ci, ci]),
+        "b200_debug_attention": (ci, [vp, ci, ci, ci, ci, ip, ip, fp, ctypes.POINTER(AttnOpts), fp]),
+        "b200_debug_attn_plan": (ci, [ci, ci, ip, ip, ip, ip, ci, ci, ci, ip, ci, ip, ctypes.POINTER(ctypes.c_int)]),
         "b200_build_info": (cp, []),
         "b200_debug_taps": (ci, [vp, ci]),
         "b200_debug_tap": (ci, [vp, cp, ci, fp, ci]),
@@ -329,6 +345,51 @@ class Engine:
         out = np.zeros((n_pos, 1024), np.float32)
         assert self.L.b200_read_kv(self.h, slot, layer, which, n_pos, _fp(out)) == 0
         return out
+
+    def debug_write_kv(self, slot, layer, which, pos0, rows):
+        rows = np.ascontiguousarray(rows, np.float32).reshape(-1, 1024)
+        rc = self.L.b200_debug_write_kv(self.h, slot, layer, which, pos0, rows.shape[0], _fp(rows))
+        if rc != 0:
+            raise RuntimeError(f"b200_debug_write_kv failed: {rc}")
+
+    def debug_set_prefix(self, slot, pfx_slot, pfx_len):
+        rc = self.L.b200_debug_set_prefix(self.h, slot, pfx_slot, pfx_len)
+        if rc != 0:
+            raise RuntimeError(f"b200_debug_set_prefix failed: {rc}")
+
+    def debug_attention(self, layer, q, rows_pos, slot0=0, rows_slot=None, prefill=False, **opts):
+        """One layer's attention dispatch over q [n][1024]; returns (out [n][1024] f32, tile work items)."""
+        q = np.ascontiguousarray(q, np.float32).reshape(-1, 1024)
+        n = q.shape[0]
+        pos = np.ascontiguousarray(rows_pos, np.int32)
+        rs = None if rows_slot is None else np.ascontiguousarray(rows_slot, np.int32)
+        assert pos.shape == (n,) and (rs is None or rs.shape == (n,))
+        out = np.zeros((n, 1024), np.float32)
+        o = AttnOpts(**opts)
+        rc = self.L.b200_debug_attention(self.h, layer, 1 if prefill else 0, slot0, n, _ip(rs) if rs is not None else None, _ip(pos), _fp(q),
+                                         ctypes.byref(o), _fp(out))
+        if rc < 0:
+            raise RuntimeError(f"b200_debug_attention failed: {rc}")
+        return out, rc
+
+
+def attn_plan(prefill, pfx_slot, pfx_len, row_slot=None, row_pos=None, num_sms=148, chunk_rows=4096, max_voices=8):
+    """Host-only work lists of the FlowLM attention (b200_debug_attn_plan): (return value, items [k][9], aux)."""
+    ps = np.ascontiguousarray(pfx_slot, np.int32); pl = np.ascontiguousarray(pfx_len, np.int32)
+    rs = None if row_slot is None else np.ascontiguousarray(row_slot, np.int32)
+    rp = None if row_pos is None else np.ascontiguousarray(row_pos, np.int32)
+    n = len(rs) if prefill else len(ps)
+    nk = ctypes.c_int()
+    cap = 64
+    while True:
+        items = np.zeros((cap, 9), np.int32)
+        aux = np.zeros(n + 2, np.int32)
+        rc = lib().b200_debug_attn_plan(1 if prefill else 0, n, _ip(rs) if rs is not None else None, _ip(rp) if rp is not None else None,
+                                        _ip(ps), _ip(pl), num_sms, chunk_rows, max_voices, _ip(items), cap, _ip(aux), ctypes.byref(nk))
+        if nk.value <= cap:
+            break
+        cap = nk.value
+    return rc, items[:nk.value], (aux[:rc + 1] if prefill and rc >= 0 else aux[:n])
 
 
 class Context:

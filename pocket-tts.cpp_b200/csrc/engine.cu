@@ -38,6 +38,62 @@ inline float h_silu(float x) { return x / (1.0f + expf(-x)); }
 struct LinW { __nv_bfloat16* w = nullptr; __nv_bfloat16* wk = nullptr; float* b = nullptr; int out = 0, in = 0; };
 struct ConvW { __half* w = nullptr; __half* wk = nullptr; float* b = nullptr; int N = 0, K = 0; };
 
+// Decode-side work list of attn_tile_kernel for rows [0, n) whose shared prefix is (row_pfx_slot[r], row_pfx_len[r]) (0 rows: none): rows
+// grouped by prefix, 64-row tiles, every prefix cut into `splits` key ranges so that tiles x splits x 16 heads fill the machine about twice.
+// The longest prefix sets `splits`; a shorter one can end before its last ranges, whose items are empty (a_k0 == a_k1) and write m = -inf,
+// l = 0 partials that the merges skip. Returns splits (0: no row has a prefix); rows receives the tile rows, items reference them.
+int plan_prefix_tiles(const int* row_pfx_slot, const int* row_pfx_len, int n, int sms, std::vector<AtItem>& items, std::vector<int>& rows) {
+    items.clear(); rows.clear();
+    std::map<std::pair<int, int>, std::vector<int>> groups;
+    for (int r = 0; r < n; r++) if (row_pfx_len[r] > 0) groups[{row_pfx_slot[r], row_pfx_len[r]}].push_back(r);
+    int tiles = 0, max_p = 0;
+    for (auto& g : groups) { tiles += ((int)g.second.size() + AT_ROWS - 1) / AT_ROWS; max_p = std::max(max_p, g.first.second); }
+    if (tiles == 0) return 0;
+    // ONE wave of tile CTAs (tiles x splits x 16 heads <= two resident CTAs per SM): a second, partly filled wave would cost a whole CTA time
+    int splits = std::min(AF_PFX_SPLITS, std::max(1, (2 * sms) / (N_HEADS * tiles)));
+    splits = std::max(1, std::min(splits, max_p / AT_KEYS));
+    for (auto& g : groups) {
+        const int plen = g.first.second;
+        int chunk = (plen + splits - 1) / splits; chunk = (chunk + AT_KEYS - 1) / AT_KEYS * AT_KEYS;
+        for (size_t i0 = 0; i0 < g.second.size(); i0 += AT_ROWS) {
+            const int nr = (int)std::min<size_t>(AT_ROWS, g.second.size() - i0);
+            for (int sp = 0; sp < splits; sp++) {
+                AtItem it{}; it.row0 = (int)(rows.size()); it.nrows = nr; it.a_slot = g.first.first; it.a_k0 = std::min(plen, sp * chunk); it.a_k1 = std::min(plen, (sp + 1) * chunk);
+                it.b_slot = 0; it.b_k0 = 0; it.b_k1 = 0; it.out_split = AF_MAX_SPLITS + sp;
+                items.push_back(it);
+            }
+            for (int i = 0; i < nr; i++) rows.push_back(g.second[i0 + i]);
+        }
+    }
+    return splits;
+}
+// Capacity of that list for max_slots rows of at most max_voices distinct prefixes.
+int prefix_tiles_capacity(int max_slots, int max_voices) { return ((max_slots + AT_ROWS - 1) / AT_ROWS + max_voices + 1) * AF_PFX_SPLITS + 8; }
+
+// Prefill work list of attn_tile_kernel (bf16 cache): the rows (slot-major, ascending positions) are cut into chunks of chunk_rows; inside a
+// chunk, one item per run of <= 64 consecutive positions of one slot, with keys [0, P) of the slot's prefix slot and its own rows [P, last
+// position of the run]. pfx_slot / pfx_len are indexed by slot. chunk_item0[c] = first item of chunk c (nchunks + 1 entries).
+void plan_prefill_items(const int* slots, const int* pos, int total, int chunk_rows, const int* pfx_slot, const int* pfx_len,
+                        std::vector<AtItem>& items, std::vector<int>& chunk_item0) {
+    const int nchunks = (total + chunk_rows - 1) / chunk_rows;
+    items.clear(); chunk_item0.assign(nchunks + 1, 0);
+    for (int c = 0; c < nchunks; c++) {
+        const int r0 = c * chunk_rows, R = std::min(chunk_rows, total - r0);
+        chunk_item0[c] = (int)items.size();
+        for (int i = 0; i < R;) {
+            int j = i + 1;
+            while (j < R && j - i < AT_ROWS && slots[r0 + j] == slots[r0 + i] && pos[r0 + j] == pos[r0 + j - 1] + 1) j++;
+            const int slot = slots[r0 + i], P = pfx_len[slot];
+            AtItem it{}; it.row0 = i; it.nrows = j - i; it.out_split = -1;
+            it.a_slot = pfx_slot[slot]; it.a_k0 = 0; it.a_k1 = P;                                  // shared prefix rows (none: P = 0)
+            it.b_slot = slot; it.b_k0 = P; it.b_k1 = pos[r0 + j - 1] + 1;                            // own rows, causal
+            items.push_back(it);
+            i = j;
+        }
+    }
+    chunk_item0[nchunks] = (int)items.size();
+}
+
 }  // namespace
 
 struct b200_engine {
@@ -343,36 +399,15 @@ struct b200_engine {
     }
 
     // Decode rows of the range [slot0, slot0+n): row r = slot slot0+r. With a shared voice prefix, (re)builds the work list of
-    // attn_tile_kernel on the host when the range or the slot -> voice assignment changed: rows grouped by voice, 64-row tiles, the
-    // prefix cut into `splits` key ranges so that tiles x splits x 16 heads fill the machine about twice. Stream-ordered upload.
+    // attn_tile_kernel (plan_prefix_tiles) on the host when the range or the slot -> voice assignment changed. Stream-ordered upload.
     void prepare_decode(int slot0, int n) {
         actx = AttnCtx{}; actx.row_slot = row_slot; actx.row_pos = row_pos; actx.cs = cs;
         if (!cfg.prefix_share || cfg.kv_f32 || n < tile_min_rows) { dec_grid_items = 0; dec_key_n = -1; return; }
         if (dec_key_slot0 == slot0 && dec_key_n == n && dec_key_version == pfx_version) return;
         dec_key_slot0 = slot0; dec_key_n = n; dec_key_version = pfx_version;
-        std::map<std::pair<int, int>, std::vector<int>> groups;
-        for (int r = 0; r < n; r++) if (h_pfx_len[slot0 + r] > 0) groups[{h_pfx_slot[slot0 + r], h_pfx_len[slot0 + r]}].push_back(r);
-        int tiles = 0, max_p = 0;
-        for (auto& g : groups) { tiles += ((int)g.second.size() + AT_ROWS - 1) / AT_ROWS; max_p = std::max(max_p, g.first.second); }
-        if (tiles == 0) { dec_grid_items = 0; return; }
-        // ONE wave of tile CTAs (tiles x splits x 16 heads <= two resident CTAs per SM): a second, partly filled wave would cost a whole CTA time
-        const int sms = tc ? tc->num_sms : 148;
-        int splits = std::min(AF_PFX_SPLITS, std::max(1, (2 * sms) / (N_HEADS * tiles)));
-        splits = std::max(1, std::min(splits, max_p / AT_KEYS));
         std::vector<AtItem> items; std::vector<int> rows;
-        for (auto& g : groups) {
-            const int plen = g.first.second;
-            int chunk = (plen + splits - 1) / splits; chunk = (chunk + AT_KEYS - 1) / AT_KEYS * AT_KEYS;
-            for (size_t i0 = 0; i0 < g.second.size(); i0 += AT_ROWS) {
-                const int nr = (int)std::min<size_t>(AT_ROWS, g.second.size() - i0);
-                for (int sp = 0; sp < splits; sp++) {
-                    AtItem it{}; it.row0 = (int)(rows.size()); it.nrows = nr; it.a_slot = g.first.first; it.a_k0 = std::min(plen, sp * chunk); it.a_k1 = std::min(plen, (sp + 1) * chunk);
-                    it.b_slot = 0; it.b_k0 = 0; it.b_k1 = 0; it.out_split = AF_MAX_SPLITS + sp;
-                    items.push_back(it);
-                }
-                for (int i = 0; i < nr; i++) rows.push_back(g.second[i0 + i]);
-            }
-        }
+        const int splits = plan_prefix_tiles(h_pfx_slot.data() + slot0, h_pfx_len.data() + slot0, n, tc ? tc->num_sms : 148, items, rows);
+        if (splits == 0) { dec_grid_items = 0; return; }
         if ((int)items.size() > dec_items_cap) { fprintf(stderr, "ptts_b200: internal error: %zu prefix tiles exceed the work-list capacity %d\n", items.size(), dec_items_cap); abort(); }
         dec_grid_items = ((int)items.size() + 7) / 8 * 8;
         const size_t bytes = 4 * sizeof(int) + rows.size() * sizeof(int) + items.size() * sizeof(AtItem);
@@ -410,17 +445,34 @@ struct b200_engine {
         else if (prec == 1) launch_k(pdl, attn_tile_kernel<1>, grid, dim3(128), (size_t)0, st, a...);
         else launch_k(pdl, attn_tile_kernel<0>, grid, dim3(128), (size_t)0, st, a...);
     }
+    // prefill chunk c (its rows start at row r0 of the `total` rows staged in pf_int; items from chunk_item0) becomes the attention context
+    void prefill_chunk(int c, int r0, int total, const std::vector<int>& chunk_item0) {
+        actx = AttnCtx{};
+        actx.row_slot = pf_int + r0; actx.row_pos = pf_int + total + r0; actx.cs = cs; actx.prefill = true;
+        actx.items = pf_items + chunk_item0[c]; actx.meta = pf_meta + 4 * c; actx.n_items = chunk_item0[c + 1] - chunk_item0[c];
+    }
     bool use_prefix_tiles(int R) const { return cfg.prefix_share && !cfg.kv_f32 && !actx.prefill && R >= tile_min_rows && dec_grid_items > 0; }
 
     // in_proj (+RoPE, KV append) and attention of layer l. Expects norm1 of layer l in n_bf; rows are described by `actx`.
-    void flow_attn_part(int l, int R) {
-        auto& L = fl[l];
+    void flow_attn_part(int l, int R) { flow_qkv(l, R); flow_attn(l, R); }
+    Epi qkv_epi(int l) const {
         Epi e; e.mode = EPI_FLOW_QKV; e.row_slot = actx.row_slot; e.row_pos = actx.row_pos; e.cs = actx.cs; e.kv_f32 = cfg.kv_f32;
         e.kv_slot_stride = kv_slot_stride; e.q_out_f32 = q;
         if (cfg.kv_f32) { e.kcache = (float*)kc + l * kv_layer_stride; e.vcache = (float*)vc + l * kv_layer_stride; }
         else { e.kcache = (__nv_bfloat16*)kc + l * kv_layer_stride; e.vcache = (__nv_bfloat16*)vc + l * kv_layer_stride; }
+        return e;
+    }
+    // in_proj of layer l: q -> `q` (f32), K/V rows appended to the cache at (row_slot, row_pos)
+    void flow_qkv(int l, int R) {
+        auto& L = fl[l];
+        const Epi e = qkv_epi(l);
         if (l > 0 && ln_in_gemv(R)) { LnArgs a; a.w = L.n1w; a.b = L.n1b; a.eps = 1e-5f; lin_ln(h, a, L.in_proj, R, e); }   // layer 0: flow_in_kernel wrote n_bf
         else lin(n_bf, L.in_proj, R, e);
+    }
+    // attention of layer l over the rows of `actx` (q in `q`, keys in the cache) -> att_bf: picks the kernels (prefill tiles, shared-prefix
+    // tiles beside the streaming kernel, streaming alone) and the merge, and launches them
+    void flow_attn(int l, int R) {
+        const Epi e = qkv_epi(l);
         int sg = -1;
         const bool pdl_saved = pdl_active;
         set_pdl(pdl_small);                                  // the KV-streaming kernel fills the machine: no early dependents around it
@@ -1178,7 +1230,7 @@ int b200_finalize_weights(b200_engine* e) {
     e->ff_bf = e->dalloc<__nv_bfloat16>((size_t)MR * D_FF);
     e->af_ml = e->dalloc<float>((size_t)MR * AF_WS_STRIDE * 32); e->af_acc = e->dalloc<float>((size_t)MR * AF_WS_STRIDE * D_MODEL); e->af_cnt = e->dalloc<int>(MR); e->af_cnt2 = e->dalloc<int>((size_t)MR * N_HEADS);
     e->pfx_slot = e->dalloc<int>(TS); e->pfx_len = e->dalloc<int>(TS);
-    e->dec_items_cap = ((S + AT_ROWS - 1) / AT_ROWS + e->cfg.max_voices + 1) * AF_PFX_SPLITS + 8;
+    e->dec_items_cap = prefix_tiles_capacity(S, e->cfg.max_voices);
     e->dec_items = e->dalloc<AtItem>(e->dec_items_cap); e->dec_meta = e->dalloc<int>(4); e->dec_rows = e->dalloc<int>(S);
     e->pf_barrier = e->dalloc<unsigned int>(4);
     e->tap_up = e->dalloc<float>((size_t)S * M_T * M_DIM);
@@ -1251,23 +1303,7 @@ static void prefill_rows(b200_engine* e, const std::vector<int>& slots, const st
     const int nchunks = (total + MRp - 1) / MRp;
     // tensor-core tile work list (bf16 cache): one item per run of <= 64 consecutive positions of one slot inside a chunk
     std::vector<AtItem> items; std::vector<int> chunk_item0(nchunks + 1, 0);
-    if (!e->cfg.kv_f32) {
-        for (int c = 0; c < nchunks; c++) {
-            const int r0 = c * MRp, R = std::min(MRp, total - r0);
-            chunk_item0[c] = (int)items.size();
-            for (int i = 0; i < R;) {
-                int j = i + 1;
-                while (j < R && j - i < AT_ROWS && slots[r0 + j] == slots[r0 + i] && pos[r0 + j] == pos[r0 + j - 1] + 1) j++;
-                const int slot = slots[r0 + i], P = e->h_pfx_len[slot];
-                AtItem it{}; it.row0 = i; it.nrows = j - i; it.out_split = -1;
-                it.a_slot = e->h_pfx_slot[slot]; it.a_k0 = 0; it.a_k1 = P;                              // shared prefix rows (none: P = 0)
-                it.b_slot = slot; it.b_k0 = P; it.b_k1 = pos[r0 + j - 1] + 1;                            // own rows, causal
-                items.push_back(it);
-                i = j;
-            }
-        }
-        chunk_item0[nchunks] = (int)items.size();
-    }
+    if (!e->cfg.kv_f32) plan_prefill_items(slots.data(), pos.data(), total, MRp, e->h_pfx_slot.data(), e->h_pfx_len.data(), items, chunk_item0);
     e->grow(e->pf_int, e->pf_int_cap, (size_t)3 * total);
     e->grow(e->pf_items, e->pf_items_cap, items.size() + 1);
     e->grow(e->pf_meta, e->pf_meta_cap, (size_t)4 * nchunks);
@@ -1293,9 +1329,7 @@ static void prefill_rows(b200_engine* e, const std::vector<int>& slots, const st
     const b200_engine::AttnCtx saved = e->actx;
     for (int c = 0; c < nchunks; c++) {
         const int r0 = c * MRp, R = std::min(MRp, total - r0);
-        e->actx = b200_engine::AttnCtx{};
-        e->actx.row_slot = e->pf_int + r0; e->actx.row_pos = e->pf_int + total + r0; e->actx.cs = e->cs; e->actx.prefill = true;
-        e->actx.items = e->pf_items + chunk_item0[c]; e->actx.meta = e->pf_meta + 4 * c; e->actx.n_items = chunk_item0[c + 1] - chunk_item0[c];
+        e->prefill_chunk(c, r0, total, chunk_item0);
         if (tokens) {
             launch_k(false, embed_gather_kernel, dim3(R), dim3(256), (size_t)(0), e->stream, e->embed, (const int*)(e->pf_int + 2 * total + r0), e->h, R);
             e->launches++;
@@ -1726,6 +1760,121 @@ int b200_read_kv(b200_engine* e, int slot, int layer, int which, int n_pos, floa
     return B200_OK;
 }
 
+// Test hook: physical cache rows [pos0, pos0 + n) of a slot (no prefix redirection), from f32 rows [n][1024] rounded to the cache type.
+int b200_debug_write_kv(b200_engine* e, int slot, int layer, int which, int pos0, int n, const float* rows) {
+    if (!e || !e->finalized || !rows || slot < 0 || slot >= e->total_slots || layer < 0 || layer >= N_LAYERS || pos0 < 0 || n < 0 ||
+        pos0 + n > e->cfg.kv_capacity) return B200_EINVAL;
+    b200_sync(e);                                              // also selects the engine's device
+    const size_t cnt = (size_t)n * D_MODEL;
+    const long long off = layer * e->kv_layer_stride + slot * e->kv_slot_stride + (long long)pos0 * D_MODEL;
+    if (e->cfg.kv_f32) {
+        PTTS_CUDA_CHECK(cudaMemcpyAsync((float*)(which ? e->vc : e->kc) + off, rows, cnt * sizeof(float), cudaMemcpyHostToDevice, e->stream));
+    } else {
+        const std::vector<__nv_bfloat16> b = b200_engine::to_bf16(std::vector<float>(rows, rows + cnt));
+        PTTS_CUDA_CHECK(cudaMemcpyAsync((__nv_bfloat16*)(which ? e->vc : e->kc) + off, b.data(), cnt * sizeof(__nv_bfloat16), cudaMemcpyHostToDevice, e->stream));
+    }
+    PTTS_CUDA_CHECK(cudaStreamSynchronize(e->stream));
+    return B200_OK;
+}
+
+// Test hook: keys [0, pfx_len) of `slot` are rows of `pfx_slot` (what a sentence start of a voice sets up; 0 = private cache).
+int b200_debug_set_prefix(b200_engine* e, int slot, int pfx_slot, int pfx_len) {
+    if (!e || !e->finalized || slot < 0 || slot >= e->cfg.max_slots || pfx_slot < 0 || pfx_slot >= e->total_slots || pfx_len < 0 ||
+        pfx_len > e->cfg.kv_capacity) return B200_EINVAL;
+    b200_sync(e);                                              // also selects the engine's device
+    e->h_pfx_slot[slot] = pfx_slot; e->h_pfx_len[slot] = pfx_len; e->pfx_version++;
+    PTTS_CUDA_CHECK(cudaMemcpyAsync(e->pfx_slot + slot, &pfx_slot, sizeof(int), cudaMemcpyHostToDevice, e->stream));
+    PTTS_CUDA_CHECK(cudaMemcpyAsync(e->pfx_len + slot, &pfx_len, sizeof(int), cudaMemcpyHostToDevice, e->stream));
+    PTTS_CUDA_CHECK(cudaStreamSynchronize(e->stream));
+    return B200_OK;
+}
+
+// Test hook: the FlowLM attention dispatch of one layer (flow_attn: the kernels, splits and merge a step or a prefill would pick) over
+// caller-given rows and q, run eagerly, synchronised; out[n][1024] = att_bf widened to f32. Rows whose output is not written keep a NaN.
+// Every upload is ordered on the engine stream: a plain cudaMemcpy / cudaMemset runs on the legacy stream, which the engine's
+// non-blocking streams do not wait for.
+int b200_debug_attention(b200_engine* e, int layer, int prefill, int slot0, int n, const int32_t* rows_slot, const int32_t* rows_pos,
+                         const float* q, const b200_attn_opts* opts, float* out) {
+    if (!e || !e->finalized || layer < 0 || layer >= N_LAYERS || n < 1 || !rows_pos || !q || !out) return B200_EINVAL;
+    const int cap = e->cfg.kv_capacity;
+    if (prefill) {
+        if (!rows_slot) return B200_EINVAL;
+        for (int r = 0; r < n; r++)
+            if (rows_slot[r] < 0 || rows_slot[r] >= e->total_slots || rows_pos[r] < 0 || rows_pos[r] >= cap ||
+                (r > 0 && (rows_slot[r] < rows_slot[r - 1] || (rows_slot[r] == rows_slot[r - 1] && rows_pos[r] <= rows_pos[r - 1])))) return B200_EINVAL;
+    } else {
+        if (slot0 < 0 || slot0 + n > e->cfg.max_slots) return B200_EINVAL;
+        for (int r = 0; r < n; r++) if (rows_pos[r] >= cap) return B200_EINVAL;
+        // prefix assignments set through b200_debug_set_prefix can form more distinct prefixes than the work list holds (it is sized for
+        // max_voices of them): refuse those here, where prepare_decode would abort
+        std::vector<AtItem> items; std::vector<int> rows;
+        plan_prefix_tiles(e->h_pfx_slot.data() + slot0, e->h_pfx_len.data() + slot0, n, e->tc ? e->tc->num_sms : 148, items, rows);
+        if ((int)items.size() > e->dec_items_cap) return B200_ECAPACITY;
+    }
+    b200_sync(e);                                              // also selects the engine's device
+    const int s_splits = e->af_splits_override, s_tprec = e->tile_prec, s_pprec = e->prefill_prec, s_min = e->tile_min_rows;
+    const bool s_fork = e->fork_tiles, s_counted = e->counted_merge, s_pdl_small = e->pdl_small, s_pdl = e->pdl_active;
+    const int s_grid = e->dec_grid_items;
+    const b200_engine::AttnCtx s_actx = e->actx;
+    if (opts) {
+        if (opts->stream_splits >= 0) e->af_splits_override = opts->stream_splits;
+        if (opts->tile_prec >= 0) e->tile_prec = opts->tile_prec;
+        if (opts->prefill_prec >= 0) e->prefill_prec = opts->prefill_prec;
+        if (opts->fork_tiles >= 0) e->fork_tiles = opts->fork_tiles != 0;
+        if (opts->counted_merge >= 0) e->counted_merge = opts->counted_merge != 0;
+        if (opts->tile_min_rows >= 0) e->tile_min_rows = opts->tile_min_rows;
+    }
+    e->pdl_small = false; e->set_pdl(false);
+    auto read_out = [&](float* dst, int R) {
+        PTTS_CUDA_CHECK(cudaStreamSynchronize(e->stream));
+        PTTS_CUDA_CHECK(cudaGetLastError());
+        std::vector<uint16_t> tmp((size_t)R * D_MODEL);
+        PTTS_CUDA_CHECK(cudaMemcpy(tmp.data(), e->att_bf, tmp.size() * 2, cudaMemcpyDeviceToHost));
+        for (size_t i = 0; i < tmp.size(); i++) { const uint32_t u = (uint32_t)tmp[i] << 16; memcpy(&dst[i], &u, 4); }
+    };
+    int tiles = 0;
+    if (!prefill) {
+        std::vector<int> rs(n), rp(n);
+        for (int r = 0; r < n; r++) { rs[r] = rows_pos[r] < 0 ? -1 : slot0 + r; rp[r] = std::max(0, (int)rows_pos[r]); }   // negative position: dead row
+        PTTS_CUDA_CHECK(cudaMemcpyAsync(e->row_slot, rs.data(), n * sizeof(int), cudaMemcpyHostToDevice, e->stream));
+        PTTS_CUDA_CHECK(cudaMemcpyAsync(e->row_pos, rp.data(), n * sizeof(int), cudaMemcpyHostToDevice, e->stream));
+        PTTS_CUDA_CHECK(cudaMemcpyAsync(e->q, q, (size_t)n * D_MODEL * sizeof(float), cudaMemcpyHostToDevice, e->stream));
+        PTTS_CUDA_CHECK(cudaMemsetAsync(e->att_bf, 0xff, (size_t)n * D_MODEL * sizeof(__nv_bfloat16), e->stream));
+        e->dec_key_n = -1;                                     // plan the prefix tiles for this call's rows and options
+        e->prepare_decode(slot0, n);
+        tiles = e->use_prefix_tiles(n) ? 1 : 0;
+        e->flow_attn(layer, n);
+        read_out(out, n);
+    } else {
+        const int MRp = e->cfg.max_prefill_rows, nchunks = (n + MRp - 1) / MRp;
+        std::vector<AtItem> items; std::vector<int> chunk_item0(nchunks + 1, 0);
+        if (!e->cfg.kv_f32) plan_prefill_items(rows_slot, rows_pos, n, MRp, e->h_pfx_slot.data(), e->h_pfx_len.data(), items, chunk_item0);
+        e->grow(e->pf_int, e->pf_int_cap, (size_t)3 * n);
+        e->grow(e->pf_items, e->pf_items_cap, items.size() + 1);
+        e->grow(e->pf_meta, e->pf_meta_cap, (size_t)4 * nchunks);
+        std::vector<int> meta((size_t)4 * nchunks, 0);
+        for (int c = 0; c < nchunks; c++) meta[4 * c] = chunk_item0[c + 1] - chunk_item0[c];
+        PTTS_CUDA_CHECK(cudaMemcpyAsync(e->pf_int, rows_slot, n * sizeof(int), cudaMemcpyHostToDevice, e->stream));
+        PTTS_CUDA_CHECK(cudaMemcpyAsync(e->pf_int + n, rows_pos, n * sizeof(int), cudaMemcpyHostToDevice, e->stream));
+        PTTS_CUDA_CHECK(cudaMemcpyAsync(e->pf_meta, meta.data(), meta.size() * sizeof(int), cudaMemcpyHostToDevice, e->stream));
+        if (!items.empty()) PTTS_CUDA_CHECK(cudaMemcpyAsync(e->pf_items, items.data(), items.size() * sizeof(AtItem), cudaMemcpyHostToDevice, e->stream));
+        for (int c = 0; c < nchunks; c++) {
+            const int r0 = c * MRp, R = std::min(MRp, n - r0);
+            e->prefill_chunk(c, r0, n, chunk_item0);
+            PTTS_CUDA_CHECK(cudaMemcpyAsync(e->q, q + (size_t)r0 * D_MODEL, (size_t)R * D_MODEL * sizeof(float), cudaMemcpyHostToDevice, e->stream));
+            PTTS_CUDA_CHECK(cudaMemsetAsync(e->att_bf, 0xff, (size_t)R * D_MODEL * sizeof(__nv_bfloat16), e->stream));
+            e->flow_attn(layer, R);
+            read_out(out + (size_t)r0 * D_MODEL, R);
+        }
+        tiles = (int)items.size();
+    }
+    e->af_splits_override = s_splits; e->tile_prec = s_tprec; e->prefill_prec = s_pprec; e->tile_min_rows = s_min;
+    e->fork_tiles = s_fork; e->counted_merge = s_counted; e->pdl_small = s_pdl_small; e->set_pdl(s_pdl);
+    e->actx = s_actx; e->dec_grid_items = s_grid;
+    e->dec_key_n = -1;                                         // the device work list is this call's: the next step plans and uploads its own
+    return tiles;
+}
+
 // Tap points for localising a parity failure (the reference's GraphContext::debug, src/context.h:526-547). Names are the ones the CPU
 // restatement under tests uses: "flow.layer<l>" = residual stream after FlowLM layer l [1024], "flow.attn<l>" = attention output of layer l [1024]
 // (both need b200_debug_taps(e, 1) before the step), "mimi.upsample" [16][512], "mimi.transformer" [16][512], "seanet.conv0" [16][512],
@@ -1787,6 +1936,32 @@ int b200_debug_gemm_plan(int R, int N, int K, int num_sms, int want_ln, int* bn,
     const TcPlan p = tc_plan((R + 127) / 128, R, N, K, num_sms, want_ln != 0);
     *bn = p.bn; *splits = p.splits;
     return B200_OK;
+}
+
+// Host-only: the attention work lists the engine builds (plan_prefix_tiles / plan_prefill_items), for tests without a device.
+int b200_debug_attn_plan(int prefill, int n, const int32_t* row_slot, const int32_t* row_pos, const int32_t* pfx_slot, const int32_t* pfx_len,
+                         int num_sms, int chunk_rows, int max_voices, int32_t* items_out, int cap, int32_t* aux_out, int* n_items) {
+    if (n < 1 || !pfx_slot || !pfx_len || !items_out || !aux_out || !n_items || cap < 0) return B200_EINVAL;
+    std::vector<AtItem> items; std::vector<int> aux;
+    int ret;
+    if (prefill) {
+        if (!row_slot || !row_pos || chunk_rows < 1) return B200_EINVAL;
+        plan_prefill_items(row_slot, row_pos, n, chunk_rows, pfx_slot, pfx_len, items, aux);
+        ret = (int)aux.size() - 1;
+    } else {
+        if (num_sms < 1) return B200_EINVAL;
+        ret = plan_prefix_tiles(pfx_slot, pfx_len, n, num_sms, items, aux);
+        if ((int)items.size() > prefix_tiles_capacity(n, max_voices)) ret = B200_ECAPACITY;
+    }
+    *n_items = (int)items.size();
+    if ((int)items.size() > cap) return B200_ECAPACITY;
+    for (size_t i = 0; i < items.size(); i++) {
+        const AtItem& it = items[i];
+        const int v[9] = {it.row0, it.nrows, it.a_slot, it.a_k0, it.a_k1, it.b_slot, it.b_k0, it.b_k1, it.out_split};
+        memcpy(items_out + 9 * i, v, sizeof(v));
+    }
+    memcpy(aux_out, aux.data(), aux.size() * sizeof(int));
+    return ret;
 }
 
 const char* b200_build_info(void) { return "ptts_b200 sm_100a " __DATE__ " " __TIME__; }

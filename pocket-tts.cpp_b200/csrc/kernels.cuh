@@ -399,8 +399,9 @@ attn_flow_split_kernel(const float* __restrict__ q, const KV* __restrict__ kc, c
 //   prefill: the query rows are consecutive positions of one slot, keys = [shared prefix | own rows up to the row's position]
 //     (causal mask key <= shift + query, transformer.h:157-169). Output = normalised bf16 rows.
 // Precision: the reference computes attention in f32 on an f32 cache. K/V are bf16 here (cfg.kv_f32 = 0); q and the probabilities
-// would lose another 8 bits as single bf16 MMA operands, so both are fed as hi + lo bf16 pairs (two MMAs each, ~16 mantissa bits):
-// the tile kernel then agrees with the f32-FMA streaming kernel to ~1e-5 relative (tests/test_gpu_attention.py).
+// would lose another 8 bits as single bf16 MMA operands, so both are fed as hi + lo bf16 pairs (two MMAs each, ~16 mantissa bits).
+// Against a float64 reference (tests/test_gpu_attention.py, values of order 1) the bf16 output of PREC 2 is within one bf16 ulp plus an
+// absolute 9e-6, as close as the f32-FMA streaming kernel (1.3e-6); PREC 1 / 0 below need 2.3e-3 / 3.5e-2 beyond the ulp.
 // No ldmatrix: the contraction index (QK^T) and the output-dim index (PV) are permuted so that every shared-memory access is a
 // conflict-free LDS.128 (same fragment scheme as attn_mimi_mma4_kernel below):
 //   * QK^T: lane (g, t) loads K[key 8j+g][32p + 8t .. +7]; its 8 values are the k-slots of two k16 steps, Q fragments use the same order;

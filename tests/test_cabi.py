@@ -68,3 +68,75 @@ def test_gemm_planner_invariants(P):
                 if R > 512:
                     assert sp.value == 1                                       # large-M GEMMs are never split
     assert L.b200_debug_gemm_plan(0, 64, 64, 148, 0, ctypes.byref(bn), ctypes.byref(sp)) != 0
+
+
+def test_attention_work_list_invariants(P):
+    """The host-side work lists of the FlowLM attention (b200_debug_attn_plan runs the builders the engine uses; no GPU).
+    Decode: every live row with a prefix gets one item per prefix split, whose key ranges tile [0, P) exactly once (a voice shorter than
+    the longest one gets empty ranges), <= 64 rows of one prefix per item, the split count the merges read equals the items' splits.
+    Prefill: every row lies in exactly one item of its own chunk; an item is a run of consecutive positions of one slot with the keys
+    [0, P) of the prefix slot and [P, last position] of its own slot; a run only ends at a chunk edge, a new slot or after 64 rows."""
+    import numpy as np
+    AF_MAX_SPLITS, AF_PFX_SPLITS, AT_ROWS = 16, 8, 64
+    rng = np.random.default_rng(0)
+    for case in range(300):
+        n = int(rng.choice([1, 3, 4, 63, 64, 65, 128, 200, 256]))
+        nv = int(rng.integers(1, 9))
+        lens = [int(rng.choice([1, 7, 63, 64, 65, 125, 1345, int(rng.integers(1, 3000))])) for _ in range(nv)]
+        voice = rng.integers(-1, nv, n)                                          # -1: private cache
+        pfx_slot = np.array([1000 + v if v >= 0 else 0 for v in voice], np.int32)
+        pfx_len = np.array([lens[v] if v >= 0 else 0 for v in voice], np.int32)
+        sms = int(rng.choice([1, 16, 132, 148]))
+        splits, items, rows = P.attn_plan(False, pfx_slot, pfx_len, num_sms=sms, max_voices=8)
+        assert splits >= 0, (case, splits)
+        if (pfx_len == 0).all():
+            assert splits == 0 and len(items) == 0
+            continue
+        assert 1 <= splits <= AF_PFX_SPLITS
+        assert len(items) <= ((n + AT_ROWS - 1) // AT_ROWS + 8 + 1) * AF_PFX_SPLITS + 8          # the engine's work-list capacity
+        per_row = {}
+        for row0, nr, a_slot, a0, a1, b_slot, b0, b1, osp in items:
+            assert 1 <= nr <= AT_ROWS and b1 == b0 and AF_MAX_SPLITS <= osp < AF_MAX_SPLITS + splits
+            for r in rows[row0:row0 + nr]:
+                assert pfx_slot[r] == a_slot and 0 <= a0 <= a1 <= pfx_len[r]
+                per_row.setdefault(int(r), []).append((osp, a0, a1))
+        assert sorted(per_row) == [r for r in range(n) if pfx_len[r] > 0]
+        for r, its in per_row.items():
+            its.sort()
+            assert [o for o, _, _ in its] == list(range(AF_MAX_SPLITS, AF_MAX_SPLITS + splits)), (case, r)
+            edge = 0
+            for _, a0, a1 in its:
+                assert a0 == min(edge, pfx_len[r]) and a1 >= a0
+                edge = max(edge, a1)
+            assert edge == pfx_len[r]
+    for case in range(300):
+        n_slots = int(rng.integers(1, 6))
+        pfx_slot = np.zeros(n_slots, np.int32); pfx_len = np.zeros(n_slots, np.int32)
+        slots, pos = [], []
+        for s in range(n_slots):
+            P_ = int(rng.choice([0, 0, 1, 64, 125, 1345]))
+            pfx_slot[s] = 50 + s if P_ else 0; pfx_len[s] = P_
+            start = P_ + int(rng.choice([0, 0, 125, int(rng.integers(0, 100))]))
+            ln = int(rng.choice([1, 63, 64, 65, 130, int(rng.integers(1, 300))]))
+            p = list(range(start, start + ln))
+            if ln > 10 and rng.random() < 0.3:                                 # a gap: two runs of one slot
+                p = p[:ln // 2] + [x + 5 for x in p[ln // 2:]]
+            slots += [s] * ln; pos += p
+        total = len(slots)
+        chunk = int(rng.choice([1, 7, 64, 100, 4096]))
+        nch, items, first = P.attn_plan(True, pfx_slot, pfx_len, row_slot=slots, row_pos=pos, chunk_rows=chunk)
+        assert nch == -(-total // chunk) and len(first) == nch + 1 and first[0] == 0 and first[-1] == len(items)
+        for c in range(nch):
+            r0, R = c * chunk, min(chunk, total - c * chunk)
+            covered = []
+            prev = None
+            for row0, nr, a_slot, a0, a1, b_slot, b0, b1, osp in items[first[c]:first[c + 1]]:
+                assert 1 <= nr <= AT_ROWS and osp == -1
+                rr = list(range(r0 + row0, r0 + row0 + nr))
+                assert all(slots[r] == b_slot for r in rr) and all(pos[r + 1] == pos[r] + 1 for r in rr[:-1])
+                P_ = pfx_len[b_slot]
+                assert (a_slot, a0, a1) == (pfx_slot[b_slot], 0, P_) and (b0, b1) == (P_, pos[rr[-1]] + 1)
+                if prev is not None and slots[prev[-1]] == b_slot and pos[rr[0]] == pos[prev[-1]] + 1:
+                    assert len(prev) == AT_ROWS                                # a run of one slot is only cut after 64 rows
+                covered += rr; prev = rr
+            assert covered == list(range(r0, r0 + R)), (case, c)

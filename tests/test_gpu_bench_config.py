@@ -1,5 +1,5 @@
 """GPU parity at the configuration the headline number is quoted on (BASELINE.json configs[3]) and the cases VERDICT r1 listed
-as unproven: batch 256, kv_capacity 2048, 1345-row voice prefix (9 prefill chunks, sentences cut by chunk boundaries), KV length
+as unproven: batch 256, kv_capacity 2048, 1345-row voice prefix (several prefill chunks, one sentence cut by the first chunk boundary), KV length
 ~1.4-1.5k, default engine options — in BOTH prefix modes (shared voice prefix = cascade attention, and the reference's private copy);
 an F32 checkpoint; two voices in one batch; the second sentence of a stream; the KV-capacity edge; tap-point localisation.
 
@@ -47,8 +47,9 @@ def test_bench_configuration_matches_oracle(share, P, bench_dir, bench_oracle, o
     texts = [bench.synth_paragraph(i) for i in range(B)]
     toks = [ctx.tokenize(t) for t in texts]
     cum = np.concatenate([[0], np.cumsum([len(t) for t in toks])])
-    straddle = int(np.searchsorted(cum, 2048, side="right") - 1)          # its token rows are cut by the first 2048-row prefill chunk
-    assert cum[straddle] < 2048 < cum[straddle + 1], (straddle, cum[straddle], cum[straddle + 1])
+    chunk = P.default_config().max_prefill_rows                           # the engine's prefill chunk size
+    straddle = int(np.searchsorted(cum, chunk, side="right") - 1)         # its token rows are cut by the end of the first prefill chunk
+    assert cum[straddle] < chunk < cum[straddle + 1], (chunk, straddle, cum[straddle], cum[straddle + 1])
     mg = [oracle_mod.max_gen_len_for(t) for t in texts]
     eng.begin_sentences(list(range(B)), [st.voice] * B, toks, mg, [1 << 20] * B, [0.7] * B)
     check = [0, straddle, B - 1]
