@@ -81,6 +81,9 @@ B200_API int  b200_begin_sentences(b200_engine* e, int n, const int32_t* slots, 
 B200_API int  b200_begin_sentences_ex(b200_engine* e, int n, const int32_t* slots, const int32_t* voices, const int32_t* tokens,
                                       const int32_t* tok_off, const int32_t* max_gen_len, const int32_t* frames_after_eos,
                                       const float* temp, const uint32_t* rng_stream);
+/* Stream-ordered: the sentences in `slots` end now. From the next enqueued step on these slots are dead rows (no KV append, no attention,
+ * produced = 0) until a sentence start reuses them. Steps already enqueued are unaffected. Nothing in this call waits on the host. */
+B200_API int  b200_end_sentences(b200_engine* e, int n, const int32_t* slots);
 B200_API int  b200_voice_len(b200_engine* e, int voice);           /* prefix rows of a resident voice */
 B200_API int  b200_kv_capacity(b200_engine* e);
 B200_API int  b200_max_slots(b200_engine* e);
@@ -211,10 +214,27 @@ B200_API int  ptts_c_batch_configure(ptts_batch_t* b, int refill_min, int refill
 B200_API int  ptts_c_batch_add(ptts_batch_t* b, const char* voice, const char* text, float temp);   /* -> utterance id */
 B200_API int  ptts_c_batch_add_tokens(ptts_batch_t* b, int voice_id, const int32_t* ids, int n_ids, int max_gen_len, int frames_after_eos,
                                       float temp, uint32_t rng_stream /* 0 = job index + 1 */);
+/* Appends one more sentence, given as token ids, to utterance `utt` (an utterance of several sentences for callers that tokenise
+ * themselves); returns utt. B200_EINVAL for a cancelled utterance. */
+B200_API int  ptts_c_batch_append_tokens(ptts_batch_t* b, int utt, int voice_id, const int32_t* ids, int n_ids, int max_gen_len, int frames_after_eos,
+                                         float temp, uint32_t rng_stream);
 B200_API long long ptts_c_batch_run(ptts_batch_t* b);                  /* runs every queued sentence to completion; frames produced */
-B200_API int  ptts_c_batch_frames(ptts_batch_t* b, int utt);
-B200_API int  ptts_c_batch_read(ptts_batch_t* b, int utt, float* pcm, int max_frames);   /* [frames][1920] */
+B200_API int  ptts_c_batch_frames(ptts_batch_t* b, int utt);           /* frames generated for the utterance so far (popped ones included) */
+B200_API int  ptts_c_batch_read(ptts_batch_t* b, int utt, float* pcm, int max_frames);   /* [n][1920]: the frames not popped yet */
 B200_API void ptts_c_batch_stats(ptts_batch_t* b, ptts_batch_stats* out);
+/* Online serving. add / add_tokens may be called at any time; utterances added since the last pump join the back of the queue, longest
+ * sentence cap first. pump runs the scheduler until max_steps steps have been collected and at least one frame was produced, leaving the
+ * pipeline full for the next call; once nothing is queued or running it drains the pipeline. Returns the frames produced, 0 when idle,
+ * or a negative engine error. */
+B200_API long long ptts_c_batch_pump(ptts_batch_t* b, int max_steps);
+/* Copies up to max_frames ready frames [n][1920] of the utterance, in order, and returns n. A frame is ready once its step was collected
+ * and every earlier sentence of the utterance is done. A sentence's audio is freed once it is done and fully popped. */
+B200_API int  ptts_c_batch_pop(ptts_batch_t* b, int utt, float* pcm, int max_frames);
+/* Drops the utterance's queued sentences and frees the slots of its running ones (their frames still in flight are discarded); its audio
+ * not popped yet is freed and its frame count stops growing. A done utterance is left as it is. */
+B200_API int  ptts_c_batch_cancel(ptts_batch_t* b, int utt);
+/* 0 queued, 1 running, 2 done, 3 cancelled; *ready_frames (optional) = frames ptts_c_batch_pop would return now. */
+B200_API int  ptts_c_batch_status(ptts_batch_t* b, int utt, int* ready_frames);
 /* The same scheduler over caller-supplied engine calls (CPU tests drive it with a mock engine). */
 typedef int (*ptts_batch_begin_fn)(void* user, int n, const int32_t* slots, const int32_t* voices, const int32_t* tokens, const int32_t* tok_off,
                                    const int32_t* max_gen_len, const int32_t* frames_after_eos, const float* temp, const uint32_t* rng_stream);
@@ -222,6 +242,10 @@ typedef int (*ptts_batch_submit_fn)(void* user, int slot0, int n);
 typedef int (*ptts_batch_collect_fn)(void* user, float* pcm, int32_t* produced);
 B200_API ptts_batch_t* ptts_c_batch_create_with_ops(void* user, ptts_batch_begin_fn begin, ptts_batch_submit_fn submit, ptts_batch_collect_fn collect,
                                                     int n_slots, int frame_size);
+/* retires slots whose sentence was cancelled (b200_end_sentences); NULL = such slots stay live on the engine until refilled */
+typedef int (*ptts_batch_end_fn)(void* user, int n, const int32_t* slots);
+B200_API ptts_batch_t* ptts_c_batch_create_with_ops_ex(void* user, ptts_batch_begin_fn begin, ptts_batch_submit_fn submit, ptts_batch_collect_fn collect,
+                                                       ptts_batch_end_fn end, int n_slots, int frame_size);
 
 /* Host-only text front end (no GPU needed): tokenizer + sentence splitter objects. */
 typedef struct ptts_text_t ptts_text_t;

@@ -47,6 +47,7 @@ _I32P, _F32P, _U32P = ctypes.POINTER(ctypes.c_int32), ctypes.POINTER(ctypes.c_fl
 BATCH_BEGIN_FN = ctypes.CFUNCTYPE(ctypes.c_int, ctypes.c_void_p, ctypes.c_int, _I32P, _I32P, _I32P, _I32P, _I32P, _I32P, _F32P, _U32P)
 BATCH_SUBMIT_FN = ctypes.CFUNCTYPE(ctypes.c_int, ctypes.c_void_p, ctypes.c_int, ctypes.c_int)
 BATCH_COLLECT_FN = ctypes.CFUNCTYPE(ctypes.c_int, ctypes.c_void_p, _F32P, _I32P)
+BATCH_END_FN = ctypes.CFUNCTYPE(ctypes.c_int, ctypes.c_void_p, ctypes.c_int, _I32P)
 
 _lib = None
 
@@ -127,6 +128,7 @@ def lib():
         "ptts_c_count_words": (ci, [cp]),
         "ptts_c_stream_pending": (ci, [vp, ci, cp, ci]),
         "b200_begin_sentences_ex": (ci, [vp, ci, ip, ip, ip, ip, ip, ip, fp, ctypes.POINTER(ctypes.c_uint32)]),
+        "b200_end_sentences": (ci, [vp, ci, ip]),
         "b200_voice_len": (ci, [vp, ci]),
         "b200_kv_capacity": (ci, [vp]),
         "b200_max_slots": (ci, [vp]),
@@ -140,6 +142,12 @@ def lib():
         "ptts_c_batch_read": (ci, [vp, ci, fp, ci]),
         "ptts_c_batch_stats": (None, [vp, ctypes.POINTER(BatchStats)]),
         "ptts_c_batch_create_with_ops": (vp, [vp, BATCH_BEGIN_FN, BATCH_SUBMIT_FN, BATCH_COLLECT_FN, ci, ci]),
+        "ptts_c_batch_create_with_ops_ex": (vp, [vp, BATCH_BEGIN_FN, BATCH_SUBMIT_FN, BATCH_COLLECT_FN, BATCH_END_FN, ci, ci]),
+        "ptts_c_batch_append_tokens": (ci, [vp, ci, ci, ip, ci, ci, ci, cf, ctypes.c_uint32]),
+        "ptts_c_batch_pump": (ctypes.c_longlong, [vp, ci]),
+        "ptts_c_batch_pop": (ci, [vp, ci, fp, ci]),
+        "ptts_c_batch_cancel": (ci, [vp, ci]),
+        "ptts_c_batch_status": (ci, [vp, ci, ctypes.POINTER(ctypes.c_int)]),
         "ptts_c_text_create": (vp, [cp]),
         "ptts_c_text_destroy": (None, [vp]),
         "ptts_c_text_encode": (ci, [vp, cp, ip, ci]),
@@ -280,6 +288,13 @@ class Engine:
 
     def set_seed(self, seed):
         self.L.b200_set_seed(self.h, seed)
+
+    def end_sentences(self, slots):
+        """b200_end_sentences: the slots' sentences end before the next enqueued step (stream-ordered)."""
+        a = np.ascontiguousarray(slots, np.int32)
+        rc = self.L.b200_end_sentences(self.h, len(a), _ip(a))
+        if rc != 0:
+            raise RuntimeError(f"b200_end_sentences failed: {rc}")
 
     def slot_position(self, slot):
         return self.L.b200_slot_position(self.h, slot)
@@ -432,14 +447,19 @@ class Context:
 
 class Batch:
     """Continuous batching over the engine's slots (ptts_c_batch_*): queue utterances, run() generates all of them, finished slots are
-    refilled with queued sentences. With `ops` = (begin, submit, collect) Python callables the scheduler runs over a mock engine (CPU tests)."""
+    refilled with queued sentences. For online serving, add() at any time, pump() a few steps, pop() each utterance's ready frames in order
+    and cancel() the ones nobody waits for. With `ops` = (begin, submit, collect[, end]) Python callables the scheduler runs over a mock
+    engine (CPU tests)."""
+
+    STATES = ("queued", "running", "done", "cancelled")
 
     def __init__(self, ctx: "Context" = None, n_slots: int = 0, ops=None, frame_size: int = FRAME):
         L = lib()
-        self.frame_size = frame_size
+        self.frame_size, self.ctx = frame_size, ctx
         if ops is not None:
-            self._cbs = (BATCH_BEGIN_FN(ops[0]), BATCH_SUBMIT_FN(ops[1]), BATCH_COLLECT_FN(ops[2]))   # keep the thunks alive
-            self.h = L.ptts_c_batch_create_with_ops(None, self._cbs[0], self._cbs[1], self._cbs[2], n_slots, frame_size)
+            end = BATCH_END_FN(ops[3]) if len(ops) > 3 and ops[3] is not None else BATCH_END_FN()
+            self._cbs = (BATCH_BEGIN_FN(ops[0]), BATCH_SUBMIT_FN(ops[1]), BATCH_COLLECT_FN(ops[2]), end)   # keep the thunks alive
+            self.h = L.ptts_c_batch_create_with_ops_ex(None, *self._cbs, n_slots, frame_size)
         else:
             self.h = L.ptts_c_batch_create(ctx.h, n_slots)
         if not self.h:
@@ -454,9 +474,13 @@ class Batch:
             raise RuntimeError(f"ptts_c_batch_add failed: {u}")
         return u
 
-    def add_tokens(self, voice_id, ids, max_gen_len, frames_after_eos, temp=0.7, rng_stream=0) -> int:
+    def add_tokens(self, voice_id, ids, max_gen_len, frames_after_eos, temp=0.7, rng_stream=0, utt=None) -> int:
+        """One sentence given as token ids: a new utterance, or the next sentence of utterance `utt`."""
         a = np.ascontiguousarray(ids, np.int32)
-        u = lib().ptts_c_batch_add_tokens(self.h, voice_id, _ip(a), len(a), max_gen_len, frames_after_eos, float(temp), rng_stream)
+        if utt is None:
+            u = lib().ptts_c_batch_add_tokens(self.h, voice_id, _ip(a), len(a), max_gen_len, frames_after_eos, float(temp), rng_stream)
+        else:
+            u = lib().ptts_c_batch_append_tokens(self.h, utt, voice_id, _ip(a), len(a), max_gen_len, frames_after_eos, float(temp), rng_stream)
         if u < 0:
             raise RuntimeError(f"ptts_c_batch_add_tokens failed: {u}")
         return u
@@ -466,6 +490,35 @@ class Batch:
         if n < 0:
             raise RuntimeError(f"ptts_c_batch_run failed: {n}")
         return n
+
+    def pump(self, max_steps: int = 1) -> int:
+        """Runs the scheduler for at least max_steps collected steps (and one produced frame); returns the frames produced, 0 when idle."""
+        n = lib().ptts_c_batch_pump(self.h, max_steps)
+        if n < 0:
+            raise RuntimeError(f"ptts_c_batch_pump failed: {n}")
+        return n
+
+    def status(self, utt):
+        """(state, ready frames): state is one of Batch.STATES."""
+        ready = ctypes.c_int()
+        st = lib().ptts_c_batch_status(self.h, utt, ctypes.byref(ready))
+        if st < 0:
+            raise RuntimeError(f"ptts_c_batch_status failed: {st}")
+        return self.STATES[st], ready.value
+
+    def pop(self, utt) -> np.ndarray:
+        """The utterance's frames that are ready and were not popped before, [n, frame_size], in order."""
+        n = self.status(utt)[1]
+        out = np.zeros((max(n, 1), self.frame_size), np.float32)
+        got = lib().ptts_c_batch_pop(self.h, utt, _fp(out), n)
+        if got < 0:
+            raise RuntimeError(f"ptts_c_batch_pop failed: {got}")
+        return out[:got]
+
+    def cancel(self, utt):
+        rc = lib().ptts_c_batch_cancel(self.h, utt)
+        if rc != 0:
+            raise RuntimeError(f"ptts_c_batch_cancel failed: {rc}")
 
     def frames(self, utt) -> int:
         return lib().ptts_c_batch_frames(self.h, utt)
@@ -485,7 +538,9 @@ class Batch:
 
     def __del__(self):
         try:
-            lib().ptts_c_batch_destroy(self.h)
+            # destroy collects the steps still in flight on the engine: not possible once the context (and its engine) was closed
+            if self.ctx is None or self.ctx.h is not None:
+                lib().ptts_c_batch_destroy(self.h)
         except Exception:
             pass
 

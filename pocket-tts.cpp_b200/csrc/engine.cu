@@ -255,6 +255,7 @@ struct b200_engine {
     }
     bool begin_used = false;
     int* begin_meta = nullptr; float* begin_temp = nullptr; size_t begin_cap = 0;   // device copy of b200_begin_sentences' per-sentence metadata
+    int* end_slots = nullptr; size_t end_slots_cap = 0;                             // device copy of b200_end_sentences' slot list
     // b200_submit / b200_collect: up to three frames in flight, a ring of four pinned staging sets
     struct Pending { float* noise = nullptr; float* pcm = nullptr; int* produced = nullptr; size_t cap = 0; int slot0 = 0, n = 0; bool busy = false;
                      cudaEvent_t done_main = nullptr, done_mimi = nullptr; } pend[4];
@@ -981,6 +982,11 @@ __global__ void begin_meta_kernel(int n, const int* __restrict__ meta, const flo
     if (i < LDIM) { lat_f32[slot * LDIM + i] = bos[i]; lat_in_bf16[slot * LDIM + i] = __float2bfloat16_rn(bos[i]); }
     for (int c = i; c < M_DIM; c += blockDim.x) e_prev[(long long)slot * M_DIM + c] = 0.f;
 }
+// b200_end_sentences: the listed slots become dead rows from the next step on (main stream, so steps enqueued earlier still see them live).
+__global__ void end_slots_kernel(int n, const int* __restrict__ slots, int* __restrict__ active) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n) active[slots[i]] = 0;
+}
 __global__ void begin_copy_prefix_kernel(int n, const int* __restrict__ meta, char* kc, char* vc, long long slot_bytes, long long layer_bytes, long long row_bytes) {
     const int j = blockIdx.z;
     const int dst_slot = meta[j], src_slot = meta[n + j];
@@ -1430,6 +1436,24 @@ int b200_begin_sentences_ex(b200_engine* e, int n, const int32_t* slots, const i
     e->reset_pending = true;
     e->launches += 3;
     if (!rs.empty()) prefill_rows(e, rs, rp, &rt, nullptr);
+    return B200_OK;
+}
+
+// Retires slots: the next step sees them as dead rows (flow_in_kernel: no KV append, no attention; step_front_kernel: produced = 0, position
+// kept), exactly like a slot whose sentence reached EOS. The slot list goes through the pinned ring, so the call never waits on the host.
+int b200_end_sentences(b200_engine* e, int n, const int32_t* slots) {
+    NvtxRange nvtx_range("ptts.end_sentences");
+    if (!e || !e->finalized || n < 0 || (n > 0 && !slots)) return B200_EINVAL;
+    for (int i = 0; i < n; i++) if (slots[i] < 0 || slots[i] >= e->cfg.max_slots) return B200_EINVAL;
+    if (n == 0) return B200_OK;
+    PTTS_CUDA_CHECK(cudaSetDevice(e->cfg.device));
+    e->grow(e->end_slots, e->end_slots_cap, (size_t)n);
+    int* ps = (int*)e->pin_acquire((size_t)n * sizeof(int));
+    memcpy(ps, slots, (size_t)n * sizeof(int));
+    PTTS_CUDA_CHECK(cudaMemcpyAsync(e->end_slots, ps, (size_t)n * sizeof(int), cudaMemcpyHostToDevice, e->stream));
+    e->pin_release(e->stream);
+    launch_k(false, end_slots_kernel, dim3((n + 127) / 128), dim3(128), (size_t)0, e->stream, n, (const int*)e->end_slots, e->active);
+    e->launches++;
     return B200_OK;
 }
 

@@ -291,7 +291,6 @@ int ptts_c_stream_pending(ptts_stream_t* s, int index, char* buf, int buflen) {
 struct ptts_batch_t {
     ptts_context_t* ctx = nullptr;                // null for a scheduler driven through caller-supplied ops (tests)
     BatchScheduler* sched = nullptr;
-    std::vector<std::vector<int>> utt_jobs;       // utterance -> its sentences' job ids, in order
 };
 static int batch_begin_engine(void* u, int n, const int32_t* sl, const int32_t* vo, const int32_t* toks, const int32_t* off, const int32_t* mg,
                               const int32_t* fae, const float* tp, const uint32_t* rs) {
@@ -299,6 +298,7 @@ static int batch_begin_engine(void* u, int n, const int32_t* sl, const int32_t* 
 }
 static int batch_submit_engine(void* u, int slot0, int n) { return b200_submit((b200_engine*)u, slot0, n, nullptr); }
 static int batch_collect_engine(void* u, float* pcm, int32_t* produced) { return b200_collect((b200_engine*)u, pcm, produced); }
+static int batch_end_engine(void* u, int n, const int32_t* slots) { return b200_end_sentences((b200_engine*)u, n, slots); }
 
 ptts_batch_t* ptts_c_batch_create(ptts_context_t* ctx, int n_slots) {
     if (!ctx) return nullptr;
@@ -307,18 +307,23 @@ ptts_batch_t* ptts_c_batch_create(ptts_context_t* ctx, int n_slots) {
     for (bool used : ctx->slot_used) if (used) { fprintf(stderr, "error: ptts_c_batch_create needs a context without open streams (slots are shared)\n"); return nullptr; }
     auto* b = new ptts_batch_t; b->ctx = ctx;
     BatchOps ops; ops.user = ctx->engine; ops.begin = batch_begin_engine; ops.submit = batch_submit_engine; ops.collect = batch_collect_engine;
+    ops.end = batch_end_engine;
     b->sched = new BatchScheduler(ops, n_slots);
     if (ctx->seed_pushed != g_seed || !ctx->seed_valid) { b200_set_seed(ctx->engine, g_seed); ctx->seed_pushed = g_seed; ctx->seed_valid = true; }
     return b;
 }
-ptts_batch_t* ptts_c_batch_create_with_ops(void* user, ptts_batch_begin_fn begin, ptts_batch_submit_fn submit, ptts_batch_collect_fn collect, int n_slots, int frame_size) {
+ptts_batch_t* ptts_c_batch_create_with_ops_ex(void* user, ptts_batch_begin_fn begin, ptts_batch_submit_fn submit, ptts_batch_collect_fn collect,
+                                              ptts_batch_end_fn end, int n_slots, int frame_size) {
     if (!begin || !submit || !collect || n_slots < 1 || frame_size < 1) return nullptr;
     auto* b = new ptts_batch_t;
-    BatchOps ops; ops.user = user; ops.begin = begin; ops.submit = submit; ops.collect = collect;
+    BatchOps ops; ops.user = user; ops.begin = begin; ops.submit = submit; ops.collect = collect; ops.end = end;
     b->sched = new BatchScheduler(ops, n_slots, frame_size);
     return b;
 }
-void ptts_c_batch_destroy(ptts_batch_t* b) { if (b) { delete b->sched; delete b; } }
+ptts_batch_t* ptts_c_batch_create_with_ops(void* user, ptts_batch_begin_fn begin, ptts_batch_submit_fn submit, ptts_batch_collect_fn collect, int n_slots, int frame_size) {
+    return ptts_c_batch_create_with_ops_ex(user, begin, submit, collect, nullptr, n_slots, frame_size);
+}
+void ptts_c_batch_destroy(ptts_batch_t* b) { if (b) { b->sched->drain(); delete b->sched; delete b; } }
 int ptts_c_batch_configure(ptts_batch_t* b, int refill_min, int refill_every, int range_quantum, int keep_pcm) {
     if (!b) return B200_EINVAL;
     if (refill_min > 0) b->sched->refill_min = refill_min;
@@ -336,8 +341,7 @@ int ptts_c_batch_add(ptts_batch_t* b, const char* voice, const char* text, float
     if ((int)rv.size() <= vid) rv.resize(vid + 1, 1 << 30);
     rv[vid] = b200_kv_capacity(b->ctx->engine) - b200_voice_len(b->ctx->engine, vid);
     SentenceSplitter sp; sp.reset(); sp.ingest(text); sp.flush();
-    const int utt = (int)b->utt_jobs.size();
-    b->utt_jobs.emplace_back();
+    const int utt = b->sched->add_utterance();
     int idx = 0;
     for (const std::string& sent : sp.sentences) {
         BatchScheduler::Job j; j.utt = utt; j.index = idx++; j.voice = vid; j.temp = temp;
@@ -345,42 +349,57 @@ int ptts_c_batch_add(ptts_batch_t* b, const char* voice, const char* text, float
         j.fae = (words <= 4 ? 3 : 1) + 2; j.max_gen = (int)((words + 2.0f) * 12.5f);
         std::vector<int> ids = b->ctx->tokenizer.encode(sent);
         j.ids.assign(ids.begin(), ids.end());
-        b->utt_jobs[utt].push_back(b->sched->add_job(std::move(j)));
+        b->sched->add_job(std::move(j));
     }
-    b->sched->on_jobs_added();
+    return utt;
+}
+// One sentence given as token ids, appended to utterance `utt`.
+static int batch_add_token_job(ptts_batch_t* b, int utt, int voice_id, const int32_t* ids, int n_ids, int max_gen_len, int frames_after_eos, float temp, uint32_t rng_stream) {
+    if (n_ids < 0 || (n_ids > 0 && !ids)) return B200_EINVAL;
+    if (b->ctx) {
+        auto& rv = b->sched->room_of_voice;
+        const int vl = b200_voice_len(b->ctx->engine, voice_id);
+        if (vl < 0) return B200_EINVAL;
+        if ((int)rv.size() <= voice_id) rv.resize(voice_id + 1, 1 << 30);
+        rv[voice_id] = b200_kv_capacity(b->ctx->engine) - vl;
+    }
+    if (utt < 0) utt = b->sched->add_utterance();
+    BatchScheduler::Job j; j.utt = utt; j.index = b->sched->sentences(utt); j.voice = voice_id; j.temp = temp; j.max_gen = max_gen_len; j.fae = frames_after_eos;
+    j.rng_stream = rng_stream; j.ids.assign(ids, ids + n_ids);
+    b->sched->add_job(std::move(j));
     return utt;
 }
 int ptts_c_batch_add_tokens(ptts_batch_t* b, int voice_id, const int32_t* ids, int n_ids, int max_gen_len, int frames_after_eos, float temp, uint32_t rng_stream) {
-    if (!b || n_ids < 0 || (n_ids > 0 && !ids)) return B200_EINVAL;
-    if (b->ctx) {
-        auto& rv = b->sched->room_of_voice;
-        if ((int)rv.size() <= voice_id) rv.resize(voice_id + 1, 1 << 30);
-        const int vl = b200_voice_len(b->ctx->engine, voice_id);
-        if (vl < 0) return B200_EINVAL;
-        rv[voice_id] = b200_kv_capacity(b->ctx->engine) - vl;
-    }
-    BatchScheduler::Job j; j.utt = (int)b->utt_jobs.size(); j.index = 0; j.voice = voice_id; j.temp = temp; j.max_gen = max_gen_len; j.fae = frames_after_eos;
-    j.rng_stream = rng_stream; j.ids.assign(ids, ids + n_ids);
-    b->utt_jobs.emplace_back();
-    b->utt_jobs.back().push_back(b->sched->add_job(std::move(j)));
-    b->sched->on_jobs_added();
-    return (int)b->utt_jobs.size() - 1;
+    if (!b) return B200_EINVAL;
+    return batch_add_token_job(b, -1, voice_id, ids, n_ids, max_gen_len, frames_after_eos, temp, rng_stream);
+}
+int ptts_c_batch_append_tokens(ptts_batch_t* b, int utt, int voice_id, const int32_t* ids, int n_ids, int max_gen_len, int frames_after_eos, float temp,
+                               uint32_t rng_stream) {
+    if (!b || !b->sched->valid_utt(utt) || b->sched->status(utt, nullptr) == BatchScheduler::kCancelled) return B200_EINVAL;
+    return batch_add_token_job(b, utt, voice_id, ids, n_ids, max_gen_len, frames_after_eos, temp, rng_stream);
 }
 long long ptts_c_batch_run(ptts_batch_t* b) { return b ? b->sched->run() : B200_EINVAL; }
+long long ptts_c_batch_pump(ptts_batch_t* b, int max_steps) { return b && max_steps > 0 ? b->sched->pump(max_steps) : B200_EINVAL; }
 int ptts_c_batch_frames(ptts_batch_t* b, int utt) {
-    if (!b || utt < 0 || utt >= (int)b->utt_jobs.size()) return B200_EINVAL;
-    int n = 0; for (int j : b->utt_jobs[utt]) n += b->sched->jobs()[j].frames;
-    return n;
+    if (!b || !b->sched->valid_utt(utt)) return B200_EINVAL;
+    return b->sched->frames(utt);
 }
 int ptts_c_batch_read(ptts_batch_t* b, int utt, float* pcm, int max_frames) {
-    if (!b || utt < 0 || utt >= (int)b->utt_jobs.size() || !pcm) return B200_EINVAL;
-    int n = 0;
-    for (int j : b->utt_jobs[utt]) {
-        const auto& J = b->sched->jobs()[j];
-        const size_t fs = J.frames ? J.pcm.size() / (size_t)J.frames : 0;
-        for (int f = 0; f < J.frames && n < max_frames && fs; f++, n++) memcpy(pcm + (size_t)n * fs, J.pcm.data() + (size_t)f * fs, fs * sizeof(float));
-    }
-    return n;
+    if (!b || !b->sched->valid_utt(utt) || !pcm) return B200_EINVAL;
+    return b->sched->read(utt, pcm, max_frames);
+}
+int ptts_c_batch_pop(ptts_batch_t* b, int utt, float* pcm, int max_frames) {
+    if (!b || !b->sched->valid_utt(utt) || !pcm) return B200_EINVAL;
+    return b->sched->pop(utt, pcm, std::max(max_frames, 0));
+}
+int ptts_c_batch_cancel(ptts_batch_t* b, int utt) {
+    if (!b || !b->sched->valid_utt(utt)) return B200_EINVAL;
+    b->sched->cancel(utt);
+    return B200_OK;
+}
+int ptts_c_batch_status(ptts_batch_t* b, int utt, int* ready_frames) {
+    if (!b || !b->sched->valid_utt(utt)) return B200_EINVAL;
+    return b->sched->status(utt, ready_frames);
 }
 void ptts_c_batch_stats(ptts_batch_t* b, ptts_batch_stats* out) {
     if (!b || !out) return;
