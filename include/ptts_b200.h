@@ -64,6 +64,15 @@ B200_API int  b200_finalize_weights(b200_engine* e);
 /* Replaces get_state_for_audio_prompt (src/pocket_tts.cpp:100-124): prefill of audio_prompt[T][1024] (f32)
  * into a resident voice prefix. Returns the voice id (>=0) or an error. */
 B200_API int  b200_voice_create(b200_engine* e, const float* audio_prompt, int T);
+/* Voice cloning (DESIGN.md 4.6; the reference port has no encoder). The checkpoint's encoder set (mimi.encoder.*, mimi.encoder_transformer.*,
+ * mimi.downsample.*, flow_lm.speaker_proj_weight) is uploaded by b200_finalize_weights when present; b200_has_encoder tells (1 / 0).
+ * pcm: n >= 1 mono float samples at 24 kHz, right-padded with zeros to a multiple of 1920; T = ceil(n / 1920) prompt rows.
+ * b200_voice_embed_audio encodes on the engine stream and returns T; with out != NULL ([T][1024]) it copies the audio_prompt rows out
+ * (synchronises). b200_voice_create_from_audio encodes and prefills a new voice without a host round trip or wait; returns the voice id.
+ * Errors: B200_ENOTFOUND no encoder weights, B200_EINVAL n < 1 or a NULL pointer, B200_ECAPACITY T > kv_capacity or max_voices reached. */
+B200_API int  b200_has_encoder(b200_engine* e);
+B200_API int  b200_voice_embed_audio(b200_engine* e, const float* pcm, long long n, float* out);
+B200_API int  b200_voice_create_from_audio(b200_engine* e, const float* pcm, long long n);
 
 /* Replaces _stream_sentence_init (src/pocket_tts.cpp:416-444): restore the voice-conditioned KV prefix
  * (copy_states, models/flow_lm.h:70-78), reset the Mimi states (models/mimi.h:71-75), prefill the text tokens,
@@ -142,7 +151,8 @@ B200_API int  b200_read_kv(b200_engine* e, int slot, int layer, int which, int n
 /* Tap points for localising a parity failure (replaces GraphContext::debug, src/context.h:526-547; names follow the tests' CPU restatement):
  * "flow.layer<l>" / "flow.attn<l>" [1024] (need b200_debug_taps(e, 1): steps then run eagerly on one stream), "mimi.upsample" [16*512],
  * "mimi.transformer" [16*512], "seanet.conv0" [16*512], "seanet.convt2" [96*256], "seanet.res3" [96*256], "seanet.res6" [480*128],
- * "seanet.res9" [1920*64] of `slot` after its last step. out == NULL returns the element count. */
+ * "seanet.res9" [1920*64] of `slot` after its last step; "enc.seanet" [16T*512], "enc.transformer" [16T*512], "enc.downsample" [T*512] of the
+ * last clone (any valid slot). out == NULL returns the element count. */
 B200_API int  b200_debug_taps(b200_engine* e, int on);
 B200_API int  b200_debug_tap(b200_engine* e, const char* name, int slot, float* out, int max_elems);
 /* Host-only: tile width (32/64/128) and deterministic split-K factor the GEMM dispatcher would use (cost model of gemm_tc.cuh). */
@@ -174,6 +184,10 @@ B200_API int  b200_debug_attention(b200_engine* e, int layer, int prefill, int s
  * items_out[cap][9] = {row0, nrows, a_slot, a_k0, a_k1, b_slot, b_k0, b_k1, out_split}; *n_items = the item count. */
 B200_API int  b200_debug_attn_plan(int prefill, int n, const int32_t* row_slot, const int32_t* row_pos, const int32_t* pfx_slot, const int32_t* pfx_len,
                                    int num_sms, int chunk_rows, int max_voices, int32_t* items_out, int cap, int32_t* aux_out, int* n_items);
+/* Unit-test hook for the voice-cloning encoder's window attention (tests/test_gpu_voice_clone.py): q, k, v [R][512] f32 (rounded to bf16;
+ * q and k as the QKV epilogue leaves them, rotated), positions = row indices, key j visible to query i iff 0 <= i - j < 250, 8 heads of 64;
+ * out [R][512] = the bf16 attention output as f32. Synchronises. */
+B200_API int  b200_debug_window_attention(b200_engine* e, int R, const float* q, const float* k, const float* v, float* out);
 B200_API const char* b200_build_info(void);
 
 /* ---- extern "C" aliases of the reference's C++ API (include/pocket_tts/pocket_tts.h:18-42) ---- */
@@ -200,6 +214,15 @@ B200_API int ptts_c_tokenize(ptts_context_t* ctx, const char* text, int32_t* ids
 B200_API int ptts_c_count_words(const char* text);
 /* Pending sentences of a stream after send/flush (conditioners/text.h:207-251); returns count, copies the i-th. */
 B200_API int ptts_c_stream_pending(ptts_stream_t* s, int index, char* buf, int buflen);
+/* Voice cloning through the context. A voice argument ending in ".wav" (RIFF PCM16 or float32, any channel count, mixed down to mono,
+ * 24 kHz only) is cloned on first use, like a voice file is loaded. ptts_c_voice_add_audio registers pcm[n] (mono) under `name`, which then
+ * works wherever a voice name does; returns the voice id or a B200_E* error (B200_EINVAL for sample_rate != 24000 or a name in use).
+ * ptts_c_voice_export writes a cloned voice's audio_prompt [1, T, 1024] as an F32 safetensors voice file (B200_ENOTFOUND: not a clone). */
+B200_API int ptts_c_voice_add_audio(ptts_context_t* ctx, const char* name, const float* pcm, long long n, int sample_rate);
+B200_API int ptts_c_voice_export(ptts_context_t* ctx, const char* name, const char* path);
+/* Host-only WAV reader: copies up to max mono samples into pcm (may be NULL), sets *sample_rate (may be NULL); returns the number of
+ * samples in the file, or B200_EINVAL for a file that is not a readable RIFF PCM16 / float32 WAV. */
+B200_API int ptts_c_wav_read(const char* path, float* pcm, long long max, int* sample_rate);
 
 /* ---- continuous batching: the batched extension of the streaming API (SURVEY 8b(3)). The reference rolls one stream to its next
  * sentence inside ptts_stream_receive (src/pocket_tts.cpp:494-519); here sentences of many utterances share the engine's slots and a

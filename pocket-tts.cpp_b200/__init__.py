@@ -155,6 +155,13 @@ def lib():
         "ptts_c_text_flush": (None, [vp]),
         "ptts_c_text_reset": (None, [vp]),
         "ptts_c_text_pop": (ci, [vp, cp, ci]),
+        "b200_has_encoder": (ci, [vp]),
+        "b200_debug_window_attention": (ci, [vp, ci, fp, fp, fp, fp]),
+        "b200_voice_embed_audio": (ci, [vp, fp, ctypes.c_longlong, fp]),
+        "b200_voice_create_from_audio": (ci, [vp, fp, ctypes.c_longlong]),
+        "ptts_c_voice_add_audio": (ci, [vp, cp, fp, ctypes.c_longlong, ci]),
+        "ptts_c_voice_export": (ci, [vp, cp, cp]),
+        "ptts_c_wav_read": (ci, [cp, fp, ctypes.c_longlong, ctypes.POINTER(ctypes.c_int)]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(L, name)
@@ -201,6 +208,38 @@ class Engine:
         v = self.L.b200_voice_create(self.h, _fp(prompt), prompt.shape[0])
         if v < 0:
             raise RuntimeError(f"b200_voice_create failed: {v}")
+        return v
+
+    @property
+    def has_encoder(self) -> bool:
+        """True when the checkpoint carries the voice-cloning encoder."""
+        return self.L.b200_has_encoder(self.h) == 1
+
+    def embed_audio(self, pcm) -> np.ndarray:
+        """Mono 24 kHz PCM -> audio_prompt rows [T, 1024] (T = ceil(n / 1920)), encoded on the device."""
+        x = np.ascontiguousarray(np.asarray(pcm, np.float32).reshape(-1))
+        T = -(-len(x) // FRAME)
+        out = np.zeros((max(T, 1), 1024), np.float32)
+        rc = self.L.b200_voice_embed_audio(self.h, _fp(x) if len(x) else None, len(x), _fp(out))
+        if rc < 0:
+            raise RuntimeError(f"b200_voice_embed_audio failed: {rc}")
+        return out[:rc]
+
+    def debug_window_attention(self, q, k, v) -> np.ndarray:
+        """The encoder's window attention alone over q, k, v [R, 512] (rotated q / k); returns the bf16 output as f32 [R, 512]."""
+        q, k, v = (np.ascontiguousarray(np.asarray(t, np.float32).reshape(-1, 512)) for t in (q, k, v))
+        out = np.zeros_like(q)
+        rc = self.L.b200_debug_window_attention(self.h, q.shape[0], _fp(q), _fp(k), _fp(v), _fp(out))
+        if rc != 0:
+            raise RuntimeError(f"b200_debug_window_attention failed: {rc}")
+        return out
+
+    def voice_from_audio(self, pcm) -> int:
+        """Clones a voice from mono 24 kHz PCM: encode + prefill on the device; returns the voice id."""
+        x = np.ascontiguousarray(np.asarray(pcm, np.float32).reshape(-1))
+        v = self.L.b200_voice_create_from_audio(self.h, _fp(x) if len(x) else None, len(x))
+        if v < 0:
+            raise RuntimeError(f"b200_voice_create_from_audio failed: {v}")
         return v
 
     def begin_sentence(self, slot, voice, tokens, max_gen_len, frames_after_eos, temp=0.0):
@@ -444,6 +483,20 @@ class Context:
     def stream(self, voice="cosette", temp=0.7) -> "Stream":
         return Stream(self, voice, temp)
 
+    def add_voice(self, name: str, pcm, sample_rate: int = SAMPLE_RATE) -> int:
+        """Clones a voice from mono PCM (24 kHz only) and registers it under `name`; returns the engine voice id."""
+        x = np.ascontiguousarray(np.asarray(pcm, np.float32).reshape(-1))
+        v = lib().ptts_c_voice_add_audio(self.h, name.encode(), _fp(x) if len(x) else None, len(x), int(sample_rate))
+        if v < 0:
+            raise RuntimeError(f"ptts_c_voice_add_audio failed: {v}")
+        return v
+
+    def export_voice(self, name: str, path: str):
+        """Writes a cloned voice as an audio_prompt [1, T, 1024] F32 safetensors voice file."""
+        rc = lib().ptts_c_voice_export(self.h, name.encode(), path.encode())
+        if rc != 0:
+            raise RuntimeError(f"ptts_c_voice_export failed: {rc}")
+
 
 class Batch:
     """Continuous batching over the engine's slots (ptts_c_batch_*): queue utterances, run() generates all of them, finished slots are
@@ -576,6 +629,17 @@ class Stream:
             lib().ptts_c_stream_pending(self.h, i, b, 65536)
             out.append(b.value)
         return out
+
+
+def read_wav(path: str):
+    """Host-only RIFF reader of the engine (PCM16 / float32, mixed down to mono): (samples float32 [n], sample_rate)."""
+    rate = ctypes.c_int()
+    n = lib().ptts_c_wav_read(path.encode(), None, 0, ctypes.byref(rate))
+    if n < 0:
+        raise ValueError(f"{path}: not a readable PCM16 / float32 WAV file")
+    out = np.zeros(max(n, 1), np.float32)
+    lib().ptts_c_wav_read(path.encode(), _fp(out), n, ctypes.byref(rate))
+    return out[:n], rate.value
 
 
 def set_seed(seed: int):

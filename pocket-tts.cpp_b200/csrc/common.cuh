@@ -134,6 +134,7 @@ struct Epi {
     int kv_f32 = 0;                    // FlowLM cache dtype (1 = f32 like the reference, 0 = bf16)
     float* q_out_f32 = nullptr;        // FlowLM: [R][1024] f32 de-interleaved rotated q
     __nv_bfloat16* q_out_bf16 = nullptr;  // Mimi: [R][512] bf16 rotated q
+    int kv_linear = 0;                 // EPI_MIMI_QKV only: k / v land in row `row` of kcache / vcache (no ring, no row_slot / row_pos)
 };
 
 }  // namespace ptts

@@ -11,6 +11,7 @@
 #include "head_fused.cuh"
 #include "seanet_tail.cuh"
 #include "seanet_res.cuh"
+#include "encoder.cuh"
 
 #include <cuda_profiler_api.h>
 #include <nvtx3/nvToolsExt.h>
@@ -953,6 +954,107 @@ struct b200_engine {
         if (nf > pin_f_n) { if (pin_f) cudaFreeHost(pin_f); PTTS_CUDA_CHECK(cudaMallocHost(&pin_f, nf * sizeof(float))); pin_f_n = nf; }
         if (ni > pin_i_n) { if (pin_i) cudaFreeHost(pin_i); PTTS_CUDA_CHECK(cudaMallocHost(&pin_i, ni * sizeof(int))); pin_i_n = ni; }
     }
+
+    // ---- voice-cloning encoder (DESIGN.md §4.6): PCM -> audio_prompt rows [T][1024] on the main stream ----
+    bool has_enc = false;
+    ConvW ec0, er1a, er1b, es3, er4a, er4b, es6, er7a, er7b, es9, ec11, eds;
+    struct { LinW in_proj, out_proj, lin1, lin2; float *n1w, *n1b, *n2w, *n2b, *ls1, *ls2; } el[M_LAYERS];
+    LinW spk;
+    // Scratch of the last clone, grown to the longest prompt so far (one allocation; its own buffers, so that a Mimi decode running on the
+    // other stream beside it shares nothing with it). The zero rows in front of the conv inputs are causal padding and are never written.
+    struct EncBufs {
+        int T = 0;
+        float *pcm, *y0, *y1, *y2, *xs, *xt, *lat, *prompt; float2* cs;
+        __half *a0, *b0, *c0, *a1, *b1, *c1, *a2, *b2, *c2, *d3, *ds;
+        __nv_bfloat16 *ln, *q, *k, *v, *att, *ff, *lat_bf;
+    } eb;
+    int enc_T = 0;                       // rows of the last clone (debug taps)
+    // Pinned staging of the clone's PCM, sized with the scratch. Not the shared pinned ring: a 10 s prompt is ~1 MB, and growing a ring
+    // slot to that size (cudaFreeHost + cudaMallocHost) on most clones stalls the serving pipeline.
+    float* enc_pin = nullptr; size_t enc_pin_cap = 0; cudaEvent_t enc_pin_ev = nullptr; bool enc_pin_used = false;
+    void enc_reserve(int T) {
+        if (T <= eb.T) return;
+        const int Tc = std::min(std::max(T, 2 * eb.T), cfg.kv_capacity);   // no clone is longer than kv_capacity rows
+        const long long L0 = (long long)ENC_HOP * Tc, L1 = L0 / 4, L2 = L1 / 5, L3 = L2 / 6;
+        size_t off = 0;
+        std::vector<std::pair<void**, size_t>> parts;
+        auto part = [&](auto*& p, size_t bytes) { parts.push_back({(void**)&p, off}); off += (bytes + 255) / 256 * 256; };
+        part(eb.pcm, (6 + L0) * 4); part(eb.y0, L0 * 64 * 4); part(eb.a0, (2 + L0) * 64 * 2); part(eb.b0, L0 * 64 * 2); part(eb.c0, (4 + L0) * 64 * 2);
+        part(eb.y1, L1 * 128 * 4); part(eb.a1, (2 + L1) * 128 * 2); part(eb.b1, L1 * 64 * 2); part(eb.c1, (5 + L1) * 128 * 2);
+        part(eb.y2, L2 * 256 * 4); part(eb.a2, (2 + L2) * 256 * 2); part(eb.b2, L2 * 128 * 2); part(eb.c2, (6 + L2) * 256 * 2);
+        part(eb.d3, (2 + L3) * 512 * 2); part(eb.xs, L3 * 512 * 4); part(eb.xt, L3 * 512 * 4); part(eb.cs, L3 * 32 * 8);
+        part(eb.ln, L3 * 512 * 2); part(eb.q, L3 * 512 * 2); part(eb.k, L3 * 512 * 2); part(eb.v, L3 * 512 * 2); part(eb.att, L3 * 512 * 2);
+        part(eb.ff, L3 * M_FF * 2); part(eb.ds, (16 + L3) * 512 * 2); part(eb.lat, (long long)Tc * 512 * 4); part(eb.lat_bf, (long long)Tc * 512 * 2);
+        part(eb.prompt, (long long)Tc * D_MODEL * 4);
+        char* base = dalloc<char>(off, true);    // zeroed: padding rows and the padded channels of b0 stay zero for every later clone
+        for (auto& pp : parts) *pp.first = base + pp.second;
+        eb.T = Tc;
+    }
+    // Encodes pcm (already in eb.pcm behind 6 zero samples, zero-padded to 1920 T) into eb.prompt [T][1024]. Main stream, no host wait.
+    void encode(int T) {
+        const int BIG = 1 << 30;
+        const long long L0 = (long long)ENC_HOP * T, L1 = L0 / 4, L2 = L1 / 5, L3 = L2 / 6;
+        set_pdl(false);
+        tc->tma_epilogue = false;                                  // the Mimi stream may be running beside the encoder
+        launch_k(false, enc_front_kernel, dim3((unsigned)((L0 * 64 + 255) / 256)), dim3(256), (size_t)0, stream, (const float*)eb.pcm, (const __half*)ec0.w,
+                 (const float*)ec0.b, (int)L0, eb.y0, eb.a0 + 2 * 64);
+        launches++;
+        // residual block: x + conv1(ELU(conv3(ELU(x)))), then ELU -> the f16 input rows of the next strided conv (behind `pad` zero rows)
+        auto resblock = [&](ConvW& ca, ConvW& cb, long long L, int C, __half* a, __half* b, int ldb, float* y, __half* c, int pad) {
+            { Epi e; e.rps = (int)L; e.bias = ca.b; e.act = ACT_ELU; e.out2 = b; e.out2_map = rows(ldb); e.out2_type = OUT2_F16;
+              gemm<__half>(a, smap((L + 2) * C, C, 0), (int)L, ca.w, ca.wk, (int)L, ca.N, ca.K, e); }
+            { Epi e; e.bias = cb.b; e.resid = y; e.resid_map = rows(C); e.act = ACT_ELU; e.out2 = c + (long long)pad * C; e.out2_map = rows(C); e.out2_type = OUT2_F16;
+              gemm<__half>(b, rows(ldb), BIG, cb.w, cb.wk, (int)L, cb.N, cb.K, e); }
+        };
+        // conv k = 2r, stride r over [L][C] = 2-tap window over rows of r*C channels (one zero row-group in front): Lo = L / r rows out
+        auto strided = [&](ConvW& cw, const __half* in, long long Lo, int rC, float* y, __half* out2, int out_pad) {
+            Epi e; e.rps = (int)Lo; e.bias = cw.b; e.act = ACT_ELU; e.out2 = out2 + (long long)out_pad * cw.N; e.out2_map = rows(cw.N); e.out2_type = OUT2_F16;
+            if (y) { e.out = y; e.out_map = rows(cw.N); }
+            gemm<__half>(in, smap((Lo + 1) * rC, rC, 0), (int)Lo, cw.w, cw.wk, (int)Lo, cw.N, cw.K, e);
+        };
+        resblock(er1a, er1b, L0, 64, eb.a0, eb.b0, 64, eb.y0, eb.c0, 4);
+        strided(es3, eb.c0, L1, 4 * 64, eb.y1, eb.a1, 2);
+        resblock(er4a, er4b, L1, 128, eb.a1, eb.b1, 64, eb.y1, eb.c1, 5);
+        strided(es6, eb.c1, L2, 5 * 128, eb.y2, eb.a2, 2);
+        resblock(er7a, er7b, L2, 256, eb.a2, eb.b2, 128, eb.y2, eb.c2, 6);
+        strided(es9, eb.c2, L3, 6 * 256, nullptr, eb.d3, 2);
+        { Epi e; e.rps = (int)L3; e.bias = ec11.b; e.out = eb.xs; e.out_map = rows(512);
+          gemm<__half>(eb.d3, smap((L3 + 2) * 512, 512, 0), (int)L3, ec11.w, ec11.wk, (int)L3, ec11.N, ec11.K, e); }
+        // encoder transformer over the 16 T rows (positions 0 .. 16T-1), layer math of the Mimi decoder's, plain causal window
+        const int R = (int)L3;
+        launch_k(false, enc_rope_kernel, dim3((R * 32 + 255) / 256), dim3(256), (size_t)0, stream, (const float*)freq_mimi, eb.cs, R);
+        launches++;
+        auto ln = [&](const float* x, const float* w, const float* b) {
+            if (R >= 512) launch_k(false, layernorm_rows_kernel<M_DIM>, dim3((R + 7) / 8), dim3(256), (size_t)0, stream, x, R, 0.0f, w, b, eb.ln);
+            else launch_k(false, layernorm_kernel<M_DIM>, dim3(R), dim3(M_DIM / 4), (size_t)0, stream, x, rows(M_DIM), BIG, R, 0.0f, w, b, nullptr, nullptr, 0, eb.ln, nullptr);
+            launches++;
+        };
+        for (int l = 0; l < M_LAYERS; l++) {
+            auto& L = el[l];
+            const float* xin = l == 0 ? eb.xs : eb.xt;
+            ln(xin, L.n1w, L.n1b);
+            Epi eq; eq.mode = EPI_MIMI_QKV; eq.kv_linear = 1; eq.cs = eb.cs; eq.kcache = eb.k; eq.vcache = eb.v; eq.q_out_bf16 = eb.q;
+            lin(eb.ln, L.in_proj, R, eq);
+            launch_k(false, attn_window_kernel, dim3((R + AW_Q - 1) / AW_Q, M_HEADS), dim3(AW_WARPS * 32), AW_SMEM, stream, (const __nv_bfloat16*)eb.q,
+                     (const __nv_bfloat16*)eb.k, (const __nv_bfloat16*)eb.v, R, eb.att);
+            launches++;
+            Epi eo; eo.colscale = L.ls1; eo.resid = xin; eo.resid_map = rows(M_DIM); eo.out = eb.xt; eo.out_map = rows(M_DIM);
+            lin(eb.att, L.out_proj, R, eo);
+            ln(eb.xt, L.n2w, L.n2b);
+            Epi e1; e1.out2 = eb.ff; e1.out2_map = rows(M_FF); e1.out2_type = OUT2_BF16; e1.act = ACT_GELU;
+            lin(eb.ln, L.lin1, R, e1);
+            Epi e2; e2.colscale = L.ls2; e2.resid = eb.xt; e2.resid_map = rows(M_DIM); e2.out = eb.xt; e2.out_map = rows(M_DIM);
+            lin(eb.ff, L.lin2, R, e2);
+        }
+        // downsample k32 s16 (replicate padding) as a 2-tap window over rows of 16 x 512, then the speaker projection
+        launch_k(false, enc_ds_pad_kernel, dim3((unsigned)(((long long)(R + 16) * M_DIM + 255) / 256)), dim3(256), (size_t)0, stream, (const float*)eb.xt, R, eb.ds);
+        { Epi e; e.rps = T; e.bias = eds.b; e.out = eb.lat; e.out_map = rows(512);
+          gemm<__half>(eb.ds, smap((long long)(T + 1) * 16 * 512, 16 * 512, 0), T, eds.w, eds.wk, T, eds.N, eds.K, e); }
+        launch_k(false, enc_to_bf16_kernel, dim3((unsigned)(((long long)T * 512 + 255) / 256)), dim3(256), (size_t)0, stream, (const float*)eb.lat, (long long)T * 512, eb.lat_bf);
+        launches += 2;
+        { Epi e; e.out = eb.prompt; e.out_map = rows(D_MODEL); lin(eb.lat_bf, spk, T, e); }
+        enc_T = T;
+    }
 };
 
 namespace {
@@ -1083,6 +1185,7 @@ void b200_engine_destroy(b200_engine* e) {
     if (e->pin_i) cudaFreeHost(e->pin_i);
     for (auto& ps : e->pins) { if (ps.p) cudaFreeHost(ps.p); if (ps.ev) cudaEventDestroy(ps.ev); }
     if (e->ev_begin) cudaEventDestroy(e->ev_begin); if (e->ev_reset) cudaEventDestroy(e->ev_reset);
+    if (e->enc_pin) cudaFreeHost(e->enc_pin); if (e->enc_pin_ev) cudaEventDestroy(e->enc_pin_ev);
     tc_plan_cache_destroy(e->tc);
     for (int i = 0; i < 2; i++) { cudaEventDestroy(e->ev_main[i]); cudaEventDestroy(e->ev_mimi[i]); cudaEventDestroy(e->ev_dec[i]); cudaEventDestroy(e->ev_copy[i]); cudaEventDestroy(e->ev_noise[i]); }
     for (auto& ev : e->ev_seg) cudaEventDestroy(ev);
@@ -1216,6 +1319,46 @@ int b200_finalize_weights(b200_engine* e) {
         }
         e->freq_flow = e->upload(ff); e->freq_mimi = e->upload(fm);
     }
+    {   // voice-cloning encoder: all or nothing. Its key names live in this one table (a checkpoint with other names is a one-line change).
+        const std::string se = "mimi.encoder.model.", te = "mimi.encoder_transformer.transformer.layers.";
+        struct ConvKey { ConvW* dst; std::string key; int co, ci, k, ci_pad; };
+        const ConvKey convs[] = {
+            {&e->ec0, se + "0", 64, 1, 7, 0},          {&e->er1a, se + "1.block.1", 32, 64, 3, 0},  {&e->er1b, se + "1.block.3", 64, 32, 1, 64},
+            {&e->es3, se + "3", 128, 64, 8, 0},        {&e->er4a, se + "4.block.1", 64, 128, 3, 0}, {&e->er4b, se + "4.block.3", 128, 64, 1, 0},
+            {&e->es6, se + "6", 256, 128, 10, 0},      {&e->er7a, se + "7.block.1", 128, 256, 3, 0}, {&e->er7b, se + "7.block.3", 256, 128, 1, 0},
+            {&e->es9, se + "9", 512, 256, 12, 0},      {&e->ec11, se + "11", 512, 512, 3, 0},       {&e->eds, "mimi.downsample.conv", 512, 512, 32, 0}};
+        const char* layer_keys[] = {"self_attn.in_proj.weight", "self_attn.out_proj.weight", "linear1.weight", "linear2.weight", "norm1.weight", "norm2.weight",
+                                    "layer_scale_1.scale", "layer_scale_2.scale"};
+        const std::string spk_key = "flow_lm.speaker_proj_weight";
+        if (e->find(se + "0.conv.weight", false)) {
+            std::vector<std::string> need;
+            for (const auto& c : convs) need.push_back(c.key + ".conv.weight");
+            for (int l = 0; l < M_LAYERS; l++) for (const char* k : layer_keys) need.push_back(te + std::to_string(l) + "." + k);
+            need.push_back(spk_key);
+            for (const auto& k : need) if (!e->find(k, false)) { fprintf(stderr, "ptts_b200: error: incomplete encoder weights, missing tensor %s\n", k.c_str()); return B200_EINVAL; }
+            for (const auto& c : convs) {
+                const auto* w = e->find(c.key + ".conv.weight");
+                if ((int64_t)w->f.size() != (int64_t)c.co * c.ci * c.k) { fprintf(stderr, "ptts_b200: error: bad shape for %s.conv.weight\n", c.key.c_str()); return B200_EINVAL; }
+                *c.dst = e->up_conv(c.key, c.co, c.ci, c.k, c.ci_pad);
+            }
+            for (int l = 0; l < M_LAYERS; l++) {
+                const std::string p = te + std::to_string(l) + ".";
+                auto& L = e->el[l];
+                L.in_proj = e->up_lin(p + "self_attn.in_proj", 3 * M_DIM, M_DIM); L.out_proj = e->up_lin(p + "self_attn.out_proj", M_DIM, M_DIM);
+                L.lin1 = e->up_lin(p + "linear1", M_FF, M_DIM); L.lin2 = e->up_lin(p + "linear2", M_DIM, M_FF);
+                L.n1w = e->up_f32(p + "norm1.weight"); L.n1b = e->up_f32(p + "norm1.bias", false);
+                L.n2w = e->up_f32(p + "norm2.weight"); L.n2b = e->up_f32(p + "norm2.bias", false);
+                L.ls1 = e->up_f32(p + "layer_scale_1.scale"); L.ls2 = e->up_f32(p + "layer_scale_2.scale");
+            }
+            {   // [1024][512] plain tensor (no .weight suffix), no bias
+                const auto* w = e->find(spk_key);
+                if ((int64_t)w->f.size() != (int64_t)D_MODEL * M_DIM) { fprintf(stderr, "ptts_b200: error: bad shape for %s\n", spk_key.c_str()); return B200_EINVAL; }
+                const auto wb = b200_engine::to_bf16(w->f);
+                e->spk.out = D_MODEL; e->spk.in = M_DIM; e->spk.w = e->upload(wb); e->spk.wk = e->upload(tc_kblock_major(wb, D_MODEL, M_DIM));
+            }
+            e->has_enc = true;
+        }
+    }
     e->host.clear();
 
     // ---------------- state + scratch ----------------
@@ -1293,6 +1436,7 @@ int b200_finalize_weights(b200_engine* e) {
     PTTS_CUDA_CHECK(cudaFuncSetAttribute(head_res_cluster_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)HF_SMEM_BYTES));
     PTTS_CUDA_CHECK(cudaFuncSetAttribute(seanet_tail_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ST_SMEM_BYTES));
     PTTS_CUDA_CHECK(cudaFuncSetAttribute(seanet_res_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SR_SMEM_BYTES));
+    PTTS_CUDA_CHECK(cudaFuncSetAttribute(attn_window_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)AW_SMEM));
     e->actx.row_slot = e->row_slot; e->actx.row_pos = e->row_pos; e->actx.cs = e->cs;
     PTTS_CUDA_CHECK(cudaStreamSynchronize(e->stream));
     e->finalized = true;
@@ -1302,7 +1446,9 @@ int b200_finalize_weights(b200_engine* e) {
 // ---- ragged FlowLM prefill (reference _run_flow_lm with T > 1, src/pocket_tts.cpp:40-98): rows = (slot, position, token | voice row), slot-major
 //      with ascending positions. Everything is staged once (pinned ring -> device) and enqueued without a host synchronisation; the rows are
 //      processed in chunks of max_prefill_rows (a later chunk of a sentence attends to the cache rows the earlier chunk appended). ----
-static void prefill_rows(b200_engine* e, const std::vector<int>& slots, const std::vector<int>& pos, const std::vector<int>* tokens, const float* x_host) {
+// x_host / x_dev: the rows' input vectors [total][1024] on the host (staged through the pinned ring) or already on the device.
+static void prefill_rows(b200_engine* e, const std::vector<int>& slots, const std::vector<int>& pos, const std::vector<int>* tokens, const float* x_host,
+                         const float* x_dev = nullptr) {
     NvtxRange nvtx_range("ptts.prefill_rows");
     const int total = (int)slots.size(), MRp = e->cfg.max_prefill_rows;
     if (total == 0) return;
@@ -1340,7 +1486,7 @@ static void prefill_rows(b200_engine* e, const std::vector<int>& slots, const st
             launch_k(false, embed_gather_kernel, dim3(R), dim3(256), (size_t)(0), e->stream, e->embed, (const int*)(e->pf_int + 2 * total + r0), e->h, R);
             e->launches++;
         } else {
-            PTTS_CUDA_CHECK(cudaMemcpyAsync(e->h, e->pf_x + (size_t)r0 * D_MODEL, (size_t)R * D_MODEL * sizeof(float), cudaMemcpyDeviceToDevice, e->stream));
+            PTTS_CUDA_CHECK(cudaMemcpyAsync(e->h, (x_dev ? x_dev : e->pf_x) + (size_t)r0 * D_MODEL, (size_t)R * D_MODEL * sizeof(float), cudaMemcpyDeviceToDevice, e->stream));
         }
         launch_k(false, rope_table_kernel, dim3((R * 32 + 255) / 256), dim3(256), (size_t)(0), e->stream, e->actx.row_pos, e->freq_flow, e->cs, R);
         e->launches++;
@@ -1360,6 +1506,56 @@ int b200_voice_create(b200_engine* e, const float* audio_prompt, int T) {
     std::vector<int> slots(T, slot), pos(T);
     for (int i = 0; i < T; i++) pos[i] = i;
     if (T > 0) prefill_rows(e, slots, pos, nullptr, audio_prompt);
+    e->voice_len[v] = T;
+    return v;
+}
+
+int b200_has_encoder(b200_engine* e) { return e && e->finalized && e->has_enc ? 1 : 0; }
+
+// Voice cloning: uploads the PCM through the pinned ring and enqueues the encoder on the main stream (no host wait). Returns T.
+static int enc_enqueue(b200_engine* e, const float* pcm, long long n) {
+    if (!e || !e->finalized || !pcm || n < 1) return B200_EINVAL;
+    if (!e->has_enc) return B200_ENOTFOUND;
+    const long long T = (n + ENC_HOP - 1) / ENC_HOP;
+    if (T > e->cfg.kv_capacity) return B200_ECAPACITY;
+    PTTS_CUDA_CHECK(cudaSetDevice(e->cfg.device));
+    e->enc_reserve((int)T);
+    const long long L0 = T * ENC_HOP;
+    if (!e->enc_pin_ev) PTTS_CUDA_CHECK(cudaEventCreateWithFlags(&e->enc_pin_ev, cudaEventDisableTiming));
+    if (e->enc_pin_used) PTTS_CUDA_CHECK(cudaEventSynchronize(e->enc_pin_ev));   // the previous clone's upload (long done in steady state)
+    if (e->enc_pin_cap < (size_t)n) {
+        if (e->enc_pin) PTTS_CUDA_CHECK(cudaFreeHost(e->enc_pin));
+        e->enc_pin_cap = (size_t)e->eb.T * ENC_HOP;
+        PTTS_CUDA_CHECK(cudaMallocHost(&e->enc_pin, e->enc_pin_cap * sizeof(float)));
+    }
+    memcpy(e->enc_pin, pcm, (size_t)n * sizeof(float));
+    PTTS_CUDA_CHECK(cudaMemcpyAsync(e->eb.pcm + 6, e->enc_pin, (size_t)n * sizeof(float), cudaMemcpyHostToDevice, e->stream));
+    PTTS_CUDA_CHECK(cudaEventRecord(e->enc_pin_ev, e->stream));
+    e->enc_pin_used = true;
+    if (L0 > n) PTTS_CUDA_CHECK(cudaMemsetAsync(e->eb.pcm + 6 + n, 0, (size_t)(L0 - n) * sizeof(float), e->stream));
+    e->encode((int)T);
+    return (int)T;
+}
+
+int b200_voice_embed_audio(b200_engine* e, const float* pcm, long long n, float* out) {
+    NvtxRange nvtx_range("ptts.voice_embed_audio");
+    const int T = enc_enqueue(e, pcm, n);
+    if (T < 0 || !out) return T;
+    PTTS_CUDA_CHECK(cudaMemcpyAsync(out, e->eb.prompt, (size_t)T * D_MODEL * sizeof(float), cudaMemcpyDeviceToHost, e->stream));
+    PTTS_CUDA_CHECK(cudaStreamSynchronize(e->stream));
+    return T;
+}
+
+int b200_voice_create_from_audio(b200_engine* e, const float* pcm, long long n) {
+    NvtxRange nvtx_range("ptts.voice_create_from_audio");
+    if (e && e->finalized && e->has_enc && pcm && n >= 1 && e->n_voices >= e->cfg.max_voices) return B200_ECAPACITY;
+    const int T = enc_enqueue(e, pcm, n);
+    if (T < 0) return T;
+    const int v = e->n_voices++;
+    const int slot = e->cfg.max_slots + v;
+    std::vector<int> slots(T, slot), pos(T);
+    for (int i = 0; i < T; i++) pos[i] = i;
+    prefill_rows(e, slots, pos, nullptr, nullptr, e->eb.prompt);
     e->voice_len[v] = T;
     return v;
 }
@@ -1917,6 +2113,7 @@ int b200_debug_tap(b200_engine* e, const char* name, int slot, float* out, int m
     e->join_mimi();
     PTTS_CUDA_CHECK(cudaStreamSynchronize(e->stream));
     const std::string s = name;
+    if (s.rfind("enc.", 0) == 0 && e->enc_T == 0) return B200_ENOTFOUND;   // no clone yet
     auto give_f32 = [&](const float* src, size_t n) -> int {
         if (!out) return (int)n;
         if ((size_t)max_elems < n) return B200_EINVAL;
@@ -1950,6 +2147,9 @@ int b200_debug_tap(b200_engine* e, const char* name, int slot, float* out, int m
     if (s == "seanet.res3") return give_16(e->buf5, true, 97LL * e->C5, 1, 96, e->C5, 256);
     if (s == "seanet.res6") return give_16(e->buf8, true, 481LL * e->C8, 1, 480, e->C8, 128);
     if (s == "seanet.res9") return give_16(e->buf11, true, 1922LL * 64, 2, 1920, 64, 64);
+    if (s == "enc.seanet") return give_f32(e->eb.xs, (size_t)e->enc_T * M_T * M_DIM);          // the last clone's buffers (slot ignored)
+    if (s == "enc.transformer") return give_f32(e->eb.xt, (size_t)e->enc_T * M_T * M_DIM);
+    if (s == "enc.downsample") return give_f32(e->eb.lat, (size_t)e->enc_T * M_DIM);
     return B200_ENOTFOUND;
 }
 
@@ -1959,6 +2159,31 @@ int b200_debug_gemm_plan(int R, int N, int K, int num_sms, int want_ln, int* bn,
     if (R < 1 || N < 32 || N % 32 != 0 || K < 64 || K % 64 != 0 || num_sms < 1 || !bn || !splits) return B200_EINVAL;
     const TcPlan p = tc_plan((R + 127) / 128, R, N, K, num_sms, want_ln != 0);
     *bn = p.bn; *splits = p.splits;
+    return B200_OK;
+}
+
+// Test hook: the encoder's window attention (attn_window_kernel) alone over q, k, v [R][512] f32 (rounded to bf16 here; q and k taken as
+// already rotated); out [R][512] = the bf16 output as f32. Synchronises. Needs no encoder weights.
+int b200_debug_window_attention(b200_engine* e, int R, const float* q, const float* k, const float* v, float* out) {
+    if (!e || !e->finalized || R < 1 || !q || !k || !v || !out) return B200_EINVAL;
+    b200_sync(e);                                              // also selects the engine's device
+    const size_t n = (size_t)R * M_DIM;
+    __nv_bfloat16* d = nullptr;
+    PTTS_CUDA_CHECK(cudaMalloc(&d, 4 * n * sizeof(__nv_bfloat16)));
+    const float* src[3] = {q, k, v};
+    for (int i = 0; i < 3; i++) {
+        const std::vector<__nv_bfloat16> b = b200_engine::to_bf16(std::vector<float>(src[i], src[i] + n));
+        PTTS_CUDA_CHECK(cudaMemcpyAsync(d + i * n, b.data(), n * sizeof(__nv_bfloat16), cudaMemcpyHostToDevice, e->stream));
+        PTTS_CUDA_CHECK(cudaStreamSynchronize(e->stream));
+    }
+    launch_k(false, attn_window_kernel, dim3((R + AW_Q - 1) / AW_Q, M_HEADS), dim3(AW_WARPS * 32), AW_SMEM, e->stream, (const __nv_bfloat16*)d,
+             (const __nv_bfloat16*)(d + n), (const __nv_bfloat16*)(d + 2 * n), R, d + 3 * n);
+    e->launches++;
+    std::vector<uint16_t> tmp(n);
+    PTTS_CUDA_CHECK(cudaMemcpyAsync(tmp.data(), d + 3 * n, n * sizeof(uint16_t), cudaMemcpyDeviceToHost, e->stream));
+    PTTS_CUDA_CHECK(cudaStreamSynchronize(e->stream));
+    PTTS_CUDA_CHECK(cudaFree(d));
+    for (size_t i = 0; i < n; i++) { const uint32_t u = (uint32_t)tmp[i] << 16; memcpy(&out[i], &u, 4); }
     return B200_OK;
 }
 

@@ -50,8 +50,8 @@ __device__ __forceinline__ void epi_apply(const Epi& e, int row, int col0, const
     //      Mimi: modules/mimi_transformer.h:586-712, rope.h:86-181) ----
     const bool mimi = (e.mode == EPI_MIMI_QKV);
     const int D = mimi ? M_DIM : D_MODEL;
-    const int slot = e.row_slot[row];
-    const int pos = e.row_pos[row];
+    const int slot = e.kv_linear ? 0 : e.row_slot[row];
+    const int pos = e.kv_linear ? row : e.row_pos[row];
     if (slot < 0) return;                 // dead row (finished utterance): nothing is appended or handed on
 #pragma unroll
     for (int p = 0; p < NV; p += 2) {
@@ -71,12 +71,12 @@ __device__ __forceinline__ void epi_apply(const Epi& e, int row, int col0, const
                 if (mimi) { e.q_out_bf16[(long long)row * D + i_re] = __float2bfloat16_rn(re); e.q_out_bf16[(long long)row * D + i_im] = __float2bfloat16_rn(im); }
                 else      { e.q_out_f32[(long long)row * D + i_re] = re; e.q_out_f32[(long long)row * D + i_im] = im; }
             } else {
-                const long long base = (long long)slot * e.kv_slot_stride + (long long)(mimi ? pos % M_CTX : pos) * D;
+                const long long base = (long long)slot * e.kv_slot_stride + (long long)(mimi && !e.kv_linear ? pos % M_CTX : pos) * D;
                 if (!mimi && e.kv_f32) { ((float*)e.kcache)[base + i_re] = re; ((float*)e.kcache)[base + i_im] = im; }
                 else { ((__nv_bfloat16*)e.kcache)[base + i_re] = __float2bfloat16_rn(re); ((__nv_bfloat16*)e.kcache)[base + i_im] = __float2bfloat16_rn(im); }
             }
         } else {
-            const long long base = (long long)slot * e.kv_slot_stride + (long long)(mimi ? pos % M_CTX : pos) * D + c;
+            const long long base = (long long)slot * e.kv_slot_stride + (long long)(mimi && !e.kv_linear ? pos % M_CTX : pos) * D + c;
             if (!mimi && e.kv_f32) { ((float*)e.vcache)[base] = a; ((float*)e.vcache)[base + 1] = b; }
             else { ((__nv_bfloat16*)e.vcache)[base] = __float2bfloat16_rn(a); ((__nv_bfloat16*)e.vcache)[base + 1] = __float2bfloat16_rn(b); }
         }

@@ -330,9 +330,9 @@ __device__ __forceinline__ void epi_qkv32(const Epi& e, int row, int col0, float
         for (int i = 0; i < 32; i++) v[i] += e.bias[col0 + i];
     }
     const int part = col0 / D, c = col0 - part * D;
-    const int slot = e.row_slot[row], pos = e.row_pos[row];
+    const int slot = e.kv_linear ? 0 : e.row_slot[row], pos = e.kv_linear ? row : e.row_pos[row];
     if (slot < 0) return;                                       // dead row (finished utterance): nothing is appended or handed on
-    const long long cbase = (long long)slot * e.kv_slot_stride + (long long)(mimi ? pos % M_CTX : pos) * D;
+    const long long cbase = (long long)slot * e.kv_slot_stride + (long long)(mimi && !e.kv_linear ? pos % M_CTX : pos) * D;
     if (part == 2) {
         if (!mimi && e.kv_f32) {
             float4* g = reinterpret_cast<float4*>((float*)e.vcache + cbase + c);

@@ -69,13 +69,72 @@ const char* kVoices[] = {"alba", "azelma", "cosette", "eponine", "fantine", "jav
 
 int env_int(const char* name, int dflt) { const char* v = getenv(name); return v && *v ? atoi(v) : dflt; }
 
+bool ends_with(const std::string& s, const char* suffix) { const size_t n = strlen(suffix); return s.size() >= n && s.compare(s.size() - n, n, suffix) == 0; }
+
+// RIFF/WAVE reader: PCM16 or float32 (format 1 / 3, or WAVE_FORMAT_EXTENSIBLE with either subformat), any channel count, mixed down
+// to mono by averaging. Returns false for anything else, including a data chunk that runs past the end of the file.
+bool read_wav(const std::string& path, std::vector<float>& out, int& sample_rate) {
+    FILE* f = fopen(path.c_str(), "rb");
+    if (!f) return false;
+    std::vector<uint8_t> b;
+    uint8_t buf[65536]; size_t got;
+    while ((got = fread(buf, 1, sizeof buf, f)) > 0) b.insert(b.end(), buf, buf + got);
+    fclose(f);
+    auto u16 = [&](size_t o) { return (uint32_t)b[o] | ((uint32_t)b[o + 1] << 8); };
+    auto u32 = [&](size_t o) { return u16(o) | (u16(o + 2) << 16); };
+    if (b.size() < 12 || memcmp(b.data(), "RIFF", 4) != 0 || memcmp(b.data() + 8, "WAVE", 4) != 0) return false;
+    int fmt = -1, channels = 0, bits = 0; bool have_fmt = false;
+    for (size_t o = 12; o + 8 <= b.size();) {
+        const uint32_t sz = u32(o + 4);
+        const size_t body = o + 8;
+        if ((uint64_t)body + sz > b.size()) return false;                        // truncated chunk
+        if (memcmp(b.data() + o, "fmt ", 4) == 0) {
+            if (sz < 16) return false;
+            fmt = (int)u16(body); channels = (int)u16(body + 2); sample_rate = (int)u32(body + 4); bits = (int)u16(body + 14);
+            if (fmt == 0xFFFE) { if (sz < 26) return false; fmt = (int)u16(body + 24); }   // extensible: the subformat GUID starts with the format tag
+            have_fmt = true;
+        } else if (memcmp(b.data() + o, "data", 4) == 0) {
+            if (!have_fmt || channels < 1) return false;
+            const bool pcm16 = fmt == 1 && bits == 16, f32 = fmt == 3 && bits == 32;
+            if (!pcm16 && !f32) return false;
+            const size_t frame_bytes = (size_t)channels * (bits / 8), n = sz / frame_bytes;
+            out.assign(n, 0.f);
+            for (size_t i = 0; i < n; i++) {
+                double acc = 0;
+                for (int c = 0; c < channels; c++) {
+                    const size_t at = body + i * frame_bytes + (size_t)c * (bits / 8);
+                    if (pcm16) acc += (int16_t)u16(at) / 32768.0;
+                    else { float v; memcpy(&v, b.data() + at, 4); acc += v; }
+                }
+                out[i] = (float)(acc / channels);
+            }
+            return true;
+        }
+        o = body + sz + (sz & 1);                                                // chunks are padded to even sizes
+    }
+    return false;
+}
+
+// audio_prompt [1, T, 1024] F32, the layout of a voice file
+bool write_voice_file(const std::string& path, const std::vector<float>& prompt) {
+    const size_t T = prompt.size() / 1024;
+    std::string h = "{\"audio_prompt\":{\"dtype\":\"F32\",\"shape\":[1," + std::to_string(T) + ",1024],\"data_offsets\":[0," + std::to_string(prompt.size() * 4) + "]}}";
+    while (h.size() % 8) h += ' ';
+    FILE* f = fopen(path.c_str(), "wb");
+    if (!f) return false;
+    const uint64_t hl = h.size();
+    bool ok = fwrite(&hl, 8, 1, f) == 1 && fwrite(h.data(), 1, h.size(), f) == h.size() && fwrite(prompt.data(), 4, prompt.size(), f) == prompt.size();
+    return fclose(f) == 0 && ok;
+}
+
 }  // namespace
 
 struct ptts_context_t {
     b200_engine* engine = nullptr;
     std::string model_path;
     SpmUnigram tokenizer;
-    std::map<std::string, int> voices;      // resolved voice file -> engine voice id
+    std::map<std::string, int> voices;      // resolved voice file or registered name -> engine voice id
+    std::map<std::string, std::vector<float>> cloned;   // voices created from audio: their audio_prompt rows [T][1024] (for export)
     std::vector<bool> slot_used;
     int n_streams = 0;
     bool lookahead = true;                  // PTTS_B200_LOOKAHEAD=0: strictly one step per receive
@@ -143,14 +202,35 @@ ptts_context_t* ptts_init(ggml_backend*, ggml_backend*, const char* model_path) 
 int ptts_get_sample_rate(ptts_context_t*) { return 24000; }   // reference :324-326
 int ptts_get_frame_size(ptts_context_t*) { return 1920; }     // reference :328-330
 
+// Clones a voice from mono 24 kHz PCM and registers it under `name`. The rows come back to the host once, so that the voice can be exported.
+static int add_audio_voice(ptts_context_t* ctx, const std::string& name, const float* pcm, long long n) {
+    const long long T = (n + 1919) / 1920;
+    if (n < 1 || T > b200_kv_capacity(ctx->engine)) return n < 1 ? B200_EINVAL : B200_ECAPACITY;
+    std::vector<float> prompt((size_t)T * 1024);
+    const int t = b200_voice_embed_audio(ctx->engine, pcm, n, prompt.data());
+    if (t < 0) return t;
+    const int vid = b200_voice_create(ctx->engine, prompt.data(), t);
+    if (vid < 0) return vid;
+    ctx->voices[name] = vid;
+    ctx->cloned[name] = std::move(prompt);
+    return vid;
+}
+
 // Voice name or path -> engine voice id; the first use loads the file and prefills the prefix (reference src/pocket_tts.cpp:356-359,100-124).
+// A path ending in ".wav" is a recording: it is cloned (add_audio_voice).
 static int resolve_voice(ptts_context_t* ctx, const char* voice_c_str) {
     std::string voice = voice_c_str;
     for (const char* v : kVoices) if (voice == v) { voice = ctx->model_path + "embeddings/" + v + ".safetensors"; break; }
     int vid;
     auto it = ctx->voices.find(voice);
     if (it != ctx->voices.end()) vid = it->second;
-    else {
+    else if (ends_with(voice, ".wav")) {
+        std::vector<float> pcm; int rate = 0;
+        if (!read_wav(voice, pcm, rate)) { fprintf(stderr, "error: failed to open voice %s\n", voice.c_str()); exit(1); }
+        if (rate != 24000) { fprintf(stderr, "error: voice %s: sample rate %d Hz, the encoder takes 24000 Hz\n", voice.c_str(), rate); exit(1); }
+        vid = add_audio_voice(ctx, voice, pcm.data(), (long long)pcm.size());
+        if (vid < 0) { fprintf(stderr, "error: failed to clone voice %s (%d)\n", voice.c_str(), vid); exit(1); }
+    } else {
         SafeTensors st;
         if (!st.open(voice)) { fprintf(stderr, "error: failed to open voice %s\n", voice.c_str()); exit(1); }
         auto e = st.entries.find("audio_prompt");
@@ -277,6 +357,25 @@ int ptts_c_tokenize(ptts_context_t* c, const char* text, int32_t* ids, int max_i
     return (int)v.size();
 }
 int ptts_c_count_words(const char* text) { return count_words_impl(text); }
+int ptts_c_voice_add_audio(ptts_context_t* c, const char* name, const float* pcm, long long n, int sample_rate) {
+    if (!c || !name || !pcm || sample_rate != 24000 || c->voices.count(name)) return B200_EINVAL;
+    for (const char* v : kVoices) if (strcmp(name, v) == 0) return B200_EINVAL;   // resolve_voice maps these to the model's voice files first
+    if (!b200_has_encoder(c->engine)) return B200_ENOTFOUND;
+    return add_audio_voice(c, name, pcm, n);
+}
+int ptts_c_voice_export(ptts_context_t* c, const char* name, const char* path) {
+    if (!c || !name || !path) return B200_EINVAL;
+    auto it = c->cloned.find(name);
+    if (it == c->cloned.end()) return B200_ENOTFOUND;
+    return write_voice_file(path, it->second) ? B200_OK : B200_EINVAL;
+}
+int ptts_c_wav_read(const char* path, float* pcm, long long max, int* sample_rate) {
+    std::vector<float> v; int rate = 0;
+    if (!path || !read_wav(path, v, rate)) return B200_EINVAL;
+    if (pcm) memcpy(pcm, v.data(), (size_t)std::min<long long>(std::max<long long>(max, 0), (long long)v.size()) * sizeof(float));
+    if (sample_rate) *sample_rate = rate;
+    return (int)v.size();
+}
 int ptts_c_stream_pending(ptts_stream_t* s, int index, char* buf, int buflen) {
     const int n = (int)s->sproc.sentences.size();
     if (index >= 0 && index < n && buf && buflen > 0) {

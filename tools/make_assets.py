@@ -202,6 +202,39 @@ def synth_weights(seed: int, eos_mode: str) -> dict[str, np.ndarray]:
     return W
 
 
+def synth_encoder_weights(seed: int) -> dict[str, np.ndarray]:
+    """The voice-cloning encoder set (DESIGN.md §4.6), drawn from its own generator so that the decoder-side stream is unchanged."""
+    rng = np.random.default_rng([seed, 0xE1C])
+    W: dict[str, np.ndarray] = {}
+
+    def conv(name, co, ci, k, bias=True):
+        W[name + ".conv.weight"] = (rng.standard_normal((co, ci, k)) / np.sqrt(ci * k)).astype(np.float32)
+        if bias:
+            W[name + ".conv.bias"] = (0.02 * rng.standard_normal(co)).astype(np.float32)
+
+    e = "mimi.encoder.model."
+    conv(e + "0", 64, 1, 7)
+    for i, c in ((1, 64), (4, 128), (7, 256)):
+        conv(e + f"{i}.block.1", c // 2, c, 3)
+        conv(e + f"{i}.block.3", c, c // 2, 1)
+    conv(e + "3", 128, 64, 8)
+    conv(e + "6", 256, 128, 10)
+    conv(e + "9", 512, 256, 12)
+    conv(e + "11", 512, 512, 3)
+    for l in range(2):
+        p = f"mimi.encoder_transformer.transformer.layers.{l}."
+        for n in ("norm1", "norm2"):
+            W[p + n + ".weight"] = (1.0 + 0.02 * rng.standard_normal(512)).astype(np.float32)
+            W[p + n + ".bias"] = (0.02 * rng.standard_normal(512)).astype(np.float32)
+        for n, o, i in (("self_attn.in_proj", 1536, 512), ("self_attn.out_proj", 512, 512), ("linear1", 2048, 512), ("linear2", 512, 2048)):
+            W[p + n + ".weight"] = (rng.standard_normal((o, i)) / np.sqrt(i)).astype(np.float32)
+        W[p + "layer_scale_1.scale"] = (0.1 + 0.01 * rng.standard_normal(512)).astype(np.float32)
+        W[p + "layer_scale_2.scale"] = (0.1 + 0.01 * rng.standard_normal(512)).astype(np.float32)
+    conv("mimi.downsample.conv", 512, 512, 32, bias=False)
+    W["flow_lm.speaker_proj_weight"] = (rng.standard_normal((1024, 512)) / np.sqrt(512)).astype(np.float32)
+    return W
+
+
 def synth_voice(name: str, seed: int, t_voice: int) -> np.ndarray:
     h = sum((i + 1) * ord(c) for i, c in enumerate(name))
     rng = np.random.default_rng(seed * 1000003 + h)
@@ -287,11 +320,14 @@ def train_tokenizer(out_model: str) -> None:
 
 # ----------------------------------------------------------------------------------
 def make_model_dir(out_dir: str, seed: int = 1234, dtype: str = "BF16", eos_mode: str = "never",
-                   t_voice: int = 125, voices=None, force: bool = False) -> str:
-    """Creates (or reuses) the model directory; returns its path WITH trailing '/' (the reference concatenates)."""
+                   t_voice: int = 125, voices=None, force: bool = False, encoder: bool = False) -> str:
+    """Creates (or reuses) the model directory; returns its path WITH trailing '/' (the reference concatenates).
+    encoder=True adds the voice-cloning encoder tensors (every other tensor stays bitwise the same)."""
     out_dir = os.path.abspath(out_dir)
     stamp = os.path.join(out_dir, "STAMP.json")
     want = {"seed": seed, "dtype": dtype, "eos_mode": eos_mode, "t_voice": t_voice, "version": 4}
+    if encoder:
+        want["encoder"] = 1
     if not force and os.path.exists(stamp):
         try:
             if json.load(open(stamp)) == want:
@@ -299,7 +335,10 @@ def make_model_dir(out_dir: str, seed: int = 1234, dtype: str = "BF16", eos_mode
         except Exception:
             pass
     os.makedirs(os.path.join(out_dir, "embeddings"), exist_ok=True)
-    write_safetensors(os.path.join(out_dir, "tts_b6369a24.safetensors"), synth_weights(seed, eos_mode), dtype)
+    weights = synth_weights(seed, eos_mode)
+    if encoder:
+        weights.update(synth_encoder_weights(seed))
+    write_safetensors(os.path.join(out_dir, "tts_b6369a24.safetensors"), weights, dtype)
     for v in (voices or VOICES):
         # Voice prompts are always written F32: with a BF16 prompt tensor the reference's residual adds
         # (ggml_add keeps src0's type) would silently run the whole voice prefill in a bf16 residual stream
@@ -313,11 +352,12 @@ def make_model_dir(out_dir: str, seed: int = 1234, dtype: str = "BF16", eos_mode
     return out_dir + "/"
 
 
-def default_model_dir(eos_mode: str = "never", dtype: str = "BF16", t_voice: int = 125, seed: int = 1234, voices=None) -> str:
+def default_model_dir(eos_mode: str = "never", dtype: str = "BF16", t_voice: int = 125, seed: int = 1234, voices=None, encoder: bool = False) -> str:
     # a cache outside the tree (which may be read-only), one per user: another user's directory on a shared machine is not writable
     root = os.environ.get("PTTS_B200_ASSETS") or os.path.join(tempfile.gettempdir(), f"ptts_b200_assets_{os.getuid()}")
     name = f"model_s{seed}_{dtype.lower()}_{eos_mode + ('7' if eos_mode == 'late' else '')}_v{t_voice}" + ("" if voices is None else "_" + "-".join(voices))
-    return make_model_dir(os.path.join(root, name), seed=seed, dtype=dtype, eos_mode=eos_mode, t_voice=t_voice, voices=voices)
+    name += "_enc" if encoder else ""
+    return make_model_dir(os.path.join(root, name), seed=seed, dtype=dtype, eos_mode=eos_mode, t_voice=t_voice, voices=voices, encoder=encoder)
 
 
 if __name__ == "__main__":
