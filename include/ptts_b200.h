@@ -90,6 +90,21 @@ B200_API int  b200_begin_sentences(b200_engine* e, int n, const int32_t* slots, 
 B200_API int  b200_begin_sentences_ex(b200_engine* e, int n, const int32_t* slots, const int32_t* voices, const int32_t* tokens,
                                       const int32_t* tok_off, const int32_t* max_gen_len, const int32_t* frames_after_eos,
                                       const float* temp, const uint32_t* rng_stream);
+/* Per-sentence sampling controls (DESIGN.md 4.7), the knobs upstream Pocket TTS exposes per request:
+ *   lsd_steps      LSD decode steps N, 1..8: x_{i+1} = x_i + v(c, i/N, (i+1)/N, x_i) / N from x_0 = noise (1 = the single-step head)
+ *   noise_clamp    a >= 0: noise drawn from N(0, temp) truncated to [-a, a] (absolute bounds, torch trunc_normal_); 0 = untruncated.
+ *                  Injected noise (b200_step's `noise`) is used as given.
+ *   eos_threshold  EOS fires when the EOS logit > eos_threshold (the reported eos_logit stays logit + 4); finite
+ * b200_default_sampling fills {1, 0, -4}: a sentence with these values runs exactly the step it runs without sampling controls. */
+#define B200_LSD_MAX_STEPS 8
+typedef struct b200_sampling { int lsd_steps; float noise_clamp; float eos_threshold; } b200_sampling;
+B200_API void b200_default_sampling(b200_sampling* s);
+/* B200_OK, or B200_EINVAL for NULL, lsd_steps outside 1..8, a negative or non-finite clamp, or a non-finite threshold. */
+B200_API int  b200_sampling_check(const b200_sampling* s);
+/* b200_begin_sentences_ex plus sampling[n] (NULL = defaults for every sentence). B200_EINVAL when any entry fails b200_sampling_check. */
+B200_API int  b200_begin_sentences_sampling(b200_engine* e, int n, const int32_t* slots, const int32_t* voices, const int32_t* tokens,
+                                            const int32_t* tok_off, const int32_t* max_gen_len, const int32_t* frames_after_eos,
+                                            const float* temp, const uint32_t* rng_stream, const b200_sampling* sampling);
 /* Stream-ordered: the sentences in `slots` end now. From the next enqueued step on these slots are dead rows (no KV append, no attention,
  * produced = 0) until a sentence start reuses them. Steps already enqueued are unaffected. Nothing in this call waits on the host. */
 B200_API int  b200_end_sentences(b200_engine* e, int n, const int32_t* slots);
@@ -207,6 +222,8 @@ B200_API void ptts_c_stream_reset(ptts_stream_t* s);
 B200_API void ptts_c_stream_flush(ptts_stream_t* s);
 B200_API void ptts_c_stream_send(ptts_stream_t* s, const char* chunk);
 B200_API int ptts_c_stream_receive(ptts_stream_t* s, float* samples);
+/* Sampling controls of the stream's sentences from the next sentence start on (B200_EINVAL: NULL or out of range, see b200_sampling_check). */
+B200_API int ptts_c_stream_set_sampling(ptts_stream_t* s, const b200_sampling* sampling);
 B200_API b200_engine* ptts_c_engine(ptts_context_t* ctx);
 B200_API void ptts_c_destroy(ptts_context_t* ctx);   /* frees the engine and the context (the reference API never frees, src/pocket_tts.cpp:313) */
 /* Text front end, exposed for bit-exactness tests (conditioners/text.h:21-27,81-94). */
@@ -241,6 +258,13 @@ B200_API int  ptts_c_batch_add_tokens(ptts_batch_t* b, int voice_id, const int32
  * themselves); returns utt. B200_EINVAL for a cancelled utterance. */
 B200_API int  ptts_c_batch_append_tokens(ptts_batch_t* b, int utt, int voice_id, const int32_t* ids, int n_ids, int max_gen_len, int frames_after_eos,
                                          float temp, uint32_t rng_stream);
+/* The same three with per-sentence sampling controls (NULL = defaults; B200_EINVAL when b200_sampling_check fails). The scheduler hands the
+ * struct to the engine's sentence start unchanged. */
+B200_API int  ptts_c_batch_add_sampling(ptts_batch_t* b, const char* voice, const char* text, float temp, const b200_sampling* sampling);
+B200_API int  ptts_c_batch_add_tokens_sampling(ptts_batch_t* b, int voice_id, const int32_t* ids, int n_ids, int max_gen_len, int frames_after_eos,
+                                               float temp, uint32_t rng_stream, const b200_sampling* sampling);
+B200_API int  ptts_c_batch_append_tokens_sampling(ptts_batch_t* b, int utt, int voice_id, const int32_t* ids, int n_ids, int max_gen_len,
+                                                  int frames_after_eos, float temp, uint32_t rng_stream, const b200_sampling* sampling);
 B200_API long long ptts_c_batch_run(ptts_batch_t* b);                  /* runs every queued sentence to completion; frames produced */
 B200_API int  ptts_c_batch_frames(ptts_batch_t* b, int utt);           /* frames generated for the utterance so far (popped ones included) */
 B200_API int  ptts_c_batch_read(ptts_batch_t* b, int utt, float* pcm, int max_frames);   /* [n][1920]: the frames not popped yet */
@@ -269,6 +293,12 @@ B200_API ptts_batch_t* ptts_c_batch_create_with_ops(void* user, ptts_batch_begin
 typedef int (*ptts_batch_end_fn)(void* user, int n, const int32_t* slots);
 B200_API ptts_batch_t* ptts_c_batch_create_with_ops_ex(void* user, ptts_batch_begin_fn begin, ptts_batch_submit_fn submit, ptts_batch_collect_fn collect,
                                                        ptts_batch_end_fn end, int n_slots, int frame_size);
+/* begin with each sentence's sampling controls (b200_begin_sentences_sampling's signature minus the engine) */
+typedef int (*ptts_batch_begin_sampling_fn)(void* user, int n, const int32_t* slots, const int32_t* voices, const int32_t* tokens, const int32_t* tok_off,
+                                            const int32_t* max_gen_len, const int32_t* frames_after_eos, const float* temp, const uint32_t* rng_stream,
+                                            const b200_sampling* sampling);
+B200_API ptts_batch_t* ptts_c_batch_create_with_ops_sampling(void* user, ptts_batch_begin_sampling_fn begin, ptts_batch_submit_fn submit,
+                                                             ptts_batch_collect_fn collect, ptts_batch_end_fn end, int n_slots, int frame_size);
 
 /* Host-only text front end (no GPU needed): tokenizer + sentence splitter objects. */
 typedef struct ptts_text_t ptts_text_t;

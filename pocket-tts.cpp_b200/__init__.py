@@ -43,8 +43,21 @@ class BatchStats(ctypes.Structure):
                 ("refills", ctypes.c_longlong), ("wall_ms", ctypes.c_double), ("begin_ms", ctypes.c_double), ("submit_ms", ctypes.c_double), ("collect_ms", ctypes.c_double)]
 
 
+class Sampling(ctypes.Structure):
+    """b200_sampling: per-sentence LSD decode steps (1..8), noise clamp (0 = off, absolute bound) and EOS threshold (DESIGN.md 4.7)."""
+    _fields_ = [("lsd_steps", ctypes.c_int), ("noise_clamp", ctypes.c_float), ("eos_threshold", ctypes.c_float)]
+
+    def __init__(self, lsd_steps=1, noise_clamp=0.0, eos_threshold=-4.0):
+        super().__init__(int(lsd_steps), float(noise_clamp), float(eos_threshold))
+
+    def astuple(self):
+        return (self.lsd_steps, self.noise_clamp, self.eos_threshold)
+
+
 _I32P, _F32P, _U32P = ctypes.POINTER(ctypes.c_int32), ctypes.POINTER(ctypes.c_float), ctypes.POINTER(ctypes.c_uint32)
+_SAMPP = ctypes.POINTER(Sampling)
 BATCH_BEGIN_FN = ctypes.CFUNCTYPE(ctypes.c_int, ctypes.c_void_p, ctypes.c_int, _I32P, _I32P, _I32P, _I32P, _I32P, _I32P, _F32P, _U32P)
+BATCH_BEGIN_SAMPLING_FN = ctypes.CFUNCTYPE(ctypes.c_int, ctypes.c_void_p, ctypes.c_int, _I32P, _I32P, _I32P, _I32P, _I32P, _I32P, _F32P, _U32P, _SAMPP)
 BATCH_SUBMIT_FN = ctypes.CFUNCTYPE(ctypes.c_int, ctypes.c_void_p, ctypes.c_int, ctypes.c_int)
 BATCH_COLLECT_FN = ctypes.CFUNCTYPE(ctypes.c_int, ctypes.c_void_p, _F32P, _I32P)
 BATCH_END_FN = ctypes.CFUNCTYPE(ctypes.c_int, ctypes.c_void_p, ctypes.c_int, _I32P)
@@ -129,6 +142,14 @@ def lib():
         "ptts_c_stream_pending": (ci, [vp, ci, cp, ci]),
         "b200_begin_sentences_ex": (ci, [vp, ci, ip, ip, ip, ip, ip, ip, fp, ctypes.POINTER(ctypes.c_uint32)]),
         "b200_end_sentences": (ci, [vp, ci, ip]),
+        "b200_default_sampling": (None, [_SAMPP]),
+        "b200_sampling_check": (ci, [_SAMPP]),
+        "b200_begin_sentences_sampling": (ci, [vp, ci, ip, ip, ip, ip, ip, ip, fp, ctypes.POINTER(ctypes.c_uint32), _SAMPP]),
+        "ptts_c_stream_set_sampling": (ci, [vp, _SAMPP]),
+        "ptts_c_batch_add_sampling": (ci, [vp, cp, cp, cf, _SAMPP]),
+        "ptts_c_batch_add_tokens_sampling": (ci, [vp, ci, ip, ci, ci, ci, cf, ctypes.c_uint32, _SAMPP]),
+        "ptts_c_batch_append_tokens_sampling": (ci, [vp, ci, ci, ip, ci, ci, ci, cf, ctypes.c_uint32, _SAMPP]),
+        "ptts_c_batch_create_with_ops_sampling": (vp, [vp, BATCH_BEGIN_SAMPLING_FN, BATCH_SUBMIT_FN, BATCH_COLLECT_FN, BATCH_END_FN, ci, ci]),
         "b200_voice_len": (ci, [vp, ci]),
         "b200_kv_capacity": (ci, [vp]),
         "b200_max_slots": (ci, [vp]),
@@ -248,14 +269,20 @@ class Engine:
         if rc != 0:
             raise RuntimeError(f"b200_begin_sentence failed: {rc}")
 
-    def begin_sentences(self, slots, voices, token_lists, max_gen_len, frames_after_eos, temps, rng_streams=None):
+    def begin_sentences(self, slots, voices, token_lists, max_gen_len, frames_after_eos, temps, rng_streams=None, sampling=None):
+        """sampling: None, or one Sampling / (lsd_steps, noise_clamp, eos_threshold) per sentence (b200_begin_sentences_sampling)."""
         n = len(slots)
         off = np.zeros(n + 1, np.int32)
         off[1:] = np.cumsum([len(t) for t in token_lists])
         toks = np.ascontiguousarray(np.concatenate([np.asarray(t, np.int32) for t in token_lists]) if n else np.zeros(0, np.int32), np.int32)
         a = [np.ascontiguousarray(x, np.int32) for x in (slots, voices, max_gen_len, frames_after_eos)]
         tp = np.ascontiguousarray(temps, np.float32)
-        if rng_streams is not None:
+        if sampling is not None:
+            sa = (Sampling * max(n, 1))(*[s if isinstance(s, Sampling) else Sampling(*s) for s in sampling])
+            rs = np.ascontiguousarray(rng_streams, np.uint32) if rng_streams is not None else None
+            rc = self.L.b200_begin_sentences_sampling(self.h, n, _ip(a[0]), _ip(a[1]), _ip(toks), _ip(off), _ip(a[2]), _ip(a[3]), _fp(tp),
+                                                      rs.ctypes.data_as(_U32P) if rs is not None else None, sa)
+        elif rng_streams is not None:
             rs = np.ascontiguousarray(rng_streams, np.uint32)
             rc = self.L.b200_begin_sentences_ex(self.h, n, _ip(a[0]), _ip(a[1]), _ip(toks), _ip(off), _ip(a[2]), _ip(a[3]), _fp(tp), rs.ctypes.data_as(_U32P))
         else:
@@ -480,8 +507,10 @@ class Context:
         n = lib().ptts_c_tokenize(self.h, text.encode(), buf, 8192)
         return list(buf[:n])
 
-    def stream(self, voice="cosette", temp=0.7) -> "Stream":
-        return Stream(self, voice, temp)
+    def stream(self, voice="cosette", temp=0.7, lsd_steps=1, noise_clamp=0.0, eos_threshold=-4.0) -> "Stream":
+        s = Stream(self, voice, temp)
+        s.set_sampling(lsd_steps, noise_clamp, eos_threshold)
+        return s
 
     def add_voice(self, name: str, pcm, sample_rate: int = SAMPLE_RATE) -> int:
         """Clones a voice from mono PCM (24 kHz only) and registers it under `name`; returns the engine voice id."""
@@ -502,14 +531,19 @@ class Batch:
     """Continuous batching over the engine's slots (ptts_c_batch_*): queue utterances, run() generates all of them, finished slots are
     refilled with queued sentences. For online serving, add() at any time, pump() a few steps, pop() each utterance's ready frames in order
     and cancel() the ones nobody waits for. With `ops` = (begin, submit, collect[, end]) Python callables the scheduler runs over a mock
-    engine (CPU tests)."""
+    engine (CPU tests); with begin_sampling=True the begin callable also receives each sentence's b200_sampling array.
+    add() / add_tokens() take the per-sentence sampling controls lsd_steps, noise_clamp and eos_threshold (DESIGN.md 4.7)."""
 
     STATES = ("queued", "running", "done", "cancelled")
 
-    def __init__(self, ctx: "Context" = None, n_slots: int = 0, ops=None, frame_size: int = FRAME):
+    def __init__(self, ctx: "Context" = None, n_slots: int = 0, ops=None, frame_size: int = FRAME, begin_sampling: bool = False):
         L = lib()
         self.frame_size, self.ctx = frame_size, ctx
-        if ops is not None:
+        if ops is not None and begin_sampling:
+            end = BATCH_END_FN(ops[3]) if len(ops) > 3 and ops[3] is not None else BATCH_END_FN()
+            self._cbs = (BATCH_BEGIN_SAMPLING_FN(ops[0]), BATCH_SUBMIT_FN(ops[1]), BATCH_COLLECT_FN(ops[2]), end)
+            self.h = L.ptts_c_batch_create_with_ops_sampling(None, *self._cbs, n_slots, frame_size)
+        elif ops is not None:
             end = BATCH_END_FN(ops[3]) if len(ops) > 3 and ops[3] is not None else BATCH_END_FN()
             self._cbs = (BATCH_BEGIN_FN(ops[0]), BATCH_SUBMIT_FN(ops[1]), BATCH_COLLECT_FN(ops[2]), end)   # keep the thunks alive
             self.h = L.ptts_c_batch_create_with_ops_ex(None, *self._cbs, n_slots, frame_size)
@@ -521,19 +555,24 @@ class Batch:
     def configure(self, refill_min=0, refill_every=0, range_quantum=0, keep_pcm=-1):
         assert lib().ptts_c_batch_configure(self.h, refill_min, refill_every, range_quantum, keep_pcm) == 0
 
-    def add(self, voice: str, text: str, temp: float = 0.7) -> int:
-        u = lib().ptts_c_batch_add(self.h, voice.encode(), text.encode(), float(temp))
+    def add(self, voice: str, text: str, temp: float = 0.7, lsd_steps: int = 1, noise_clamp: float = 0.0, eos_threshold: float = -4.0) -> int:
+        sp = Sampling(lsd_steps, noise_clamp, eos_threshold)
+        u = lib().ptts_c_batch_add_sampling(self.h, voice.encode(), text.encode(), float(temp), ctypes.byref(sp))
         if u < 0:
             raise RuntimeError(f"ptts_c_batch_add failed: {u}")
         return u
 
-    def add_tokens(self, voice_id, ids, max_gen_len, frames_after_eos, temp=0.7, rng_stream=0, utt=None) -> int:
+    def add_tokens(self, voice_id, ids, max_gen_len, frames_after_eos, temp=0.7, rng_stream=0, utt=None, lsd_steps=1, noise_clamp=0.0,
+                   eos_threshold=-4.0) -> int:
         """One sentence given as token ids: a new utterance, or the next sentence of utterance `utt`."""
         a = np.ascontiguousarray(ids, np.int32)
+        sp = Sampling(lsd_steps, noise_clamp, eos_threshold)
         if utt is None:
-            u = lib().ptts_c_batch_add_tokens(self.h, voice_id, _ip(a), len(a), max_gen_len, frames_after_eos, float(temp), rng_stream)
+            u = lib().ptts_c_batch_add_tokens_sampling(self.h, voice_id, _ip(a), len(a), max_gen_len, frames_after_eos, float(temp), rng_stream,
+                                                       ctypes.byref(sp))
         else:
-            u = lib().ptts_c_batch_append_tokens(self.h, utt, voice_id, _ip(a), len(a), max_gen_len, frames_after_eos, float(temp), rng_stream)
+            u = lib().ptts_c_batch_append_tokens_sampling(self.h, utt, voice_id, _ip(a), len(a), max_gen_len, frames_after_eos, float(temp),
+                                                          rng_stream, ctypes.byref(sp))
         if u < 0:
             raise RuntimeError(f"ptts_c_batch_add_tokens failed: {u}")
         return u
@@ -606,6 +645,13 @@ class Stream:
         self.h = lib().ptts_c_stream_from_safetensors(ctx.h, voice.encode(), float(temp))
         self.slot = lib().ptts_c_slot(self.h)
         self.voice = lib().ptts_c_voice(self.h)
+
+    def set_sampling(self, lsd_steps=1, noise_clamp=0.0, eos_threshold=-4.0):
+        """Sampling controls (DESIGN.md 4.7) of this stream's sentences from the next sentence start on."""
+        sp = Sampling(lsd_steps, noise_clamp, eos_threshold)
+        rc = lib().ptts_c_stream_set_sampling(self.h, ctypes.byref(sp))
+        if rc != 0:
+            raise ValueError(f"ptts_c_stream_set_sampling: invalid sampling controls {sp.astuple()}")
 
     def reset(self):
         lib().ptts_c_stream_reset(self.h)

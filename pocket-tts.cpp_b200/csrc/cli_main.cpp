@@ -5,6 +5,7 @@
 // rate, :454,517-520) with the same defaults (bench sentence, seed 0, temperature 0, :229-236). Audio goes to a 16-bit PCM WAV
 // file with -o (the reference encodes through FFmpeg or plays through SDL; neither belongs to the generation path).
 #include "../../include/pocket_tts/pocket_tts.h"
+#include "../../include/ptts_b200.h"
 
 #include <chrono>
 #include <cmath>
@@ -28,6 +29,9 @@ void usage(const char* prog) {
             "  -i FILE,  --input FILE        read the text from a file\n"
             "  -s N,     --seed N            RNG seed\n"
             "  -t T,     --temperature T     sampling temperature (default 0.7)\n"
+            "            --lsd-decode-steps N  LSD decode steps of the flow head, 1..8 (default 1)\n"
+            "            --noise-clamp A     truncate the sampling noise to [-A, A] (default 0 = off)\n"
+            "            --eos-threshold T   end of speech when the EOS logit exceeds T (default -4)\n"
             "            --bench             fixed sentence, seed 0, temperature 0; prints frames/s like the reference\n",
             prog);
     exit(1);
@@ -64,6 +68,7 @@ int main(int argc, char** argv) {
     std::string model_path = "kyutai/pocket-tts-without-voice-cloning/", voice = "cosette", output, input, text;
     bool bench = false, seed_set = false, temp_set = false, have_text = false;
     float temperature = 0.7f;
+    b200_sampling sampling; b200_default_sampling(&sampling);
     for (int i = 1; i < argc; i++) {
         const std::string a = argv[i];
         auto value = [&]() -> const char* { if (i + 1 >= argc) { fprintf(stderr, "error: \"%s\" requires value\n", argv[i]); exit(1); } return argv[++i]; };
@@ -74,6 +79,9 @@ int main(int argc, char** argv) {
         else if (a == "-i" || a == "--input") input = value();
         else if (a == "-s" || a == "--seed") { seed_set = true; ptts_set_seed((unsigned)std::stoi(value())); }
         else if (a == "-t" || a == "--temperature") { temp_set = true; temperature = (float)std::stod(value()); }
+        else if (a == "--lsd-decode-steps") sampling.lsd_steps = std::stoi(value());
+        else if (a == "--noise-clamp") sampling.noise_clamp = (float)std::stod(value());
+        else if (a == "--eos-threshold") sampling.eos_threshold = (float)std::stod(value());
         else if (a == "--bench") bench = true;
         else if (!a.empty() && a[0] == '-') { fprintf(stderr, "error: unrecognized option \"%s\"\n", argv[i]); exit(1); }
         else if (!have_text) { text = a; have_text = true; }
@@ -89,12 +97,17 @@ int main(int argc, char** argv) {
         if (!seed_set) ptts_set_seed(0);
         if (!temp_set) temperature = 0.f;
     }
+    if (b200_sampling_check(&sampling) != B200_OK) {
+        fprintf(stderr, "error: sampling controls out of range (--lsd-decode-steps 1..8, --noise-clamp >= 0, finite --eos-threshold)\n");
+        return 1;
+    }
     if (!have_text) usage(argv[0]);
     if (!model_path.empty() && model_path.back() != '/') model_path += '/';
 
     ptts_context_t* ctx = ptts_init(nullptr, nullptr, model_path.c_str());     // the engine is the backend: ggml pointers are ignored
     const int sample_rate = ptts_get_sample_rate(ctx), frame_size = ptts_get_frame_size(ctx);
     ptts_stream_t* stream = ptts_stream_from_safetensors(ctx, voice.c_str(), temperature);
+    ptts_c_stream_set_sampling(stream, &sampling);
 
     printf("seed: %d\n", (int)ptts_get_seed());
     const double gen_start = now_ms();

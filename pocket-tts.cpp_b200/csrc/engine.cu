@@ -3,6 +3,7 @@
 // graphs on two streams (run_step: the Mimi decode of frame t overlaps the FlowLM step of frame t+1).
 // C ABI declared in include/ptts_b200.h. No CPU fallback: everything below runs on the device or aborts.
 #include "../../include/ptts_b200.h"
+#include <cmath>
 #include "common.cuh"
 #include "gemm.cuh"
 #include "gemm_tc.cuh"
@@ -179,6 +180,12 @@ struct b200_engine {
     long long mkv_slot_stride = 0, mkv_layer_stride = 0;
     int *cur_len = nullptr, *mimi_off = nullptr, *gen_step = nullptr, *eos_step = nullptr, *max_gen = nullptr, *fae = nullptr, *active = nullptr;
     float* temp = nullptr; unsigned int* rng_id = nullptr;   // per-slot sampling temperature, RNG stream id of the sentence in the slot
+    // per-slot sampling controls (DESIGN.md 4.7): LSD decode steps, noise clamp (0 = untruncated), EOS threshold on the logit. Host mirrors of
+    // the last values begun in each slot choose the step's substep count and whether batch 1-2 may use the persistent kernel.
+    int* lsd_steps = nullptr; float *noise_clamp = nullptr, *eos_thr = nullptr;
+    std::vector<int> h_lsd; std::vector<char> h_custom;
+    int step_nsub = 1; bool step_custom = false;               // of the slot range prepare_decode last saw
+    float *lsd_dtab = nullptr, *stepw = nullptr;               // [36][512] t_combined(i/N, (i+1)/N) for N = 1..8, i < N; [slots][32] step weights
     __nv_bfloat16* lat_in_bf16 = nullptr; float* lat_f32 = nullptr;   // [slot][32] backbone input / last latent
     float* e_prev = nullptr;                                          // upsampler state [slot][512]
     std::vector<int> h_cur_len;                                       // host mirror of cur_len
@@ -403,6 +410,8 @@ struct b200_engine {
     // Decode rows of the range [slot0, slot0+n): row r = slot slot0+r. With a shared voice prefix, (re)builds the work list of
     // attn_tile_kernel (plan_prefix_tiles) on the host when the range or the slot -> voice assignment changed. Stream-ordered upload.
     void prepare_decode(int slot0, int n) {
+        step_nsub = 1; step_custom = false;
+        for (int s = slot0; s < slot0 + n; s++) { step_nsub = std::max(step_nsub, h_lsd[s]); step_custom = step_custom || h_custom[s]; }
         actx = AttnCtx{}; actx.row_slot = row_slot; actx.row_pos = row_pos; actx.cs = cs;
         if (!cfg.prefix_share || cfg.kv_f32 || n < tile_min_rows) { dec_grid_items = 0; dec_key_n = -1; return; }
         if (dec_key_slot0 == slot0 && dec_key_n == n && dec_key_version == pfx_version) return;
@@ -559,13 +568,40 @@ struct b200_engine {
     bool fused_head_allowed = getenv("PTTS_B200_FUSED_HEAD") ? atoi(getenv("PTTS_B200_FUSED_HEAD")) != 0 : true;   // tuning hook
     int fused_head_min_rows = getenv("PTTS_B200_FUSED_HEAD_MIN") ? atoi(getenv("PTTS_B200_FUSED_HEAD_MIN")) : 3;
     bool use_fused_head(int R) const { return fused_head_allowed && cfg.gemm_path == 0 && !taps_on && R >= fused_head_min_rows; }
-    // out_norm + EOS + 1-step LSD head over R rows of `h` (reference models/flow_lm.h:114-142, modules/mlp.h:233-251).
-    void flow_head(int R) {
-        const int BIG = 1 << 30;
+    // out_norm + EOS + LSD head over R rows of `h` = slots [slot0, slot0+R) (reference models/flow_lm.h:114-142, modules/mlp.h:233-251).
+    // nsub = 1: the single step latent = noise + v(c, 0, 1, noise). nsub > 1: substep i of a row with N steps is x_{i+1} = x_i + v(c, i/N,
+    // (i+1)/N, x_i) / N while i < N (DESIGN.md 4.7); cond_embed(c) once, then per substep time conditioning, adaLN GEMM, input_proj(bf16(x_i)),
+    // residual chain and final layer.
+    void flow_head(int R, int slot0, int nsub) {
         launch_k(pdl_l(), head_pre_kernel, dim3(R), dim3(256), (size_t)(0), stream, h, R, onw, onb, w_eos, b_eos, c_bf, eos);
         // y = t_combined + cond_embed(c); sy = silu(y)
         Epi ec; ec.resid = t_combined; ec.resid_map = RowMap{}; ec.out2 = sy_bf; ec.out2_map = rows(D_FLOW); ec.out2_type = OUT2_BF16; ec.act = ACT_SILU;
         lin(c_bf, cond_embed, R, ec);
+        if (nsub > 1) {
+            // cond = cond_embed(c) in f32 for the substeps' own time conditioning. A separate plain-output GEMM: an f32 output on the GEMM above
+            // would change its epilogue class (no tensor-core kernel for it), and with it the rows that keep N = 1
+            Epi ey; ey.out = ycond; ey.out_map = rows(D_FLOW);
+            lin(c_bf, cond_embed, R, ey);
+        }
+        launches += 1;                                       // head_pre_kernel
+        for (int sub = 0; sub < nsub; sub++) {
+            if (sub > 0) {                                   // xh = input_proj(bf16(x_sub))
+                launch_k(pdl_l(), noise_inproj_kernel, dim3(R), dim3(128), (size_t)(0), stream, slot0, R, (const float*)latent, (const unsigned long long*)d_seed,
+                         (const float*)temp, (const float*)noise_clamp, (const int*)gen_step, (const unsigned int*)rng_id, (float*)nullptr,
+                         (const __nv_bfloat16*)input_proj_t, (const float*)input_proj.b, xh);
+                launches++;
+            }
+            if (nsub > 1) {
+                launch_k(pdl_l(), lsd_time_kernel, dim3(R), dim3(128), (size_t)(0), stream, slot0, R, sub, (const int*)lsd_steps, (const float*)ycond,
+                         (const float*)lsd_dtab, sy_bf, stepw);
+                launches++;
+            }
+            head_substep(R, sub == 0 ? noise_f32 : latent, nsub > 1 ? stepw : nullptr);
+        }
+    }
+    // adaLN projections of sy + six residual blocks + final layer: latent = x_in + final(...) (* stepw when given).
+    void head_substep(int R, const float* x_in, const float* w) {
+        const int BIG = 1 << 30;
         // all seven adaLN projections of silu(y) in one GEMM: [6 x (shift|scale|gate)] + [shift|scale]
         Epi em; em.out = mod; em.out_map = rows(ada_all.out);
         lin(sy_bf, ada_all, R, em);
@@ -574,9 +610,9 @@ struct b200_engine {
             HfParams hp{};
             hp.R = R; hp.xh = xh; hp.mod = mod; hp.mod_ld = ada_all.out;
             for (int r = 0; r < N_RES; r++) hp.rb[r] = {rb[r].lnw, rb[r].lnb, rb[r].mlp0.w, rb[r].mlp0.b, rb[r].mlp2.w, rb[r].mlp2.b};
-            hp.fnw = fnw; hp.fnb = fnb; hp.wf = final_lin.w; hp.bf = final_lin.b; hp.noise = noise_f32; hp.latent = latent;
+            hp.fnw = fnw; hp.fnb = fnb; hp.wf = final_lin.w; hp.bf = final_lin.b; hp.noise = x_in; hp.latent = latent; hp.stepw = w;
             launch_k(pdl_active, head_res_cluster_kernel, dim3((R + HF_ROWS - 1) / HF_ROWS * HF_CLUSTER), dim3(HF_THREADS), HF_SMEM_BYTES, stream, hp);
-            launches += 2;                                   // + head_pre_kernel
+            launches += 1;
             return;
         }
         for (int r = 0; r < N_RES; r++) {
@@ -592,14 +628,14 @@ struct b200_engine {
             lin(h1_bf, rb[r].mlp2, R, e2);
         }
         const float* m = mod + N_RES * 3 * D_FLOW;
-        Epi ef; ef.resid = noise_f32; ef.resid_map = rows(LDIM); ef.out = latent; ef.out_map = rows(LDIM);
+        Epi ef; ef.resid = x_in; ef.resid_map = rows(LDIM); ef.out = latent; ef.out_map = rows(LDIM);
+        if (w) { ef.rowmul = w; ef.rowmul_ld = LDIM; }
         if (ln_in_gemv(R)) { LnArgs a; a.w = fnw; a.b = fnb; a.eps = 1e-6f; a.shift = m; a.scale = m + D_FLOW; a.mod_ld = ada_all.out; lin_ln(xh, a, final_lin, R, ef); }
         else {
             launch_k(pdl_l(), layernorm_kernel<D_FLOW>, dim3(R), dim3(D_FLOW / 4), (size_t)(0), stream, xh, rows(D_FLOW), BIG, R, 1e-6f, fnw, fnb, m, m + D_FLOW, ada_all.out, hn_bf, nullptr);
             launches++;
             lin(hn_bf, final_lin, R, ef);
         }
-        launches += 1;
     }
 
     // Mimi front end (latent -> 16 transformer input rows, written to `xbuf`), reference models/mimi.h:77-83 + modules/conv.h:283-331.
@@ -728,7 +764,7 @@ struct b200_engine {
     unsigned int* pf_barrier = nullptr;
     bool persistent_allowed = getenv("PTTS_B200_PERSISTENT") ? atoi(getenv("PTTS_B200_PERSISTENT")) != 0 : true;
     bool use_persistent(int n) const {
-        return persistent_allowed && n <= PF_RMAX && !cfg.kv_f32 && cfg.gemm_path == 0 && !taps_on && !profiling && cfg.kv_capacity <= 8 * PF_MAX_KEYS;
+        return persistent_allowed && !step_custom && n <= PF_RMAX && !cfg.kv_f32 && cfg.gemm_path == 0 && !taps_on && !profiling && cfg.kv_capacity <= 8 * PF_MAX_KEYS;
     }
     void flow_persistent(int slot0, int n, bool injected, float* xbuf) {
         PfParams p{};
@@ -759,7 +795,7 @@ struct b200_engine {
         PTTS_CUDA_CHECK(cudaLaunchKernelEx(&lc, flow_persistent_kernel, p));
         launches++;
         launch_k(false, step_front_kernel, dim3(n), dim3(M_DIM), (size_t)(0), stream, slot0, n, (const float*)eos, (const float*)latent, cur_len, gen_step, eos_step, (const int*)max_gen,
-                 (const int*)fae, active, lat_in_bf16, lat_f32, produced, eos_out, (const float*)emb_std, (const float*)emb_mean, (const __half*)wq, (const float*)wup, (const float*)bup, e_prev, xbuf);
+                 (const int*)fae, (const float*)eos_thr, active, lat_in_bf16, lat_f32, produced, eos_out, (const float*)emb_std, (const float*)emb_mean, (const __half*)wq, (const float*)wup, (const float*)bup, e_prev, xbuf);
         launches++;
     }
 
@@ -786,14 +822,15 @@ struct b200_engine {
         seg_end(s_flow);
         const int s_head = seg_begin(2);
         launch_k(pdl_l(), noise_inproj_kernel, dim3(n), dim3(128), (size_t)(0), stream, slot0, n, (const float*)(injected ? noise_src : nullptr), (const unsigned long long*)d_seed,
-                 (const float*)temp, (const int*)gen_step, (const unsigned int*)rng_id, noise_f32, (const __nv_bfloat16*)input_proj_t, (const float*)input_proj.b, xh);
-        flow_head(n);
+                 (const float*)temp, (const float*)noise_clamp, (const int*)gen_step, (const unsigned int*)rng_id, noise_f32, (const __nv_bfloat16*)input_proj_t,
+                 (const float*)input_proj.b, xh);
+        flow_head(n, slot0, step_nsub);
         launches += 1;
         seg_end(s_head);
         set_pdl(pdl_small);
         // stop rule + latent hand-off + Mimi front end (writes the 16 transformer input rows of every slot to xbuf)
         launch_k(pdl_l(), step_front_kernel, dim3(n), dim3(M_DIM), (size_t)(0), stream, slot0, n, (const float*)eos, (const float*)latent, cur_len, gen_step, eos_step, (const int*)max_gen,
-                 (const int*)fae, active, lat_in_bf16, lat_f32, produced, eos_out, (const float*)emb_std, (const float*)emb_mean, (const __half*)wq, (const float*)wup, (const float*)bup, e_prev, xbuf);
+                 (const int*)fae, (const float*)eos_thr, active, lat_in_bf16, lat_f32, produced, eos_out, (const float*)emb_std, (const float*)emb_mean, (const __half*)wq, (const float*)wup, (const float*)bup, e_prev, xbuf);
         launches++;
     }
     void step_enqueue(int slot0, int n, bool injected) {       // single-stream form (eager / profiling)
@@ -826,7 +863,10 @@ struct b200_engine {
             else mimi(slot0, n, mx2[par], part == ALL_PARTS ? -1 : part);
         };
         if (!cfg.cuda_graphs || profiling || taps_on) { body(); return; }
-        const auto gkey = std::make_tuple((kind * 2 + par) * 16 + part, slot0, n, (injected ? 1 : 0) | (pcm_out != pcm ? 2 : 0) | (noise_src != noise_inj ? 4 : 0), (kind == 0 || kind == 2) ? dec_grid_items : 0);
+        // FlowLM graphs are also keyed by the LSD substep count and by whether non-default sampling rules the persistent kernel out: both are
+        // 1 / false for default sentences, which therefore replay the same graphs as without sampling controls
+        const int samp = (kind == 0 || kind == 2) ? ((step_nsub - 1) << 3) | (step_custom ? 64 : 0) : 0;
+        const auto gkey = std::make_tuple((kind * 2 + par) * 16 + part, slot0, n, (injected ? 1 : 0) | (pcm_out != pcm ? 2 : 0) | (noise_src != noise_inj ? 4 : 0) | samp, (kind == 0 || kind == 2) ? dec_grid_items : 0);
         if (!graphs.count(gkey)) { graphs[gkey].last_use = ++graph_clock; evict_graphs(); }
         GraphEntry& g = graphs[gkey];
         g.last_use = ++graph_clock;
@@ -1060,26 +1100,33 @@ struct b200_engine {
 namespace {
 
 __global__ void set_meta_kernel(int slot, int cur, int mg, int f, float t, const float* bos, int* cur_len, int* gen_step, int* eos_step,
-                                int* max_gen, int* fae, int* active, float* temp, __nv_bfloat16* lat_in_bf16, float* lat_f32) {
+                                int* max_gen, int* fae, int* active, float* temp, __nv_bfloat16* lat_in_bf16, float* lat_f32,
+                                int* lsd_steps, float* noise_clamp, float* eos_thr) {
     pdl_prologue();
     const int i = threadIdx.x;
-    if (i == 0) { cur_len[slot] = cur; gen_step[slot] = 0; eos_step[slot] = -1; max_gen[slot] = mg; fae[slot] = f; active[slot] = mg > 0 ? 1 : 0; temp[slot] = t; }
+    if (i == 0) {
+        cur_len[slot] = cur; gen_step[slot] = 0; eos_step[slot] = -1; max_gen[slot] = mg; fae[slot] = f; active[slot] = mg > 0 ? 1 : 0; temp[slot] = t;
+        lsd_steps[slot] = 1; noise_clamp[slot] = 0.f; eos_thr[slot] = -4.f;
+    }
     if (i < LDIM) { lat_f32[slot * LDIM + i] = bos[i]; lat_in_bf16[slot * LDIM + i] = __float2bfloat16_rn(bos[i]); }
 }
 
 // Batched sentence start (b200_begin_sentences; reference _stream_sentence_init src/pocket_tts.cpp:416-444, copy_states models/flow_lm.h:70-78,
 // init(mimi_states) models/mimi.h:71-75): one launch each for all n sentences instead of three launches per sentence.
-// meta = [slot | src voice slot | prefix rows | cur_len | max_gen | frames_after_eos | shared prefix rows (0 = private copy) | RNG stream id] x n (ints), temps[n].
+// meta = [slot | src voice slot | prefix rows | cur_len | max_gen | frames_after_eos | shared prefix rows (0 = private copy) | RNG stream id |
+// LSD steps] x n (ints), then [temp | noise clamp | EOS threshold] x n (floats).
 // FlowLM-side state (main stream): stop-rule counters, BOS latent, upsampler carry, prefix assignment.
 __global__ void begin_meta_kernel(int n, const int* __restrict__ meta, const float* __restrict__ temps, const float* bos, int* cur_len, int* gen_step, int* eos_step,
                                   int* max_gen, int* fae, int* active, float* temp, __nv_bfloat16* lat_in_bf16, float* lat_f32,
-                                  int* __restrict__ pfx_slot, int* __restrict__ pfx_len, float* __restrict__ e_prev, unsigned int* __restrict__ rng_id) {
+                                  int* __restrict__ pfx_slot, int* __restrict__ pfx_len, float* __restrict__ e_prev, unsigned int* __restrict__ rng_id,
+                                  int* __restrict__ lsd_steps, float* __restrict__ noise_clamp, float* __restrict__ eos_thr) {
     const int j = blockIdx.x, i = threadIdx.x;
     if (j >= n) return;
     const int slot = meta[j], cur = meta[3 * n + j], mg = meta[4 * n + j], f = meta[5 * n + j];
     if (i == 0) {
         cur_len[slot] = cur; gen_step[slot] = 0; eos_step[slot] = -1; max_gen[slot] = mg; fae[slot] = f; active[slot] = mg > 0 ? 1 : 0; temp[slot] = temps[j];
         pfx_slot[slot] = meta[n + j]; pfx_len[slot] = meta[6 * n + j]; rng_id[slot] = (unsigned int)meta[7 * n + j];
+        lsd_steps[slot] = meta[8 * n + j]; noise_clamp[slot] = temps[n + j]; eos_thr[slot] = temps[2 * n + j];
     }
     if (i < LDIM) { lat_f32[slot * LDIM + i] = bos[i]; lat_in_bf16[slot * LDIM + i] = __float2bfloat16_rn(bos[i]); }
     for (int c = i; c < M_DIM; c += blockDim.x) e_prev[(long long)slot * M_DIM + c] = 0.f;
@@ -1260,9 +1307,11 @@ int b200_finalize_weights(b200_engine* e) {
     }
     e->final_lin = e->up_lin(f + "final_layer.linear", LDIM, D_FLOW);
     e->fnw = e->up_f32(f + "final_layer.norm_final.weight", false); e->fnb = e->up_f32(f + "final_layer.norm_final.bias", false);
-    {   // constant timestep embedding t_combined = (TE1(t=1) + TE0(s=0)) / 2 (reference modules/mlp.h:92-106,18-37,241-245)
+    // timestep embedding t_combined(s, t) = (TE1(t) + TE0(s)) / 2 (reference modules/mlp.h:92-106,18-37,241-245): the constant (0, 1) of the
+    // single-step head, and for multi-step LSD the table t_combined(i/N, (i+1)/N), N = 1..8, i < N (DESIGN.md 4.7)
+    auto time_cond = [&](float s_val, float t_val) {
         std::vector<float> tc(D_FLOW, 0.f);
-        const float tval[2] = {0.0f, 1.0f};
+        const float tval[2] = {s_val, t_val};
         for (int idx = 0; idx < 2; idx++) {
             const std::string p = f + "time_embed." + std::to_string(idx) + ".";
             auto *w0 = e->find(p + "mlp.0.weight"), *b0 = e->find(p + "mlp.0.bias", false), *w2 = e->find(p + "mlp.2.weight"), *b2 = e->find(p + "mlp.2.bias", false);
@@ -1278,7 +1327,18 @@ int b200_finalize_weights(b200_engine* e) {
             for (int i = 0; i < D_FLOW; i++) tc[i] += alpha->f[i] * (u[i] / sd);
         }
         for (auto& v : tc) v *= 0.5f;
-        e->t_combined = e->upload(tc);
+        return tc;
+    };
+    {
+        const std::vector<float> t01 = time_cond(0.0f, 1.0f);
+        e->t_combined = e->upload(t01);
+        std::vector<float> dt((size_t)B200_LSD_MAX_STEPS * (B200_LSD_MAX_STEPS + 1) / 2 * D_FLOW);
+        for (int N = 1; N <= B200_LSD_MAX_STEPS; N++)
+            for (int i = 0; i < N; i++) {
+                const std::vector<float> ti = time_cond((float)i / (float)N, (float)(i + 1) / (float)N);
+                std::copy(ti.begin(), ti.end(), dt.begin() + ((size_t)N * (N - 1) / 2 + i) * D_FLOW);
+            }
+        e->lsd_dtab = e->upload(dt);
     }
     // Mimi
     {
@@ -1372,6 +1432,8 @@ int b200_finalize_weights(b200_engine* e) {
     e->cur_len = e->dalloc<int>(TS); e->mimi_off = e->dalloc<int>(S); e->gen_step = e->dalloc<int>(S); e->eos_step = e->dalloc<int>(S);
     e->max_gen = e->dalloc<int>(S); e->fae = e->dalloc<int>(S); e->active = e->dalloc<int>(S); e->temp = e->dalloc<float>(S);
     { std::vector<unsigned int> ids(S); for (int i = 0; i < S; i++) ids[i] = (unsigned int)i; e->rng_id = e->upload(ids); }
+    e->lsd_steps = e->upload(std::vector<int>(S, 1)); e->noise_clamp = e->dalloc<float>(S); e->eos_thr = e->upload(std::vector<float>(S, -4.f));
+    e->h_lsd.assign(S, 1); e->h_custom.assign(S, 0);
     e->lat_in_bf16 = e->dalloc<__nv_bfloat16>((size_t)S * LDIM); e->lat_f32 = e->dalloc<float>((size_t)S * LDIM);
     e->e_prev = e->dalloc<float>((size_t)S * M_DIM);
     e->h = e->dalloc<float>((size_t)MR * D_MODEL); e->q = e->dalloc<float>((size_t)MR * D_MODEL);
@@ -1387,6 +1449,7 @@ int b200_finalize_weights(b200_engine* e) {
     e->row_slot = e->dalloc<int>(MR); e->row_pos = e->dalloc<int>(MR); e->tok = e->dalloc<int>(MR); e->cs = e->dalloc<float2>((size_t)MR * 32);
     e->c_bf = e->dalloc<__nv_bfloat16>((size_t)S * D_MODEL); e->sy_bf = e->dalloc<__nv_bfloat16>((size_t)S * D_FLOW);
     e->hn_bf = e->dalloc<__nv_bfloat16>((size_t)S * D_FLOW); e->h1_bf = e->dalloc<__nv_bfloat16>((size_t)S * D_FLOW);
+    e->ycond = e->dalloc<float>((size_t)S * D_FLOW); e->stepw = e->dalloc<float>((size_t)S * LDIM);
     e->eos = e->dalloc<float>(S); e->eos_out = e->dalloc<float>(S); e->mod = e->dalloc<float>((size_t)S * e->ada_all.out); e->xh = e->dalloc<float>((size_t)S * D_FLOW);
     e->noise_f32 = e->dalloc<float>((size_t)S * LDIM); e->noise_inj = e->dalloc<float>((size_t)S * LDIM); e->noise_src = e->noise_inj;
     for (int i = 0; i < 2; i++) e->noise_alt[i] = e->dalloc<float>((size_t)S * LDIM); e->latent = e->dalloc<float>((size_t)S * LDIM);
@@ -1567,8 +1630,25 @@ int b200_begin_sentences(b200_engine* e, int n, const int32_t* slots, const int3
 
 int b200_begin_sentences_ex(b200_engine* e, int n, const int32_t* slots, const int32_t* voices, const int32_t* tokens, const int32_t* tok_off,
                             const int32_t* max_gen_len, const int32_t* frames_after_eos, const float* temp, const uint32_t* rng_stream) {
+    return b200_begin_sentences_sampling(e, n, slots, voices, tokens, tok_off, max_gen_len, frames_after_eos, temp, rng_stream, nullptr);
+}
+
+void b200_default_sampling(b200_sampling* s) {
+    if (s) { s->lsd_steps = 1; s->noise_clamp = 0.f; s->eos_threshold = -4.f; }
+}
+
+int b200_sampling_check(const b200_sampling* s) {
+    if (!s || s->lsd_steps < 1 || s->lsd_steps > B200_LSD_MAX_STEPS || !(s->noise_clamp >= 0.f) || !std::isfinite(s->noise_clamp) ||
+        !std::isfinite(s->eos_threshold)) return B200_EINVAL;
+    return B200_OK;
+}
+
+int b200_begin_sentences_sampling(b200_engine* e, int n, const int32_t* slots, const int32_t* voices, const int32_t* tokens, const int32_t* tok_off,
+                                  const int32_t* max_gen_len, const int32_t* frames_after_eos, const float* temp, const uint32_t* rng_stream,
+                                  const b200_sampling* sampling) {
     NvtxRange nvtx_range("ptts.begin_sentences");
     if (!e || !e->finalized || n < 0) return B200_EINVAL;
+    if (sampling) for (int i = 0; i < n; i++) if (b200_sampling_check(&sampling[i]) != B200_OK) return B200_EINVAL;
     PTTS_CUDA_CHECK(cudaSetDevice(e->cfg.device));
     std::vector<int> rs, rp, rt;
     for (int i = 0; i < n; i++) {
@@ -1591,9 +1671,11 @@ int b200_begin_sentences_ex(b200_engine* e, int n, const int32_t* slots, const i
     if (e->begin_used) PTTS_CUDA_CHECK(cudaStreamWaitEvent(e->stream, e->ev_reset, 0));
     e->begin_used = true;
     const size_t elt = e->cfg.kv_f32 ? 4 : 2;
-    // per-sentence metadata in one upload: [slot | src voice slot | prefix rows | cur_len | max_gen | frames_after_eos | shared rows] x n, then temps
-    int* pm = (int*)e->pin_acquire((size_t)9 * n * sizeof(int));
-    float* pt = (float*)(pm + 8 * n);
+    // per-sentence metadata in one upload: [slot | src voice slot | prefix rows | cur_len | max_gen | frames_after_eos | shared rows | RNG id |
+    // LSD steps] x n, then [temp | noise clamp | EOS threshold] x n
+    int* pm = (int*)e->pin_acquire((size_t)12 * n * sizeof(int));
+    float* pt = (float*)(pm + 9 * n);
+    b200_sampling def; b200_default_sampling(&def);
     int max_copy = 0;
     for (int i = 0; i < n; i++) {
         const int slot = slots[i], v = voices[i];
@@ -1607,22 +1689,25 @@ int b200_begin_sentences_ex(b200_engine* e, int n, const int32_t* slots, const i
         const int shared = e->cfg.prefix_share ? start : 0;
         pm[i] = slot; pm[n + i] = e->cfg.max_slots + v; pm[2 * n + i] = start; pm[3 * n + i] = start + nt;
         pm[4 * n + i] = mg; pm[5 * n + i] = frames_after_eos[i]; pm[6 * n + i] = shared; pm[7 * n + i] = (int)(rng_stream ? rng_stream[i] : (uint32_t)slot);
-        pt[i] = temp[i];
+        const b200_sampling& sp = sampling ? sampling[i] : def;
+        pm[8 * n + i] = sp.lsd_steps; pt[i] = temp[i]; pt[n + i] = sp.noise_clamp; pt[2 * n + i] = sp.eos_threshold;
+        e->h_lsd[slot] = sp.lsd_steps; e->h_custom[slot] = sp.lsd_steps != 1 || sp.noise_clamp != 0.f || sp.eos_threshold != -4.f;
         e->h_cur_len[slot] = start + nt;
         if (e->h_pfx_slot[slot] != e->cfg.max_slots + v || e->h_pfx_len[slot] != shared) { e->h_pfx_slot[slot] = e->cfg.max_slots + v; e->h_pfx_len[slot] = shared; e->pfx_version++; }
         if (!e->cfg.prefix_share) max_copy = std::max(max_copy, start);
     }
     if ((size_t)n > e->begin_cap) {
-        e->begin_meta = e->dalloc<int>((size_t)8 * n, false); e->begin_temp = e->dalloc<float>((size_t)n, false); e->begin_cap = n;
+        e->begin_meta = e->dalloc<int>((size_t)9 * n, false); e->begin_temp = e->dalloc<float>((size_t)3 * n, false); e->begin_cap = n;
     }
-    PTTS_CUDA_CHECK(cudaMemcpyAsync(e->begin_meta, pm, (size_t)8 * n * sizeof(int), cudaMemcpyHostToDevice, e->stream));
-    PTTS_CUDA_CHECK(cudaMemcpyAsync(e->begin_temp, pt, (size_t)n * sizeof(float), cudaMemcpyHostToDevice, e->stream));
+    PTTS_CUDA_CHECK(cudaMemcpyAsync(e->begin_meta, pm, (size_t)9 * n * sizeof(int), cudaMemcpyHostToDevice, e->stream));
+    PTTS_CUDA_CHECK(cudaMemcpyAsync(e->begin_temp, pt, (size_t)3 * n * sizeof(float), cudaMemcpyHostToDevice, e->stream));
     e->pin_release(e->stream);
     if (max_copy > 0)   // reference semantics (prefix_share = 0): private copy of the voice-conditioned prefix, models/flow_lm.h:70-78
         launch_k(false, begin_copy_prefix_kernel, dim3(8, 2 * N_LAYERS, n), dim3(256), (size_t)0, e->stream, n, (const int*)e->begin_meta, (char*)e->kc, (char*)e->vc,
                  (long long)(e->kv_slot_stride * elt), (long long)(e->kv_layer_stride * elt), (long long)(D_MODEL * elt));
     launch_k(false, begin_meta_kernel, dim3(n), dim3(128), (size_t)0, e->stream, n, (const int*)e->begin_meta, (const float*)e->begin_temp, (const float*)e->d_bos, e->cur_len,
-             e->gen_step, e->eos_step, e->max_gen, e->fae, e->active, e->temp, e->lat_in_bf16, e->lat_f32, e->pfx_slot, e->pfx_len, e->e_prev, e->rng_id);
+             e->gen_step, e->eos_step, e->max_gen, e->fae, e->active, e->temp, e->lat_in_bf16, e->lat_f32, e->pfx_slot, e->pfx_len, e->e_prev, e->rng_id,
+             e->lsd_steps, e->noise_clamp, e->eos_thr);
     // Mimi-side reset on the Mimi stream: behind every Mimi decode already enqueued there, ahead of the new sentences' first decode. The
     // main stream only waits for it when it touches Mimi state itself (join_mimi: synchronous b200_step, Mimi-only calls).
     PTTS_CUDA_CHECK(cudaEventRecord(e->ev_begin, e->stream));
@@ -1643,6 +1728,7 @@ int b200_end_sentences(b200_engine* e, int n, const int32_t* slots) {
     for (int i = 0; i < n; i++) if (slots[i] < 0 || slots[i] >= e->cfg.max_slots) return B200_EINVAL;
     if (n == 0) return B200_OK;
     PTTS_CUDA_CHECK(cudaSetDevice(e->cfg.device));
+    for (int i = 0; i < n; i++) { e->h_lsd[slots[i]] = 1; e->h_custom[slots[i]] = 0; }   // a dead row does not hold its range to more substeps
     e->grow(e->end_slots, e->end_slots_cap, (size_t)n);
     int* ps = (int*)e->pin_acquire((size_t)n * sizeof(int));
     memcpy(ps, slots, (size_t)n * sizeof(int));
@@ -1843,7 +1929,8 @@ int b200_debug_set_position(b200_engine* e, int slot0, int n, int pos, int max_g
     for (int s = slot0; s < slot0 + n; s++) {
         launch_k(false, reset_slot_kernel, dim3(1, e->shifts.n), dim3(256), (size_t)(0), e->stream, e->shifts, s, e->e_prev, e->mimi_off);
         launch_k(false, set_meta_kernel, dim3(1), dim3(32), (size_t)(0), e->stream, s, pos, max_gen_len, 1 << 28, 0.f, bos, e->cur_len, e->gen_step, e->eos_step, e->max_gen, e->fae, e->active,
-                                                 e->temp, e->lat_in_bf16, e->lat_f32);
+                                                 e->temp, e->lat_in_bf16, e->lat_f32, e->lsd_steps, e->noise_clamp, e->eos_thr);
+        e->h_lsd[s] = 1; e->h_custom[s] = 0;
     }
     e->launches += 2 * n;
     return B200_OK;

@@ -40,8 +40,9 @@ struct HfParams {
     const float* mod; int mod_ld;        // [R][mod_ld] adaLN projections: 6 x (shift | scale | gate), then (shift | scale)
     struct { const float *lnw, *lnb; const __nv_bfloat16* w0; const float* b0; const __nv_bfloat16* w2; const float* b2; } rb[N_RES];
     const float *fnw, *fnb; const __nv_bfloat16* wf; const float* bf;   // final layer (512 -> 32)
-    const float* noise;                  // [R][32] the step's noise (latent = noise + flow)
-    float* latent;                       // [R][32]
+    const float* noise;                  // [R][32] the step's noise, or x_i of LSD substep i (latent = noise + flow)
+    float* latent;                       // [R][32] (may alias noise: each element is read and written by the same thread)
+    const float* stepw;                  // [R][32] multi-step LSD: latent = noise + flow * stepw (lsd_time_kernel); nullptr = one step
 };
 
 __device__ __forceinline__ uint32_t hf_mapa(const void* p, int rank) {     // address of the same shared-memory location in CTA `rank` of the cluster
@@ -290,8 +291,13 @@ __global__ void __cluster_dims__(HF_CLUSTER, 1, 1) __launch_bounds__(HF_THREADS,
             const int row = row0 + 8 * hf + g;
             if (row < p.R) {
                 const long long o = (long long)row * LDIM + c;
-                p.latent[o] = __fadd_rn(__fadd_rn(acc[j][2 * hf], b0), p.noise[o]);
-                p.latent[o + 1] = __fadd_rn(__fadd_rn(acc[j][2 * hf + 1], b1), p.noise[o + 1]);
+                if (p.stepw) {
+                    p.latent[o] = __fadd_rn(__fmul_rn(__fadd_rn(acc[j][2 * hf], b0), p.stepw[o]), p.noise[o]);
+                    p.latent[o + 1] = __fadd_rn(__fmul_rn(__fadd_rn(acc[j][2 * hf + 1], b1), p.stepw[o + 1]), p.noise[o + 1]);
+                } else {
+                    p.latent[o] = __fadd_rn(__fadd_rn(acc[j][2 * hf], b0), p.noise[o]);
+                    p.latent[o + 1] = __fadd_rn(__fadd_rn(acc[j][2 * hf + 1], b1), p.noise[o + 1]);
+                }
             }
         }
     }

@@ -21,6 +21,8 @@
 #include <string>
 #include <vector>
 
+#include "../../../include/ptts_b200.h"
+
 namespace ptts_host {
 
 struct BatchOps {
@@ -33,6 +35,10 @@ struct BatchOps {
     // optional: the sentences of these slots end before the next submitted step (slots freed by cancel and not refilled); null = such
     // slots keep generating on the engine, unattributed, until a sentence start reuses them
     int (*end)(void* user, int n, const int32_t* slots) = nullptr;
+    // optional: `begin` plus each sentence's sampling controls (b200_begin_sentences_sampling); when set it is called instead of `begin`
+    int (*begin_sampling)(void* user, int n, const int32_t* slots, const int32_t* voices, const int32_t* tokens, const int32_t* tok_off,
+                          const int32_t* max_gen_len, const int32_t* frames_after_eos, const float* temp, const uint32_t* rng_stream,
+                          const b200_sampling* sampling) = nullptr;
 };
 
 struct BatchStats {
@@ -53,6 +59,7 @@ public:
         std::vector<int32_t> ids;            // SentencePiece ids
         int max_gen = 0, fae = 0;            // reference stop rule: cap int((words + 2) * 12.5), frames_after_eos (src/pocket_tts.cpp:429-430,504-506)
         uint32_t rng_stream = 0;
+        b200_sampling sampling{1, 0.f, -4.f};  // LSD steps, noise clamp, EOS threshold (b200_default_sampling)
         std::vector<float> pcm; int frames = 0; bool done = false, started = false;
     };
     enum { kQueued = 0, kRunning = 1, kDone = 2, kCancelled = 3 };
@@ -103,7 +110,7 @@ public:
                 for (int s = 0; s < n_slots_; s++) { if (slots_[s].job >= 0) { busy++; top = s + 1; } else n_free++; }
                 // ---- refill free slots ----
                 if (!pending_.empty() && n_free > 0 && (busy == 0 || n_free >= std::min(refill_min, (int)pending_.size()) || since_refill_ >= refill_every)) {
-                    std::vector<int32_t> sl, vo, toks, off{0}, mg, fae; std::vector<float> tp; std::vector<uint32_t> rs;
+                    std::vector<int32_t> sl, vo, toks, off{0}, mg, fae; std::vector<float> tp; std::vector<uint32_t> rs; std::vector<b200_sampling> sa;
                     for (int s = 0; s < n_slots_ && !pending_.empty(); s++) {
                         if (slots_[s].job >= 0) continue;
                         const int j = pending_.front(); pending_.pop_front();
@@ -114,11 +121,13 @@ public:
                         // frame re-faulted every page several times and cost more host time per step than the GPU step itself
                         if (keep_pcm) J.pcm.reserve((size_t)effective_cap(J) * frame_);
                         sl.push_back(s); vo.push_back(J.voice); toks.insert(toks.end(), J.ids.begin(), J.ids.end()); off.push_back((int32_t)toks.size());
-                        mg.push_back(J.max_gen); fae.push_back(J.fae); tp.push_back(J.temp); rs.push_back(J.rng_stream);
+                        mg.push_back(J.max_gen); fae.push_back(J.fae); tp.push_back(J.temp); rs.push_back(J.rng_stream); sa.push_back(J.sampling);
                     }
                     if (!sl.empty()) {
                         const auto tb = clk::now();
-                        const int rc = ops_.begin(ops_.user, (int)sl.size(), sl.data(), vo.data(), toks.data(), off.data(), mg.data(), fae.data(), tp.data(), rs.data());
+                        const int rc = ops_.begin_sampling
+                            ? ops_.begin_sampling(ops_.user, (int)sl.size(), sl.data(), vo.data(), toks.data(), off.data(), mg.data(), fae.data(), tp.data(), rs.data(), sa.data())
+                            : ops_.begin(ops_.user, (int)sl.size(), sl.data(), vo.data(), toks.data(), off.data(), mg.data(), fae.data(), tp.data(), rs.data());
                         stats_.begin_ms += std::chrono::duration<double, std::milli>(clk::now() - tb).count();
                         if (rc != 0) return rc;
                         stats_.refills++; since_refill_ = 0;

@@ -145,6 +145,7 @@ struct ptts_stream_t {
     ptts_context_t* ctx = nullptr;
     int slot = -1, voice = -1;
     float temp = 0.7f;
+    b200_sampling sampling{1, 0.f, -4.f};   // applies from the next sentence (ptts_c_stream_set_sampling)
     SentenceSplitter sproc;
     int frames_after_eos = 0, max_gen_len = 0, generation_step = 0;
     int inflight = 0;                       // frames submitted to the engine but not collected yet (look-ahead pipeline)
@@ -322,7 +323,8 @@ bool ptts_stream_receive(ptts_stream_t* s, float* samples) {          // referen
         std::vector<int> ids = s->ctx->tokenizer.encode(text);
         std::vector<int32_t> ids32(ids.begin(), ids.end());
         stream_drain(s);
-        const int rc = b200_begin_sentence(s->ctx->engine, s->slot, s->voice, ids32.data(), (int)ids32.size(), max_gen_len, fae, s->temp);
+        const int32_t off[2] = {0, (int32_t)ids32.size()};
+        const int rc = b200_begin_sentences_sampling(s->ctx->engine, 1, &s->slot, &s->voice, ids32.data(), off, &max_gen_len, &fae, &s->temp, nullptr, &s->sampling);
         if (rc != B200_OK) { fprintf(stderr, "error: sentence init failed (%d)\n", rc); exit(1); }
         s->frames_after_eos = fae; s->max_gen_len = max_gen_len; s->generation_step = 0;
         if (stream_step(s, samples)) return true;
@@ -347,6 +349,11 @@ void ptts_c_stream_reset(ptts_stream_t* s) { ptts_stream_reset(s); }
 void ptts_c_stream_flush(ptts_stream_t* s) { ptts_stream_flush(s); }
 void ptts_c_stream_send(ptts_stream_t* s, const char* chunk) { ptts_stream_send(s, chunk); }
 int ptts_c_stream_receive(ptts_stream_t* s, float* samples) { return ptts_stream_receive(s, samples) ? 1 : 0; }
+int ptts_c_stream_set_sampling(ptts_stream_t* s, const b200_sampling* sp) {
+    if (!s || b200_sampling_check(sp) != B200_OK) return B200_EINVAL;
+    s->sampling = *sp;
+    return B200_OK;
+}
 b200_engine* ptts_c_engine(ptts_context_t* c) { return c ? c->engine : nullptr; }
 // The reference API has no destroy functions (contexts live for the process, src/pocket_tts.cpp:313,381); long-running hosts and
 // tests that create several engines need one. Streams of the context must not be used afterwards.
@@ -392,8 +399,8 @@ struct ptts_batch_t {
     BatchScheduler* sched = nullptr;
 };
 static int batch_begin_engine(void* u, int n, const int32_t* sl, const int32_t* vo, const int32_t* toks, const int32_t* off, const int32_t* mg,
-                              const int32_t* fae, const float* tp, const uint32_t* rs) {
-    return b200_begin_sentences_ex((b200_engine*)u, n, sl, vo, toks, off, mg, fae, tp, rs);
+                              const int32_t* fae, const float* tp, const uint32_t* rs, const b200_sampling* sa) {
+    return b200_begin_sentences_sampling((b200_engine*)u, n, sl, vo, toks, off, mg, fae, tp, rs, sa);
 }
 static int batch_submit_engine(void* u, int slot0, int n) { return b200_submit((b200_engine*)u, slot0, n, nullptr); }
 static int batch_collect_engine(void* u, float* pcm, int32_t* produced) { return b200_collect((b200_engine*)u, pcm, produced); }
@@ -405,7 +412,7 @@ ptts_batch_t* ptts_c_batch_create(ptts_context_t* ctx, int n_slots) {
     if (n_slots <= 0 || n_slots > max_slots) n_slots = max_slots;
     for (bool used : ctx->slot_used) if (used) { fprintf(stderr, "error: ptts_c_batch_create needs a context without open streams (slots are shared)\n"); return nullptr; }
     auto* b = new ptts_batch_t; b->ctx = ctx;
-    BatchOps ops; ops.user = ctx->engine; ops.begin = batch_begin_engine; ops.submit = batch_submit_engine; ops.collect = batch_collect_engine;
+    BatchOps ops; ops.user = ctx->engine; ops.begin_sampling = batch_begin_engine; ops.submit = batch_submit_engine; ops.collect = batch_collect_engine;
     ops.end = batch_end_engine;
     b->sched = new BatchScheduler(ops, n_slots);
     if (ctx->seed_pushed != g_seed || !ctx->seed_valid) { b200_set_seed(ctx->engine, g_seed); ctx->seed_pushed = g_seed; ctx->seed_valid = true; }
@@ -422,6 +429,14 @@ ptts_batch_t* ptts_c_batch_create_with_ops_ex(void* user, ptts_batch_begin_fn be
 ptts_batch_t* ptts_c_batch_create_with_ops(void* user, ptts_batch_begin_fn begin, ptts_batch_submit_fn submit, ptts_batch_collect_fn collect, int n_slots, int frame_size) {
     return ptts_c_batch_create_with_ops_ex(user, begin, submit, collect, nullptr, n_slots, frame_size);
 }
+ptts_batch_t* ptts_c_batch_create_with_ops_sampling(void* user, ptts_batch_begin_sampling_fn begin, ptts_batch_submit_fn submit, ptts_batch_collect_fn collect,
+                                                    ptts_batch_end_fn end, int n_slots, int frame_size) {
+    if (!begin || !submit || !collect || n_slots < 1 || frame_size < 1) return nullptr;
+    auto* b = new ptts_batch_t;
+    BatchOps ops; ops.user = user; ops.begin_sampling = begin; ops.submit = submit; ops.collect = collect; ops.end = end;
+    b->sched = new BatchScheduler(ops, n_slots, frame_size);
+    return b;
+}
 void ptts_c_batch_destroy(ptts_batch_t* b) { if (b) { b->sched->drain(); delete b->sched; delete b; } }
 int ptts_c_batch_configure(ptts_batch_t* b, int refill_min, int refill_every, int range_quantum, int keep_pcm) {
     if (!b) return B200_EINVAL;
@@ -434,7 +449,11 @@ int ptts_c_batch_configure(ptts_batch_t* b, int refill_min, int refill_every, in
 // One utterance = text in the reference's streaming sense: split into sentences (str_processor, conditioners/text.h:181-251), each
 // sentence is one job with the reference's cap and frames_after_eos (src/pocket_tts.cpp:429-430,504-506).
 int ptts_c_batch_add(ptts_batch_t* b, const char* voice, const char* text, float temp) {
+    return ptts_c_batch_add_sampling(b, voice, text, temp, nullptr);
+}
+int ptts_c_batch_add_sampling(ptts_batch_t* b, const char* voice, const char* text, float temp, const b200_sampling* sampling) {
     if (!b || !b->ctx || !voice || !text) return B200_EINVAL;
+    if (sampling && b200_sampling_check(sampling) != B200_OK) return B200_EINVAL;
     const int vid = resolve_voice(b->ctx, voice);
     auto& rv = b->sched->room_of_voice;
     if ((int)rv.size() <= vid) rv.resize(vid + 1, 1 << 30);
@@ -444,6 +463,7 @@ int ptts_c_batch_add(ptts_batch_t* b, const char* voice, const char* text, float
     int idx = 0;
     for (const std::string& sent : sp.sentences) {
         BatchScheduler::Job j; j.utt = utt; j.index = idx++; j.voice = vid; j.temp = temp;
+        if (sampling) j.sampling = *sampling;
         const int words = count_words_impl(sent);
         j.fae = (words <= 4 ? 3 : 1) + 2; j.max_gen = (int)((words + 2.0f) * 12.5f);
         std::vector<int> ids = b->ctx->tokenizer.encode(sent);
@@ -453,8 +473,10 @@ int ptts_c_batch_add(ptts_batch_t* b, const char* voice, const char* text, float
     return utt;
 }
 // One sentence given as token ids, appended to utterance `utt`.
-static int batch_add_token_job(ptts_batch_t* b, int utt, int voice_id, const int32_t* ids, int n_ids, int max_gen_len, int frames_after_eos, float temp, uint32_t rng_stream) {
+static int batch_add_token_job(ptts_batch_t* b, int utt, int voice_id, const int32_t* ids, int n_ids, int max_gen_len, int frames_after_eos, float temp,
+                               uint32_t rng_stream, const b200_sampling* sampling) {
     if (n_ids < 0 || (n_ids > 0 && !ids)) return B200_EINVAL;
+    if (sampling && b200_sampling_check(sampling) != B200_OK) return B200_EINVAL;
     if (b->ctx) {
         auto& rv = b->sched->room_of_voice;
         const int vl = b200_voice_len(b->ctx->engine, voice_id);
@@ -465,17 +487,28 @@ static int batch_add_token_job(ptts_batch_t* b, int utt, int voice_id, const int
     if (utt < 0) utt = b->sched->add_utterance();
     BatchScheduler::Job j; j.utt = utt; j.index = b->sched->sentences(utt); j.voice = voice_id; j.temp = temp; j.max_gen = max_gen_len; j.fae = frames_after_eos;
     j.rng_stream = rng_stream; j.ids.assign(ids, ids + n_ids);
+    if (sampling) j.sampling = *sampling;
     b->sched->add_job(std::move(j));
     return utt;
 }
 int ptts_c_batch_add_tokens(ptts_batch_t* b, int voice_id, const int32_t* ids, int n_ids, int max_gen_len, int frames_after_eos, float temp, uint32_t rng_stream) {
     if (!b) return B200_EINVAL;
-    return batch_add_token_job(b, -1, voice_id, ids, n_ids, max_gen_len, frames_after_eos, temp, rng_stream);
+    return batch_add_token_job(b, -1, voice_id, ids, n_ids, max_gen_len, frames_after_eos, temp, rng_stream, nullptr);
+}
+int ptts_c_batch_add_tokens_sampling(ptts_batch_t* b, int voice_id, const int32_t* ids, int n_ids, int max_gen_len, int frames_after_eos, float temp,
+                                     uint32_t rng_stream, const b200_sampling* sampling) {
+    if (!b) return B200_EINVAL;
+    return batch_add_token_job(b, -1, voice_id, ids, n_ids, max_gen_len, frames_after_eos, temp, rng_stream, sampling);
 }
 int ptts_c_batch_append_tokens(ptts_batch_t* b, int utt, int voice_id, const int32_t* ids, int n_ids, int max_gen_len, int frames_after_eos, float temp,
                                uint32_t rng_stream) {
     if (!b || !b->sched->valid_utt(utt) || b->sched->status(utt, nullptr) == BatchScheduler::kCancelled) return B200_EINVAL;
-    return batch_add_token_job(b, utt, voice_id, ids, n_ids, max_gen_len, frames_after_eos, temp, rng_stream);
+    return batch_add_token_job(b, utt, voice_id, ids, n_ids, max_gen_len, frames_after_eos, temp, rng_stream, nullptr);
+}
+int ptts_c_batch_append_tokens_sampling(ptts_batch_t* b, int utt, int voice_id, const int32_t* ids, int n_ids, int max_gen_len, int frames_after_eos,
+                                        float temp, uint32_t rng_stream, const b200_sampling* sampling) {
+    if (!b || !b->sched->valid_utt(utt) || b->sched->status(utt, nullptr) == BatchScheduler::kCancelled) return B200_EINVAL;
+    return batch_add_token_job(b, utt, voice_id, ids, n_ids, max_gen_len, frames_after_eos, temp, rng_stream, sampling);
 }
 long long ptts_c_batch_run(ptts_batch_t* b) { return b ? b->sched->run() : B200_EINVAL; }
 long long ptts_c_batch_pump(ptts_batch_t* b, int max_steps) { return b && max_steps > 0 ? b->sched->pump(max_steps) : B200_EINVAL; }

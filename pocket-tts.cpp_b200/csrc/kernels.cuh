@@ -1031,7 +1031,8 @@ __global__ void __launch_bounds__(256) head_pre_kernel(const float* __restrict__
 
 // noise -> (f32, bf16) per row. Noise is either injected by the caller (identical-noise parity runs, the
 // reference's injection point is GraphContext::normal_, src/context.h:465-509) or drawn on the device from a
-// counter-based generator keyed by (seed, sentence stream id, generation step): Philox-4x32-10 + Box-Muller, std = sqrt(temp).
+// counter-based generator keyed by (seed, sentence stream id, generation step): Philox-4x32-10 + Box-Muller, std = sqrt(temp). A slot
+// with noise_clamp a > 0 draws from N(0, temp) truncated to [-a, a] instead (inverse CDF of the same Philox draw, DESIGN.md 4.7).
 __device__ __forceinline__ void philox4x32_10(uint32_t k0, uint32_t k1, uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3, uint32_t (&out)[4]) {
 #pragma unroll
     for (int r = 0; r < 10; r++) {
@@ -1047,8 +1048,8 @@ __device__ __forceinline__ void philox4x32_10(uint32_t k0, uint32_t k1, uint32_t
 // One CTA (128 threads) per row: the first 32 threads draw the row's noise, then every thread computes 4 of the 512 outputs of
 // input_proj(bf16(noise)) (32 -> 512, reference modules/mlp.h:236; bf16 operands, fp32 accumulation like every linear here).
 __global__ void __launch_bounds__(128) noise_inproj_kernel(int slot0, int n, const float* __restrict__ injected, const unsigned long long* __restrict__ seed_ptr,
-                                                           const float* __restrict__ temp, const int* __restrict__ gen_step, const unsigned int* __restrict__ rng_id,
-                                                           float* __restrict__ noise_f32,
+                                                           const float* __restrict__ temp, const float* __restrict__ clamp, const int* __restrict__ gen_step,
+                                                           const unsigned int* __restrict__ rng_id, float* __restrict__ noise_f32,
                                                            const __nv_bfloat16* __restrict__ w_in_t, const float* __restrict__ b_in, float* __restrict__ xh) {
     pdl_prologue();
     __shared__ float zs[LDIM];
@@ -1067,14 +1068,25 @@ __global__ void __launch_bounds__(128) noise_inproj_kernel(int slot0, int n, con
                 // counter = (sentence stream id, generation step, draw pair): the id defaults to the slot; a batch scheduler sets it to the
                 // sentence's global index so that the audio does not depend on the slot / GPU the sentence happens to land on
                 philox4x32_10((uint32_t)seed, (uint32_t)(seed >> 32), rng_id[slot], (uint32_t)gen_step[slot], (uint32_t)(i >> 1), 0x5054545Au, o);
-                const float u1 = ((float)(o[0] >> 8) + 0.5f) * (1.0f / 16777216.0f);
-                const float u2 = ((float)(o[1] >> 8) + 0.5f) * (1.0f / 16777216.0f);
-                const float rad = sqrtf(-2.0f * logf(u1));
-                float sn, cn; sincosf(6.28318530717958647692f * u2, &sn, &cn);
-                z = ((i & 1) ? rad * sn : rad * cn) * std;
+                const float a = clamp[slot];
+                if (a > 0.f) {
+                    // truncated normal by inverse CDF: lane pair (2k, 2k+1) takes words 0 / 2 of its draw. The lower half of the
+                    // uniform maps to [-a, 0], the upper half mirrors it, so neither tail loses resolution near p = 1.
+                    const float u = ((float)(o[2 * (i & 1)] >> 8) + 0.5f) * (1.0f / 16777216.0f);
+                    const float pl = normcdff(-a / std);
+                    const float h = u < 0.5f ? u : 1.0f - u;
+                    const float zl = fmaxf(std * normcdfinvf(fmaf(h, 1.0f - 2.0f * pl, pl)), -a);
+                    z = u < 0.5f ? zl : -zl;
+                } else {
+                    const float u1 = ((float)(o[0] >> 8) + 0.5f) * (1.0f / 16777216.0f);
+                    const float u2 = ((float)(o[1] >> 8) + 0.5f) * (1.0f / 16777216.0f);
+                    const float rad = sqrtf(-2.0f * logf(u1));
+                    float sn, cn; sincosf(6.28318530717958647692f * u2, &sn, &cn);
+                    z = ((i & 1) ? rad * sn : rad * cn) * std;
+                }
             }
         }
-        noise_f32[r * LDIM + i] = z;
+        if (noise_f32) noise_f32[r * LDIM + i] = z;
         zs[i] = __bfloat162float(__float2bfloat16_rn(z));
     }
     __syncthreads();
@@ -1176,14 +1188,36 @@ __global__ void __launch_bounds__(512) mimi_front_kernel(int slot0, const float*
     }
 }
 
+// Multi-step LSD (DESIGN.md 4.7), substep `sub` of row r with N = lsd_steps[slot] steps: sy = bf16(silu(cond + t_combined(sub/N, (sub+1)/N)))
+// from cond = cond_embed(c) (f32) and the table dtab[(N, sub)] = t_combined(sub/N, (sub+1)/N), and the step weight of the final layer: stepw = 1/N while sub < N, 0 afterwards (x_{i+1} = x_i + v * stepw keeps a finished row's x).
+// At sub = 0 a row with N = 1 keeps the sy of the single-step cond GEMM, so it computes exactly the single-step head. One CTA (128 threads) per row.
+__global__ void __launch_bounds__(128) lsd_time_kernel(int slot0, int n, int sub, const int* __restrict__ lsd_steps, const float* __restrict__ cond,
+                                                       const float* __restrict__ dtab, __nv_bfloat16* __restrict__ sy, float* __restrict__ stepw) {
+    pdl_prologue();
+    const int r = blockIdx.x, i = threadIdx.x;
+    if (r >= n) return;
+    const int N = lsd_steps[slot0 + r];
+    if (i < LDIM) stepw[r * LDIM + i] = sub < N ? 1.0f / (float)N : 0.f;
+    if (sub == 0 && N == 1) return;
+    const float* d = dtab + (long long)(N * (N - 1) / 2 + min(sub, N - 1)) * D_FLOW;
+    for (int c = i * 4; c < D_FLOW; c += 128 * 4) {
+        const float4 y = *reinterpret_cast<const float4*>(cond + (long long)r * D_FLOW + c), t = *reinterpret_cast<const float4*>(d + c);
+        const __nv_bfloat162 a = __floats2bfloat162_rn(apply_act(__fadd_rn(y.x, t.x), ACT_SILU), apply_act(__fadd_rn(y.y, t.y), ACT_SILU));
+        const __nv_bfloat162 b = __floats2bfloat162_rn(apply_act(__fadd_rn(y.z, t.z), ACT_SILU), apply_act(__fadd_rn(y.w, t.w), ACT_SILU));
+        *reinterpret_cast<__nv_bfloat162*>(sy + (long long)r * D_FLOW + c) = a;
+        *reinterpret_cast<__nv_bfloat162*>(sy + (long long)r * D_FLOW + c + 2) = b;
+    }
+}
+
 // Stop rule + bookkeeping after the head (reference src/pocket_tts.cpp:457-467,487-489) and the Mimi front end in one launch. Per slot:
-//   eos_step = first step with logit+4 > 0; stop when gen_step >= eos_step + frames_after_eos; hard cap max_gen_len.
+//   eos_step = first step with logit+4 > eos_thr+4 (eos_thr = -4 by default: the reference's logit > -4, i.e. logit+4 > 0 exactly);
+//   stop when gen_step >= eos_step + frames_after_eos; hard cap max_gen_len.
 // produced[r] = 1 when this step emits a frame. Hands the new latent to the next step (bf16 copy = the A operand of input_linear),
 // advances the FlowLM position, then runs mimi_front_kernel's math on the latent this step produced.
 __global__ void __launch_bounds__(512) step_front_kernel(int slot0, int n, const float* __restrict__ eos, const float* __restrict__ latent,
                                                          int* __restrict__ cur_len, int* __restrict__ gen_step, int* __restrict__ eos_step,
-                                                         const int* __restrict__ max_gen, const int* __restrict__ fae, int* __restrict__ active,
-                                                         __nv_bfloat16* __restrict__ lat_in_bf16, float* __restrict__ lat_f32, int* __restrict__ produced,
+                                                         const int* __restrict__ max_gen, const int* __restrict__ fae, const float* __restrict__ eos_thr,
+                                                         int* __restrict__ active, __nv_bfloat16* __restrict__ lat_in_bf16, float* __restrict__ lat_f32, int* __restrict__ produced,
                                                          float* __restrict__ eos_out, const float* __restrict__ emb_std, const float* __restrict__ emb_mean,
                                                          const __half* __restrict__ wq_t, const float* __restrict__ wup_t, const float* __restrict__ bup,
                                                          float* __restrict__ e_prev, float* __restrict__ x) {
@@ -1197,7 +1231,7 @@ __global__ void __launch_bounds__(512) step_front_kernel(int slot0, int n, const
         if (active[slot]) {
             const int g = gen_step[slot];
             int es = eos_step[slot];
-            if (eos[r] > 0.f && es == -1) es = g;
+            if (eos[r] > eos_thr[slot] + 4.0f && es == -1) es = g;
             eos_step[slot] = es;
             cur_len[slot] += 1;                                   // increment_states (pocket_tts.cpp:96)
             if (es != -1 && g >= es + fae[slot]) { gen_step[slot] = max_gen[slot]; active[slot] = 0; }
