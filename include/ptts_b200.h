@@ -66,13 +66,19 @@ B200_API int  b200_finalize_weights(b200_engine* e);
 B200_API int  b200_voice_create(b200_engine* e, const float* audio_prompt, int T);
 /* Voice cloning (DESIGN.md 4.6; the reference port has no encoder). The checkpoint's encoder set (mimi.encoder.*, mimi.encoder_transformer.*,
  * mimi.downsample.*, flow_lm.speaker_proj_weight) is uploaded by b200_finalize_weights when present; b200_has_encoder tells (1 / 0).
- * pcm: n >= 1 mono float samples at 24 kHz, right-padded with zeros to a multiple of 1920; T = ceil(n / 1920) prompt rows.
- * b200_voice_embed_audio encodes on the engine stream and returns T; with out != NULL ([T][1024]) it copies the audio_prompt rows out
- * (synchronises). b200_voice_create_from_audio encodes and prefills a new voice without a host round trip or wait; returns the voice id.
- * Errors: B200_ENOTFOUND no encoder weights, B200_EINVAL n < 1 or a NULL pointer, B200_ECAPACITY T > kv_capacity or max_voices reached. */
+ * pcm: n >= 1 mono float samples at sample_rate Hz, any integer in [8000, 192000]. Other rates than 24000 are resampled to 24 kHz on the
+ * device (torchaudio.functional.resample with its defaults, DESIGN.md 4.6) into n24 = ceil(24000 n / sample_rate) samples; 24 kHz input
+ * is used as is (n24 = n). The signal is right-padded with zeros to a multiple of 1920; T = ceil(n24 / 1920) prompt rows.
+ * b200_voice_embed_audio_rate encodes on the engine stream and returns T; with out != NULL ([T][1024]) it copies the audio_prompt rows
+ * out (synchronises). b200_voice_create_from_audio_rate encodes and prefills a new voice without a host round trip or wait; returns the
+ * voice id. b200_voice_embed_audio / b200_voice_create_from_audio are these with sample_rate = 24000.
+ * Errors: B200_ENOTFOUND no encoder weights, B200_EINVAL n < 1, a NULL pointer or a sample rate outside [8000, 192000], B200_ECAPACITY
+ * T > kv_capacity or max_voices reached. */
 B200_API int  b200_has_encoder(b200_engine* e);
 B200_API int  b200_voice_embed_audio(b200_engine* e, const float* pcm, long long n, float* out);
 B200_API int  b200_voice_create_from_audio(b200_engine* e, const float* pcm, long long n);
+B200_API int  b200_voice_embed_audio_rate(b200_engine* e, const float* pcm, long long n, int sample_rate, float* out);
+B200_API int  b200_voice_create_from_audio_rate(b200_engine* e, const float* pcm, long long n, int sample_rate);
 
 /* Replaces _stream_sentence_init (src/pocket_tts.cpp:416-444): restore the voice-conditioned KV prefix
  * (copy_states, models/flow_lm.h:70-78), reset the Mimi states (models/mimi.h:71-75), prefill the text tokens,
@@ -166,7 +172,7 @@ B200_API int  b200_read_kv(b200_engine* e, int slot, int layer, int which, int n
 /* Tap points for localising a parity failure (replaces GraphContext::debug, src/context.h:526-547; names follow the tests' CPU restatement):
  * "flow.layer<l>" / "flow.attn<l>" [1024] (need b200_debug_taps(e, 1): steps then run eagerly on one stream), "mimi.upsample" [16*512],
  * "mimi.transformer" [16*512], "seanet.conv0" [16*512], "seanet.convt2" [96*256], "seanet.res3" [96*256], "seanet.res6" [480*128],
- * "seanet.res9" [1920*64] of `slot` after its last step; "enc.seanet" [16T*512], "enc.transformer" [16T*512], "enc.downsample" [T*512] of the
+ * "seanet.res9" [1920*64] of `slot` after its last step; "enc.input" [1920T] (the 24 kHz signal the encoder read), "enc.seanet" [16T*512], "enc.transformer" [16T*512], "enc.downsample" [T*512] of the
  * last clone (any valid slot). out == NULL returns the element count. */
 B200_API int  b200_debug_taps(b200_engine* e, int on);
 B200_API int  b200_debug_tap(b200_engine* e, const char* name, int slot, float* out, int max_elems);
@@ -231,14 +237,15 @@ B200_API int ptts_c_tokenize(ptts_context_t* ctx, const char* text, int32_t* ids
 B200_API int ptts_c_count_words(const char* text);
 /* Pending sentences of a stream after send/flush (conditioners/text.h:207-251); returns count, copies the i-th. */
 B200_API int ptts_c_stream_pending(ptts_stream_t* s, int index, char* buf, int buflen);
-/* Voice cloning through the context. A voice argument ending in ".wav" (RIFF PCM16 or float32, any channel count, mixed down to mono,
- * 24 kHz only) is cloned on first use, like a voice file is loaded. ptts_c_voice_add_audio registers pcm[n] (mono) under `name`, which then
- * works wherever a voice name does; returns the voice id or a B200_E* error (B200_EINVAL for sample_rate != 24000 or a name in use).
+/* Voice cloning through the context. A voice argument ending in ".wav" (RIFF PCM 16 / 24 / 32-bit or float32, any channel count, mixed
+ * down to mono, at its own sample rate in [8000, 192000] Hz) is cloned on first use, like a voice file is loaded. ptts_c_voice_add_audio
+ * registers pcm[n] (mono, at sample_rate Hz) under `name`, which then works wherever a voice name does; returns the voice id or a B200_E*
+ * error (B200_EINVAL for a sample rate outside [8000, 192000] or a name in use).
  * ptts_c_voice_export writes a cloned voice's audio_prompt [1, T, 1024] as an F32 safetensors voice file (B200_ENOTFOUND: not a clone). */
 B200_API int ptts_c_voice_add_audio(ptts_context_t* ctx, const char* name, const float* pcm, long long n, int sample_rate);
 B200_API int ptts_c_voice_export(ptts_context_t* ctx, const char* name, const char* path);
 /* Host-only WAV reader: copies up to max mono samples into pcm (may be NULL), sets *sample_rate (may be NULL); returns the number of
- * samples in the file, or B200_EINVAL for a file that is not a readable RIFF PCM16 / float32 WAV. */
+ * samples in the file, or B200_EINVAL for a file that is not a readable RIFF PCM 16 / 24 / 32-bit or float32 WAV. */
 B200_API int ptts_c_wav_read(const char* path, float* pcm, long long max, int* sample_rate);
 
 /* ---- continuous batching: the batched extension of the streaming API (SURVEY 8b(3)). The reference rolls one stream to its next

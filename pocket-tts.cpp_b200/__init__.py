@@ -180,6 +180,8 @@ def lib():
         "b200_debug_window_attention": (ci, [vp, ci, fp, fp, fp, fp]),
         "b200_voice_embed_audio": (ci, [vp, fp, ctypes.c_longlong, fp]),
         "b200_voice_create_from_audio": (ci, [vp, fp, ctypes.c_longlong]),
+        "b200_voice_embed_audio_rate": (ci, [vp, fp, ctypes.c_longlong, ci, fp]),
+        "b200_voice_create_from_audio_rate": (ci, [vp, fp, ctypes.c_longlong, ci]),
         "ptts_c_voice_add_audio": (ci, [vp, cp, fp, ctypes.c_longlong, ci]),
         "ptts_c_voice_export": (ci, [vp, cp, cp]),
         "ptts_c_wav_read": (ci, [cp, fp, ctypes.c_longlong, ctypes.POINTER(ctypes.c_int)]),
@@ -236,14 +238,17 @@ class Engine:
         """True when the checkpoint carries the voice-cloning encoder."""
         return self.L.b200_has_encoder(self.h) == 1
 
-    def embed_audio(self, pcm) -> np.ndarray:
-        """Mono 24 kHz PCM -> audio_prompt rows [T, 1024] (T = ceil(n / 1920)), encoded on the device."""
+    def embed_audio(self, pcm, sample_rate: int = SAMPLE_RATE) -> np.ndarray:
+        """Mono PCM at sample_rate Hz (any integer in [8000, 192000]; resampled to 24 kHz on the device) -> audio_prompt rows [T, 1024]
+        (T = ceil(n24 / 1920), n24 = ceil(24000 n / sample_rate)), encoded on the device."""
         x = np.ascontiguousarray(np.asarray(pcm, np.float32).reshape(-1))
-        T = -(-len(x) // FRAME)
+        sr = int(sample_rate)
+        n24 = -(-len(x) * SAMPLE_RATE // sr) if sr > 0 else 0   # an invalid rate is refused by the call
+        T = -(-n24 // FRAME)
         out = np.zeros((max(T, 1), 1024), np.float32)
-        rc = self.L.b200_voice_embed_audio(self.h, _fp(x) if len(x) else None, len(x), _fp(out))
+        rc = self.L.b200_voice_embed_audio_rate(self.h, _fp(x) if len(x) else None, len(x), sr, _fp(out))
         if rc < 0:
-            raise RuntimeError(f"b200_voice_embed_audio failed: {rc}")
+            raise RuntimeError(f"b200_voice_embed_audio_rate failed: {rc}")
         return out[:rc]
 
     def debug_window_attention(self, q, k, v) -> np.ndarray:
@@ -255,12 +260,13 @@ class Engine:
             raise RuntimeError(f"b200_debug_window_attention failed: {rc}")
         return out
 
-    def voice_from_audio(self, pcm) -> int:
-        """Clones a voice from mono 24 kHz PCM: encode + prefill on the device; returns the voice id."""
+    def voice_from_audio(self, pcm, sample_rate: int = SAMPLE_RATE) -> int:
+        """Clones a voice from mono PCM at sample_rate Hz (any integer in [8000, 192000]): resample + encode + prefill on the device;
+        returns the voice id."""
         x = np.ascontiguousarray(np.asarray(pcm, np.float32).reshape(-1))
-        v = self.L.b200_voice_create_from_audio(self.h, _fp(x) if len(x) else None, len(x))
+        v = self.L.b200_voice_create_from_audio_rate(self.h, _fp(x) if len(x) else None, len(x), int(sample_rate))
         if v < 0:
-            raise RuntimeError(f"b200_voice_create_from_audio failed: {v}")
+            raise RuntimeError(f"b200_voice_create_from_audio_rate failed: {v}")
         return v
 
     def begin_sentence(self, slot, voice, tokens, max_gen_len, frames_after_eos, temp=0.0):
@@ -513,7 +519,8 @@ class Context:
         return s
 
     def add_voice(self, name: str, pcm, sample_rate: int = SAMPLE_RATE) -> int:
-        """Clones a voice from mono PCM (24 kHz only) and registers it under `name`; returns the engine voice id."""
+        """Clones a voice from mono PCM at sample_rate Hz (any integer in [8000, 192000]; resampled to 24 kHz on the device) and
+        registers it under `name`; returns the engine voice id."""
         x = np.ascontiguousarray(np.asarray(pcm, np.float32).reshape(-1))
         v = lib().ptts_c_voice_add_audio(self.h, name.encode(), _fp(x) if len(x) else None, len(x), int(sample_rate))
         if v < 0:
@@ -678,11 +685,12 @@ class Stream:
 
 
 def read_wav(path: str):
-    """Host-only RIFF reader of the engine (PCM16 / float32, mixed down to mono): (samples float32 [n], sample_rate)."""
+    """Host-only RIFF reader of the engine (integer PCM of 16, 24 or 32 bits, or float32; mixed down to mono): (samples float32 [n],
+    sample_rate). The rate is the file's; every voice-cloning call takes it as is."""
     rate = ctypes.c_int()
     n = lib().ptts_c_wav_read(path.encode(), None, 0, ctypes.byref(rate))
     if n < 0:
-        raise ValueError(f"{path}: not a readable PCM16 / float32 WAV file")
+        raise ValueError(f"{path}: not a readable PCM 16 / 24 / 32-bit or float32 WAV file")
     out = np.zeros(max(n, 1), np.float32)
     lib().ptts_c_wav_read(path.encode(), _fp(out), n, ctypes.byref(rate))
     return out[:n], rate.value

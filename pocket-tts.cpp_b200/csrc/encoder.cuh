@@ -1,7 +1,8 @@
-// encoder.cuh — kernels of the voice-cloning encoder (DESIGN.md §4.6): 24 kHz PCM -> SEANet encoder -> encoder transformer -> strided
+// encoder.cuh — kernels of the voice-cloning encoder (DESIGN.md §4.6): PCM resampled to 24 kHz -> SEANet encoder -> encoder transformer -> strided
 // downsample -> speaker projection -> audio_prompt rows. Everything that is a GEMM runs through the engine's GEMM family (strided convs as
 // 2-tap windows over rows of r*C channels); the kernels here are the pieces that are not a GEMM.
 #pragma once
+#include <algorithm>
 #include "common.cuh"
 
 namespace ptts {
@@ -9,6 +10,83 @@ namespace ptts {
 constexpr int ENC_WIN = M_CTX;               // encoder attention: key j is visible to query i iff 0 <= i - j < ENC_WIN
 constexpr int ENC_HOP = 1920;                // samples per 12.5 Hz output row
 constexpr int ENC_FRONT_K = 7;
+constexpr int ENC_SR = 24000, ENC_SR_MIN = 8000, ENC_SR_MAX = 192000;   // the encoder's rate; accepted input rates (integers)
+
+// ---- resampling to 24 kHz in front of the encoder: torchaudio.functional.resample(x, sr, 24000) with its defaults (sinc_interp_hann,
+// lowpass_filter_width L = 6, rolloff 0.99), its float64 filter rounded to f32. With o = sr / g and m = 24000 / g (g = gcd), output
+// j = q m + i is sum_k K[i][k] xpad[q o + k], xpad = [w zeros | x | w + o zeros], w = ceil(L o / base), base = 0.99 min(o, m), and
+// K[i][k] = sinc(pi t) cos^2(pi t / 2L) base / o with t = ((k - w) / o - i / m) base clamped to +-L. A tap is nonzero in f32 only for
+// |t| < L, i.e. |(k - w) m - i o| <= X = floor(600 max(o, m) / 99) (exact integers), so phase i is a band of taps starting at
+// d = k - w = ceil((i o - X) / m): output j reads x[s(j) .. s(j) + W - 1] with s(j) = ceil((j o - X) / m), and W is the widest band.
+constexpr int RS_L = 6, RS_THREADS = 256;
+
+__host__ __device__ inline long long rs_ceil_div(long long a, long long b) { return a >= 0 ? (a + b - 1) / b : -((-a) / b); }
+__host__ __device__ inline long long rs_floor_div(long long a, long long b) { return a >= 0 ? a / b : -((-a + b - 1) / b); }
+
+struct ResamplePlan {
+    int sr = 0, o = 0, m = 0, w = 0, W = 0; long long X = 0;
+    long long first_tap(long long j) const { return rs_ceil_div(j * o - X, m); }
+    int span_max() const { return (int)rs_ceil_div((long long)(RS_THREADS - 1) * o, m) + W; }   // input samples one CTA stages
+};
+inline ResamplePlan resample_plan(int sr) {
+    ResamplePlan p; p.sr = sr;
+    long long a = sr, b = ENC_SR;
+    while (b) { const long long r = a % b; a = b; b = r; }
+    p.o = (int)(sr / a); p.m = (int)(ENC_SR / a);
+    const double base = (double)std::min(p.o, p.m) * 0.99;
+    p.w = (int)std::ceil((double)(RS_L * p.o) / base);
+    p.X = 600LL * std::max(p.o, p.m) / 99;
+    for (int i = 0; i < p.m; i++)
+        p.W = std::max(p.W, (int)(rs_floor_div((long long)i * p.o + p.X, p.m) - rs_ceil_div((long long)i * p.o - p.X, p.m) + 1));
+    return p;
+}
+
+// coef[i][b] = K[i][w + ceil((i o - X) / m) + b] for b < W (0 past the phase's band), evaluated in float64 in torchaudio's operation
+// order and rounded once.
+__global__ void resample_table_kernel(int o, int m, int w, int W, long long X, float* __restrict__ coef) {
+    const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (idx >= (long long)m * W) return;
+    const int i = (int)(idx / W), b = (int)(idx % W);
+    const long long d = rs_ceil_div((long long)i * o - X, m) + b;
+    float c = 0.f;
+    if (d <= rs_floor_div((long long)i * o + X, m) && d >= -w && d < w + o) {
+        const double base = (double)min(o, m) * 0.99;
+        double t = (double)(-i) / m + (double)d / o;
+        t *= base;
+        t = fmin(fmax(t, -(double)RS_L), (double)RS_L);
+        const double cw = cos(t * M_PI / RS_L / 2), window = cw * cw;
+        t *= M_PI;
+        double k = t == 0.0 ? 1.0 : sin(t) / t;
+        k *= window * (base / o);
+        c = __double2float_rn(k);
+    }
+    coef[idx] = c;
+}
+
+// One thread per 24 kHz output y[j], j < L0 (= 1920 T): sum_b coef[j % m][b] x[s(j) + b] over the band in increasing b (f32 FMA), x = 0
+// outside [0, n); outputs n24 .. L0-1 are the encoder's zero right padding. Each CTA stages the input span its 256 outputs read.
+__global__ void __launch_bounds__(RS_THREADS) resample_kernel(const float* __restrict__ x, long long n, const float* __restrict__ coef, int o, int m,
+                                                             int W, long long X, long long n24, long long L0, float* __restrict__ y) {
+    extern __shared__ float rs_span[];
+    const long long j0 = (long long)blockIdx.x * RS_THREADS, j = j0 + threadIdx.x;
+    if (j0 >= n24) { if (j < L0) y[j] = 0.f; return; }
+    const long long s0 = rs_ceil_div(j0 * o - X, m), jl = min(j0 + RS_THREADS, n24) - 1;
+    const int span = (int)(rs_ceil_div(jl * o - X, m) + W - s0);
+    for (int p = threadIdx.x; p < span; p += RS_THREADS) {
+        const long long g = s0 + p;
+        rs_span[p] = g >= 0 && g < n ? x[g] : 0.f;
+    }
+    __syncthreads();
+    if (j < n24) {
+        const float* c = coef + (j % m) * W;
+        const float* xs = rs_span + (rs_ceil_div(j * o - X, m) - s0);
+        float acc = 0.f;
+        for (int b = 0; b < W; b++) acc = fmaf(c[b], xs[b], acc);
+        y[j] = acc;
+    } else if (j < L0) {
+        y[j] = 0.f;
+    }
+}
 
 // Front conv k7 1 -> 64 (C = 1 is no GEMM: K % 64 != 0). pcm = 6 zero samples of causal padding followed by the (zero-padded) signal.
 // y[t][c] = b[c] + sum_j w[c][j] * f16(pcm[t + j]) (f16 operands, f32 accumulation like every conv); writes the f32 residual row and

@@ -1012,6 +1012,25 @@ struct b200_engine {
     // Pinned staging of the clone's PCM, sized with the scratch. Not the shared pinned ring: a 10 s prompt is ~1 MB, and growing a ring
     // slot to that size (cudaFreeHost + cudaMallocHost) on most clones stalls the serving pipeline.
     float* enc_pin = nullptr; size_t enc_pin_cap = 0; cudaEvent_t enc_pin_ev = nullptr; bool enc_pin_used = false;
+    // Input at another rate than 24 kHz: its samples on the device, and the coefficient table [m][W] of the last clone's rate (rebuilt
+    // in stream order when the rate changes; a grown buffer leaves the old one to the kernels still queued on it).
+    float* enc_raw = nullptr; size_t enc_raw_cap = 0;
+    float* rs_coef = nullptr; size_t rs_coef_cap = 0; ResamplePlan rs_plan;
+    // Resamples n samples at sr Hz (in enc_raw) into eb.pcm + 6: n24 samples, then zeros up to L0. Main stream, no host wait.
+    void resample_to_24k(int sr, long long n, long long n24, long long L0) {
+        if (rs_plan.sr != sr) {
+            rs_plan = resample_plan(sr);
+            const long long nc = (long long)rs_plan.m * rs_plan.W;
+            grow(rs_coef, rs_coef_cap, (size_t)nc);
+            launch_k(false, resample_table_kernel, dim3((unsigned)((nc + 255) / 256)), dim3(256), (size_t)0, stream, rs_plan.o, rs_plan.m, rs_plan.w,
+                     rs_plan.W, rs_plan.X, rs_coef);
+            launches++;
+        }
+        const ResamplePlan& p = rs_plan;
+        launch_k(false, resample_kernel, dim3((unsigned)((L0 + RS_THREADS - 1) / RS_THREADS)), dim3(RS_THREADS), (size_t)p.span_max() * sizeof(float), stream,
+                 (const float*)enc_raw, n, (const float*)rs_coef, p.o, p.m, p.W, p.X, n24, L0, eb.pcm + 6);
+        launches++;
+    }
     void enc_reserve(int T) {
         if (T <= eb.T) return;
         const int Tc = std::min(std::max(T, 2 * eb.T), cfg.kv_capacity);   // no clone is longer than kv_capacity rows
@@ -1030,7 +1049,7 @@ struct b200_engine {
         for (auto& pp : parts) *pp.first = base + pp.second;
         eb.T = Tc;
     }
-    // Encodes pcm (already in eb.pcm behind 6 zero samples, zero-padded to 1920 T) into eb.prompt [T][1024]. Main stream, no host wait.
+    // Encodes 24 kHz pcm (already in eb.pcm behind 6 zero samples, zero-padded to 1920 T) into eb.prompt [T][1024]. Main stream, no host wait.
     void encode(int T) {
         const int BIG = 1 << 30;
         const long long L0 = (long long)ENC_HOP * T, L1 = L0 / 4, L2 = L1 / 5, L3 = L2 / 6;
@@ -1575,44 +1594,54 @@ int b200_voice_create(b200_engine* e, const float* audio_prompt, int T) {
 
 int b200_has_encoder(b200_engine* e) { return e && e->finalized && e->has_enc ? 1 : 0; }
 
-// Voice cloning: uploads the PCM through the pinned ring and enqueues the encoder on the main stream (no host wait). Returns T.
-static int enc_enqueue(b200_engine* e, const float* pcm, long long n) {
-    if (!e || !e->finalized || !pcm || n < 1) return B200_EINVAL;
+// Voice cloning: uploads the PCM through the encoder's pinned staging, resamples it to 24 kHz when sr differs and enqueues the encoder
+// on the main stream (no host wait). Returns T.
+static int enc_enqueue(b200_engine* e, const float* pcm, long long n, int sr) {
+    if (!e || !e->finalized || !pcm || n < 1 || sr < ENC_SR_MIN || sr > ENC_SR_MAX) return B200_EINVAL;
     if (!e->has_enc) return B200_ENOTFOUND;
-    const long long T = (n + ENC_HOP - 1) / ENC_HOP;
-    if (T > e->cfg.kv_capacity) return B200_ECAPACITY;
+    // T = ceil(n24 / 1920) <= kv_capacity  <=>  n24 = ceil(24000 n / sr) <= 1920 kv_capacity  <=>  n <= floor(1920 kv_capacity sr / 24000)
+    if (n > (long long)ENC_HOP * e->cfg.kv_capacity * sr / ENC_SR) return B200_ECAPACITY;
+    const long long n24 = (n * ENC_SR + sr - 1) / sr;
+    const long long T = (n24 + ENC_HOP - 1) / ENC_HOP;
     PTTS_CUDA_CHECK(cudaSetDevice(e->cfg.device));
     e->enc_reserve((int)T);
     const long long L0 = T * ENC_HOP;
     if (!e->enc_pin_ev) PTTS_CUDA_CHECK(cudaEventCreateWithFlags(&e->enc_pin_ev, cudaEventDisableTiming));
     if (e->enc_pin_used) PTTS_CUDA_CHECK(cudaEventSynchronize(e->enc_pin_ev));   // the previous clone's upload (long done in steady state)
-    if (e->enc_pin_cap < (size_t)n) {
+    if (e->enc_pin_cap < (size_t)n) {               // sized with the scratch: eb.T rows at sr hold at least n samples
         if (e->enc_pin) PTTS_CUDA_CHECK(cudaFreeHost(e->enc_pin));
-        e->enc_pin_cap = (size_t)e->eb.T * ENC_HOP;
+        e->enc_pin_cap = (size_t)((long long)e->eb.T * ENC_HOP * sr / ENC_SR);
         PTTS_CUDA_CHECK(cudaMallocHost(&e->enc_pin, e->enc_pin_cap * sizeof(float)));
     }
     memcpy(e->enc_pin, pcm, (size_t)n * sizeof(float));
-    PTTS_CUDA_CHECK(cudaMemcpyAsync(e->eb.pcm + 6, e->enc_pin, (size_t)n * sizeof(float), cudaMemcpyHostToDevice, e->stream));
+    if (sr != ENC_SR) e->grow(e->enc_raw, e->enc_raw_cap, (size_t)n);
+    PTTS_CUDA_CHECK(cudaMemcpyAsync(sr == ENC_SR ? e->eb.pcm + 6 : e->enc_raw, e->enc_pin, (size_t)n * sizeof(float), cudaMemcpyHostToDevice, e->stream));
     PTTS_CUDA_CHECK(cudaEventRecord(e->enc_pin_ev, e->stream));
     e->enc_pin_used = true;
-    if (L0 > n) PTTS_CUDA_CHECK(cudaMemsetAsync(e->eb.pcm + 6 + n, 0, (size_t)(L0 - n) * sizeof(float), e->stream));
+    if (sr != ENC_SR) e->resample_to_24k(sr, n, n24, L0);
+    else if (L0 > n) PTTS_CUDA_CHECK(cudaMemsetAsync(e->eb.pcm + 6 + n, 0, (size_t)(L0 - n) * sizeof(float), e->stream));
     e->encode((int)T);
     return (int)T;
 }
 
-int b200_voice_embed_audio(b200_engine* e, const float* pcm, long long n, float* out) {
+int b200_voice_embed_audio(b200_engine* e, const float* pcm, long long n, float* out) { return b200_voice_embed_audio_rate(e, pcm, n, ENC_SR, out); }
+
+int b200_voice_embed_audio_rate(b200_engine* e, const float* pcm, long long n, int sample_rate, float* out) {
     NvtxRange nvtx_range("ptts.voice_embed_audio");
-    const int T = enc_enqueue(e, pcm, n);
+    const int T = enc_enqueue(e, pcm, n, sample_rate);
     if (T < 0 || !out) return T;
     PTTS_CUDA_CHECK(cudaMemcpyAsync(out, e->eb.prompt, (size_t)T * D_MODEL * sizeof(float), cudaMemcpyDeviceToHost, e->stream));
     PTTS_CUDA_CHECK(cudaStreamSynchronize(e->stream));
     return T;
 }
 
-int b200_voice_create_from_audio(b200_engine* e, const float* pcm, long long n) {
+int b200_voice_create_from_audio(b200_engine* e, const float* pcm, long long n) { return b200_voice_create_from_audio_rate(e, pcm, n, ENC_SR); }
+
+int b200_voice_create_from_audio_rate(b200_engine* e, const float* pcm, long long n, int sample_rate) {
     NvtxRange nvtx_range("ptts.voice_create_from_audio");
-    if (e && e->finalized && e->has_enc && pcm && n >= 1 && e->n_voices >= e->cfg.max_voices) return B200_ECAPACITY;
-    const int T = enc_enqueue(e, pcm, n);
+    if (e && e->finalized && e->has_enc && pcm && n >= 1 && sample_rate >= ENC_SR_MIN && sample_rate <= ENC_SR_MAX && e->n_voices >= e->cfg.max_voices)
+        return B200_ECAPACITY;
+    const int T = enc_enqueue(e, pcm, n, sample_rate);
     if (T < 0) return T;
     const int v = e->n_voices++;
     const int slot = e->cfg.max_slots + v;
@@ -2234,6 +2263,7 @@ int b200_debug_tap(b200_engine* e, const char* name, int slot, float* out, int m
     if (s == "seanet.res3") return give_16(e->buf5, true, 97LL * e->C5, 1, 96, e->C5, 256);
     if (s == "seanet.res6") return give_16(e->buf8, true, 481LL * e->C8, 1, 480, e->C8, 128);
     if (s == "seanet.res9") return give_16(e->buf11, true, 1922LL * 64, 2, 1920, 64, 64);
+    if (s == "enc.input") return give_f32(e->eb.pcm + 6, (size_t)e->enc_T * ENC_HOP);
     if (s == "enc.seanet") return give_f32(e->eb.xs, (size_t)e->enc_T * M_T * M_DIM);          // the last clone's buffers (slot ignored)
     if (s == "enc.transformer") return give_f32(e->eb.xt, (size_t)e->enc_T * M_T * M_DIM);
     if (s == "enc.downsample") return give_f32(e->eb.lat, (size_t)e->enc_T * M_DIM);

@@ -65,14 +65,17 @@ struct SentenceSplitter {
 unsigned int g_seed = 0x5eed5eedu;
 bool g_seed_set = false;
 
+const int kMinRate = 8000, kMaxRate = 192000;   // input sample rates the voice encoder accepts (b200_voice_embed_audio_rate)
+
 const char* kVoices[] = {"alba", "azelma", "cosette", "eponine", "fantine", "javert", "jean", "marius"};
 
 int env_int(const char* name, int dflt) { const char* v = getenv(name); return v && *v ? atoi(v) : dflt; }
 
 bool ends_with(const std::string& s, const char* suffix) { const size_t n = strlen(suffix); return s.size() >= n && s.compare(s.size() - n, n, suffix) == 0; }
 
-// RIFF/WAVE reader: PCM16 or float32 (format 1 / 3, or WAVE_FORMAT_EXTENSIBLE with either subformat), any channel count, mixed down
-// to mono by averaging. Returns false for anything else, including a data chunk that runs past the end of the file.
+// RIFF/WAVE reader: integer PCM of 16, 24 or 32 bits or float32 (format 1 / 3, or WAVE_FORMAT_EXTENSIBLE with either subformat), any
+// channel count, mixed down to mono by averaging. Integer samples scale by 2^-(bits-1). Returns false for anything else, including a data
+// chunk that runs past the end of the file.
 bool read_wav(const std::string& path, std::vector<float>& out, int& sample_rate) {
     FILE* f = fopen(path.c_str(), "rb");
     if (!f) return false;
@@ -95,16 +98,19 @@ bool read_wav(const std::string& path, std::vector<float>& out, int& sample_rate
             have_fmt = true;
         } else if (memcmp(b.data() + o, "data", 4) == 0) {
             if (!have_fmt || channels < 1) return false;
-            const bool pcm16 = fmt == 1 && bits == 16, f32 = fmt == 3 && bits == 32;
-            if (!pcm16 && !f32) return false;
-            const size_t frame_bytes = (size_t)channels * (bits / 8), n = sz / frame_bytes;
+            const bool pcm = fmt == 1 && (bits == 16 || bits == 24 || bits == 32), f32 = fmt == 3 && bits == 32;
+            if (!pcm && !f32) return false;
+            const size_t bytes = (size_t)bits / 8, frame_bytes = (size_t)channels * bytes, n = sz / frame_bytes;
+            const double scale = 1.0 / (double)(1u << (bits - 1));   // 2^-(bits-1) for integer PCM
             out.assign(n, 0.f);
             for (size_t i = 0; i < n; i++) {
                 double acc = 0;
                 for (int c = 0; c < channels; c++) {
-                    const size_t at = body + i * frame_bytes + (size_t)c * (bits / 8);
-                    if (pcm16) acc += (int16_t)u16(at) / 32768.0;
-                    else { float v; memcpy(&v, b.data() + at, 4); acc += v; }
+                    const size_t at = body + i * frame_bytes + (size_t)c * bytes;
+                    if (f32) { float v; memcpy(&v, b.data() + at, 4); acc += v; }
+                    else if (bits == 16) acc += (int16_t)u16(at) * scale;
+                    else if (bits == 24) acc += (double)((int32_t)((u16(at) | ((uint32_t)b[at + 2] << 16)) << 8) >> 8) * scale;
+                    else acc += (double)(int32_t)u32(at) * scale;
                 }
                 out[i] = (float)(acc / channels);
             }
@@ -203,12 +209,14 @@ ptts_context_t* ptts_init(ggml_backend*, ggml_backend*, const char* model_path) 
 int ptts_get_sample_rate(ptts_context_t*) { return 24000; }   // reference :324-326
 int ptts_get_frame_size(ptts_context_t*) { return 1920; }     // reference :328-330
 
-// Clones a voice from mono 24 kHz PCM and registers it under `name`. The rows come back to the host once, so that the voice can be exported.
-static int add_audio_voice(ptts_context_t* ctx, const std::string& name, const float* pcm, long long n) {
-    const long long T = (n + 1919) / 1920;
-    if (n < 1 || T > b200_kv_capacity(ctx->engine)) return n < 1 ? B200_EINVAL : B200_ECAPACITY;
+// Clones a voice from mono PCM at sample_rate Hz (resampled to 24 kHz on the device) and registers it under `name`. The rows come back to
+// the host once, so that the voice can be exported.
+static int add_audio_voice(ptts_context_t* ctx, const std::string& name, const float* pcm, long long n, int sample_rate) {
+    if (n < 1) return B200_EINVAL;
+    if (n > 1920LL * b200_kv_capacity(ctx->engine) * sample_rate / 24000) return B200_ECAPACITY;   // T > kv_capacity
+    const long long n24 = (n * 24000 + sample_rate - 1) / sample_rate, T = (n24 + 1919) / 1920;
     std::vector<float> prompt((size_t)T * 1024);
-    const int t = b200_voice_embed_audio(ctx->engine, pcm, n, prompt.data());
+    const int t = b200_voice_embed_audio_rate(ctx->engine, pcm, n, sample_rate, prompt.data());
     if (t < 0) return t;
     const int vid = b200_voice_create(ctx->engine, prompt.data(), t);
     if (vid < 0) return vid;
@@ -218,7 +226,7 @@ static int add_audio_voice(ptts_context_t* ctx, const std::string& name, const f
 }
 
 // Voice name or path -> engine voice id; the first use loads the file and prefills the prefix (reference src/pocket_tts.cpp:356-359,100-124).
-// A path ending in ".wav" is a recording: it is cloned (add_audio_voice).
+// A path ending in ".wav" is a recording: it is cloned at its own sample rate (add_audio_voice).
 static int resolve_voice(ptts_context_t* ctx, const char* voice_c_str) {
     std::string voice = voice_c_str;
     for (const char* v : kVoices) if (voice == v) { voice = ctx->model_path + "embeddings/" + v + ".safetensors"; break; }
@@ -228,8 +236,10 @@ static int resolve_voice(ptts_context_t* ctx, const char* voice_c_str) {
     else if (ends_with(voice, ".wav")) {
         std::vector<float> pcm; int rate = 0;
         if (!read_wav(voice, pcm, rate)) { fprintf(stderr, "error: failed to open voice %s\n", voice.c_str()); exit(1); }
-        if (rate != 24000) { fprintf(stderr, "error: voice %s: sample rate %d Hz, the encoder takes 24000 Hz\n", voice.c_str(), rate); exit(1); }
-        vid = add_audio_voice(ctx, voice, pcm.data(), (long long)pcm.size());
+        if (rate < kMinRate || rate > kMaxRate) {
+            fprintf(stderr, "error: voice %s: sample rate %d Hz, the encoder takes %d to %d Hz\n", voice.c_str(), rate, kMinRate, kMaxRate); exit(1);
+        }
+        vid = add_audio_voice(ctx, voice, pcm.data(), (long long)pcm.size(), rate);
         if (vid < 0) { fprintf(stderr, "error: failed to clone voice %s (%d)\n", voice.c_str(), vid); exit(1); }
     } else {
         SafeTensors st;
@@ -365,10 +375,10 @@ int ptts_c_tokenize(ptts_context_t* c, const char* text, int32_t* ids, int max_i
 }
 int ptts_c_count_words(const char* text) { return count_words_impl(text); }
 int ptts_c_voice_add_audio(ptts_context_t* c, const char* name, const float* pcm, long long n, int sample_rate) {
-    if (!c || !name || !pcm || sample_rate != 24000 || c->voices.count(name)) return B200_EINVAL;
+    if (!c || !name || !pcm || sample_rate < kMinRate || sample_rate > kMaxRate || c->voices.count(name)) return B200_EINVAL;
     for (const char* v : kVoices) if (strcmp(name, v) == 0) return B200_EINVAL;   // resolve_voice maps these to the model's voice files first
     if (!b200_has_encoder(c->engine)) return B200_ENOTFOUND;
-    return add_audio_voice(c, name, pcm, n);
+    return add_audio_voice(c, name, pcm, n, sample_rate);
 }
 int ptts_c_voice_export(ptts_context_t* c, const char* name, const char* path) {
     if (!c || !name || !path) return B200_EINVAL;

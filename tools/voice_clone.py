@@ -10,7 +10,14 @@
     (b200_voice_create_from_audio) every N pumps against none.
 (e) the float64 torch restatement's CPU time (tests/encoder_ref.py) for 1 and 10 s, as context.
 
+With --rates, recordings at other rates than 24 kHz instead (profiles/voice_clone_rates_b200.json):
+(f) the device resampler alone (resample_kernel, from torch.profiler's CUDA kernel records) for 10 / 30 s at 16 / 44.1 / 48 / 96 kHz,
+    medians after a warm-up, and the bytes it moves (input read + table + 24 kHz output written) over that time;
+(g) encode + prefill device time and wall time to a voice id for 10 s at 24 / 44.1 / 48 kHz, as in (a);
+(h) as (d): a 10 s 24 kHz and a 10 s 44.1 kHz clone every 50 pumps against none, in alternating rounds (medians).
+
     python tools/voice_clone.py --out profiles/voice_clone_b200.json
+    python tools/voice_clone.py --rates --out profiles/voice_clone_rates_b200.json
 """
 from __future__ import annotations
 
@@ -51,7 +58,11 @@ def main():
     ap.add_argument("--batch-steps", type=int, default=600)
     ap.add_argument("--clone-every", default="50,150")
     ap.add_argument("--out", default=None)
+    ap.add_argument("--rates", action="store_true", help="measure recordings at other sample rates (f, g, h)")
+    ap.add_argument("--rounds", type=int, default=3, help="--rates: alternating rounds of the batch-cost runs")
     a = ap.parse_args()
+    if a.rates:
+        return emit(measure_rates(a), a.out)
 
     import torch
     import ptts_b200 as P
@@ -107,28 +118,9 @@ def main():
     c.close()
 
     # (d) cost to a running 256-slot batch
-    from test_gpu_batch import TEXTS
-    words = " ".join(TEXTS).split()
     costs = {}
     for every in [0] + [int(v) for v in a.clone_every.split(",")]:
-        c = P.Context(md, max_slots=256, max_voices=2 + (a.batch_steps // every if every else 0), kv_capacity=1024)
-        P.set_seed(1)
-        b = P.Batch(c)
-        r = np.random.default_rng(2)
-        for i in range(1024):
-            n = int(r.integers(3, 30))
-            b.add("cosette", " ".join(words[(7 * i + j) % len(words)] for j in range(n)) + ".", temp=0.7)
-        for _ in range(20):
-            b.pump(1)
-        clones, frames, t0 = 0, 0, time.perf_counter()
-        for step in range(a.batch_steps):
-            if every and step % every == every - 1:
-                c.engine.voice_from_audio(pcm[10]); clones += 1
-            frames += b.pump(1)
-        dt = time.perf_counter() - t0
-        costs["none" if not every else f"every_{every}"] = {"frames_per_s": frames / dt, "frames": frames, "clones": clones, "seconds": dt}
-        del b
-        c.close()
+        costs["none" if not every else f"every_{every}"] = batch_fps(P, md, every, a.batch_steps, lambda e: e.voice_from_audio(pcm[10]))
     res["batch_cost"] = costs
 
     # (e) CPU restatement
@@ -140,11 +132,117 @@ def main():
         t0 = time.perf_counter(); ref.embed(pcm[s]); cpu[f"{s}s"] = (time.perf_counter() - t0) * 1e3
     res["cpu_restatement_ms"] = {"torch_threads": torch.get_num_threads(), **cpu}
 
+    emit(res, a.out)
+
+
+def emit(res, out):
     txt = json.dumps(res, indent=1)
     print(txt)
-    if a.out:
-        os.makedirs(os.path.dirname(os.path.abspath(a.out)), exist_ok=True)
-        open(a.out, "w").write(txt + "\n")
+    if out:
+        os.makedirs(os.path.dirname(os.path.abspath(out)), exist_ok=True)
+        open(out, "w").write(txt + "\n")
+
+
+def batch_fps(P, md, every, steps, clone):
+    """frames/s of a 256-slot ragged online batch driven by pump(1), calling clone() every `every` pumps (0: never)."""
+    from test_gpu_batch import TEXTS
+    words = " ".join(TEXTS).split()
+    c = P.Context(md, max_slots=256, max_voices=2 + (steps // every if every else 0), kv_capacity=1024)
+    P.set_seed(1)
+    b = P.Batch(c)
+    r = np.random.default_rng(2)
+    for i in range(1024):
+        n = int(r.integers(3, 30))
+        b.add("cosette", " ".join(words[(7 * i + j) % len(words)] for j in range(n)) + ".", temp=0.7)
+    for _ in range(20):
+        b.pump(1)
+    clones, frames, t0 = 0, 0, time.perf_counter()
+    for step in range(steps):
+        if every and step % every == every - 1:
+            clone(c.engine); clones += 1
+        frames += b.pump(1)
+    dt = time.perf_counter() - t0
+    del b
+    c.close()
+    return {"frames_per_s": frames / dt, "frames": frames, "clones": clones, "seconds": dt}
+
+
+def measure_rates(a):
+    import torch
+    import ptts_b200 as P
+    import resample_ref as R
+    from make_assets import default_model_dir
+    from online_batch import gpu_info
+    assert torch.cuda.is_available(), "needs a CUDA device"
+    res = {"gpu_info": gpu_info(0)}
+    md = default_model_dir(eos_mode="never", encoder=True)
+    L = P.lib()
+    fp = lambda x: x.ctypes.data_as(ctypes.POINTER(ctypes.c_float))
+    med = lambda v: float(np.median(v))
+    rng = np.random.default_rng(0)
+    noise = lambda n: (0.3 * rng.standard_normal(n)).astype(np.float32)
+
+    # (f) the resampler alone. Each clone of a rate reuses its table (built by the warm-up), so resample_kernel is the only added kernel.
+    c = P.Context(md, max_slots=1, max_voices=2, kv_capacity=1024)
+    eng = c.engine
+    rs = {}
+    for sr in (16000, 44100, 48000, 96000):
+        for s in (10, 30):
+            x = noise(s * sr)
+            for _ in range(3):
+                assert L.b200_voice_embed_audio_rate(eng.h, fp(x), len(x), sr, None) > 0
+            eng.sync()
+            with torch.profiler.profile(activities=[torch.profiler.ProfilerActivity.CUDA]) as prof:
+                for _ in range(a.reps):
+                    L.b200_voice_embed_audio_rate(eng.h, fp(x), len(x), sr, None)
+                eng.sync()
+            us = [e.time_range.elapsed_us() for e in prof.events() if "resample_kernel(" in e.name and "table" not in e.name]
+            assert len(us) == a.reps, [e.name for e in prof.events()][:20]
+            n24 = R.out_len(len(x), sr)
+            p = R.plan(sr)
+            nbytes = 4 * (len(x) + p["m"] * p["W"] + 1920 * -(-n24 // 1920))
+            rs[f"{sr}Hz_{s}s"] = {"n": len(x), "n24": n24, "band": p["W"], "phases": p["m"], "kernel_us": med(us),
+                                  "kernel_us_spread": [min(us), max(us)], "bytes": nbytes, "GB_per_s": nbytes / med(us) / 1e3}
+    res["resampler"] = rs
+    c.close()
+
+    # (g) encode + prefill, 10 s
+    c = P.Context(md, max_slots=1, max_voices=4 + 3 * (a.reps + 1), kv_capacity=1024)
+    eng = c.engine
+    st = torch.cuda.ExternalStream(eng.stream_handle())
+    lat = {}
+    for sr in (24000, 44100, 48000):
+        x = noise(10 * sr)
+        eng.embed_audio(x, sr); eng.voice_from_audio(x, sr); eng.sync()
+        enc_ms, all_ms, wall_ms = [], [], []
+        for _ in range(a.reps):
+            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            eng.sync()
+            e0.record(st)
+            assert L.b200_voice_embed_audio_rate(eng.h, fp(x), len(x), sr, None) > 0
+            e1.record(st); e1.synchronize(); enc_ms.append(e0.elapsed_time(e1))
+            eng.sync()
+            t0 = time.perf_counter(); e0.record(st)
+            eng.voice_from_audio(x, sr)
+            e1.record(st); eng.sync(); wall_ms.append((time.perf_counter() - t0) * 1e3)
+            all_ms.append(e0.elapsed_time(e1))
+        lat[f"{sr}Hz_10s"] = {"encode_device_ms": med(enc_ms), "encode_prefill_device_ms": med(all_ms), "wall_ms_to_voice_id": med(wall_ms),
+                              "encode_ms_spread": [min(enc_ms), max(enc_ms)]}
+    res["latency_10s"] = lat
+    c.close()
+
+    # (h) cost to a running 256-slot batch
+    # (h) cost to a running 256-slot batch: no clones, a 10 s 24 kHz clone and a 10 s 44.1 kHz clone every 50 pumps, in alternating rounds
+    x24, x44 = noise(10 * 24000), noise(10 * 44100)
+    runs = {"none": (0, None), "every_50_24k": (50, lambda e: e.voice_from_audio(x24, 24000)),
+            "every_50_44k": (50, lambda e: e.voice_from_audio(x44, 44100))}
+    fps = {k: [] for k in runs}
+    for _ in range(a.rounds):
+        for k, (every, fn) in runs.items():
+            fps[k].append(batch_fps(P, md, every, a.batch_steps, fn)["frames_per_s"])
+    res["batch_cost"] = {"batch_steps": a.batch_steps, "rounds": a.rounds,
+                         **{k: {"frames_per_s_median": med(v), "frames_per_s": v} for k, v in fps.items()}}
+    return res
 
 
 if __name__ == "__main__":
