@@ -285,10 +285,26 @@ B200_API long long ptts_c_batch_pump(ptts_batch_t* b, int max_steps);
  * and every earlier sentence of the utterance is done. A sentence's audio is freed once it is done and fully popped. */
 B200_API int  ptts_c_batch_pop(ptts_batch_t* b, int utt, float* pcm, int max_frames);
 /* Drops the utterance's queued sentences and frees the slots of its running ones (their frames still in flight are discarded); its audio
- * not popped yet is freed and its frame count stops growing. A done utterance is left as it is. */
+ * not popped yet is freed and its frame count stops growing. A done utterance is left as it is. An open utterance is also closed. */
 B200_API int  ptts_c_batch_cancel(ptts_batch_t* b, int utt);
-/* 0 queued, 1 running, 2 done, 3 cancelled; *ready_frames (optional) = frames ptts_c_batch_pop would return now. */
+/* 0 queued, 1 running, 2 done, 3 cancelled, 4 open and waiting for text (ptts_c_batch_open: none of its sentences queued or running; an open
+ * utterance is never reported done); *ready_frames (optional) = frames ptts_c_batch_pop would return now. */
 B200_API int  ptts_c_batch_status(ptts_batch_t* b, int utt, int* ready_frames);
+/* Streamed text, the batched counterpart of ptts_stream_send / ptts_stream_flush: an LLM can feed its reply as it is written.
+ * ptts_c_batch_open returns an utterance id that accepts text; the voice is resolved as ptts_c_batch_add resolves it (name, voice file or
+ * .wav) and sampling may be NULL (defaults). ptts_c_batch_send feeds a chunk of any size to the utterance's sentence splitter; every
+ * sentence it completes (once the first character after its terminator arrives, as in ptts_stream_send) becomes a sentence of the
+ * utterance, queued at the next pump like any addition; returns the number of sentences added (an empty chunk adds nothing, it does not
+ * flush). ptts_c_batch_close ends the text: the splitter's flush applies the final-period rule and emits the tail; returns the sentences
+ * added. From then on the utterance behaves like one made by ptts_c_batch_add. Each sentence's RNG stream id is the job index + 1 when it
+ * is split off, so with no other addition between the first send and the close the audio is bitwise that of ptts_c_batch_add of the same
+ * text. send / close on an utterance that is not open (never opened, closed, cancelled) return B200_EINVAL. */
+B200_API int  ptts_c_batch_open(ptts_batch_t* b, const char* voice, float temp, const b200_sampling* sampling);
+B200_API int  ptts_c_batch_send(ptts_batch_t* b, int utt, const char* chunk);
+B200_API int  ptts_c_batch_close(ptts_batch_t* b, int utt);
+/* ptts_c_batch_open with an engine voice id (B200_EINVAL for an unknown voice). On a batch over caller-supplied ops it needs a tokenizer
+ * from ptts_c_batch_set_text. */
+B200_API int  ptts_c_batch_open_id(ptts_batch_t* b, int voice_id, float temp, const b200_sampling* sampling);
 /* The same scheduler over caller-supplied engine calls (CPU tests drive it with a mock engine). */
 typedef int (*ptts_batch_begin_fn)(void* user, int n, const int32_t* slots, const int32_t* voices, const int32_t* tokens, const int32_t* tok_off,
                                    const int32_t* max_gen_len, const int32_t* frames_after_eos, const float* temp, const uint32_t* rng_stream);
@@ -316,6 +332,9 @@ B200_API void ptts_c_text_send(ptts_text_t* t, const char* chunk);
 B200_API void ptts_c_text_flush(ptts_text_t* t);
 B200_API void ptts_c_text_reset(ptts_text_t* t);
 B200_API int  ptts_c_text_pop(ptts_text_t* t, char* buf, int buflen);
+/* Gives a batch without a context (ptts_c_batch_create_with_ops*) the tokenizer of t for ptts_c_batch_open_id / send / close; t is borrowed
+ * and must outlive the batch. B200_EINVAL on a batch over a context, which uses the context's tokenizer. */
+B200_API int  ptts_c_batch_set_text(ptts_batch_t* b, const ptts_text_t* text);
 
 #ifdef __cplusplus
 }

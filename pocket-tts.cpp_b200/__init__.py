@@ -150,6 +150,11 @@ def lib():
         "ptts_c_batch_add_tokens_sampling": (ci, [vp, ci, ip, ci, ci, ci, cf, ctypes.c_uint32, _SAMPP]),
         "ptts_c_batch_append_tokens_sampling": (ci, [vp, ci, ci, ip, ci, ci, ci, cf, ctypes.c_uint32, _SAMPP]),
         "ptts_c_batch_create_with_ops_sampling": (vp, [vp, BATCH_BEGIN_SAMPLING_FN, BATCH_SUBMIT_FN, BATCH_COLLECT_FN, BATCH_END_FN, ci, ci]),
+        "ptts_c_batch_open": (ci, [vp, cp, cf, _SAMPP]),
+        "ptts_c_batch_open_id": (ci, [vp, ci, cf, _SAMPP]),
+        "ptts_c_batch_send": (ci, [vp, ci, cp]),
+        "ptts_c_batch_close": (ci, [vp, ci]),
+        "ptts_c_batch_set_text": (ci, [vp, vp]),
         "b200_voice_len": (ci, [vp, ci]),
         "b200_kv_capacity": (ci, [vp]),
         "b200_max_slots": (ci, [vp]),
@@ -539,9 +544,12 @@ class Batch:
     refilled with queued sentences. For online serving, add() at any time, pump() a few steps, pop() each utterance's ready frames in order
     and cancel() the ones nobody waits for. With `ops` = (begin, submit, collect[, end]) Python callables the scheduler runs over a mock
     engine (CPU tests); with begin_sampling=True the begin callable also receives each sentence's b200_sampling array.
-    add() / add_tokens() take the per-sentence sampling controls lsd_steps, noise_clamp and eos_threshold (DESIGN.md 4.7)."""
+    add() / add_tokens() take the per-sentence sampling controls lsd_steps, noise_clamp and eos_threshold (DESIGN.md 4.7).
+    For text that is still being written (an LLM's reply), open() an utterance, send() its text in chunks of any size as it arrives and
+    close() it at the end: every completed sentence is queued at once (DESIGN.md 4.3, "Streamed text"). An open utterance that waits for
+    text is in state "open", never "done"."""
 
-    STATES = ("queued", "running", "done", "cancelled")
+    STATES = ("queued", "running", "done", "cancelled", "open")
 
     def __init__(self, ctx: "Context" = None, n_slots: int = 0, ops=None, frame_size: int = FRAME, begin_sampling: bool = False):
         L = lib()
@@ -584,7 +592,40 @@ class Batch:
             raise RuntimeError(f"ptts_c_batch_add_tokens failed: {u}")
         return u
 
+    def open(self, voice, temp: float = 0.7, lsd_steps: int = 1, noise_clamp: float = 0.0, eos_threshold: float = -4.0) -> int:
+        """An utterance whose text arrives through send(); `voice` is a voice name, voice file or .wav, or an engine voice id."""
+        sp = Sampling(lsd_steps, noise_clamp, eos_threshold)
+        if isinstance(voice, str):
+            u = lib().ptts_c_batch_open(self.h, voice.encode(), float(temp), ctypes.byref(sp))
+        else:
+            u = lib().ptts_c_batch_open_id(self.h, int(voice), float(temp), ctypes.byref(sp))
+        if u < 0:
+            raise RuntimeError(f"ptts_c_batch_open failed: {u}")
+        return u
+
+    def send(self, utt, text) -> int:
+        """Feeds text to an open utterance; returns the number of sentences it completed (queued at the next pump)."""
+        n = lib().ptts_c_batch_send(self.h, utt, text.encode() if isinstance(text, str) else text)
+        if n < 0:
+            raise RuntimeError(f"ptts_c_batch_send failed: {n}")
+        return n
+
+    def close(self, utt) -> int:
+        """Ends the utterance's text (the splitter's flush: the tail gets its final period); returns the number of sentences added."""
+        n = lib().ptts_c_batch_close(self.h, utt)
+        if n < 0:
+            raise RuntimeError(f"ptts_c_batch_close failed: {n}")
+        return n
+
+    def set_text(self, front: "TextFrontEnd"):
+        """Tokenizer for open() / send() on a batch over `ops`, which has no context; the batch keeps `front` alive."""
+        rc = lib().ptts_c_batch_set_text(self.h, front.h)
+        if rc != 0:
+            raise RuntimeError(f"ptts_c_batch_set_text failed: {rc}")
+        self._text = front
+
     def run(self) -> int:
+        """Runs every queued sentence to completion and returns the frames produced; it does not wait for the text of open utterances."""
         n = lib().ptts_c_batch_run(self.h)
         if n < 0:
             raise RuntimeError(f"ptts_c_batch_run failed: {n}")

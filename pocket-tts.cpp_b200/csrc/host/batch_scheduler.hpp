@@ -10,6 +10,9 @@
 // The loop is resumable (pump): utterances may be added, their audio handed out in order (pop) and cancelled between two calls, so
 // one scheduler serves requests that arrive over time. run() is pump until idle.
 //
+// An utterance may be open (its text is still arriving, ptts_c_batch_send): more jobs will be appended to it. That changes only its status
+// (kOpen instead of kDone while none of its jobs is queued or running); an open utterance waiting for text is not work, so run() returns.
+//
 // The engine is reached through a table of calls so that the scheduling logic can be driven by a mock engine in CPU tests.
 #pragma once
 #include <algorithm>
@@ -62,7 +65,7 @@ public:
         b200_sampling sampling{1, 0.f, -4.f};  // LSD steps, noise clamp, EOS threshold (b200_default_sampling)
         std::vector<float> pcm; int frames = 0; bool done = false, started = false;
     };
-    enum { kQueued = 0, kRunning = 1, kDone = 2, kCancelled = 3 };
+    enum { kQueued = 0, kRunning = 1, kDone = 2, kCancelled = 3, kOpen = 4 };
 
     BatchScheduler(const BatchOps& ops, int n_slots, int frame = 1920) : ops_(ops), n_slots_(n_slots), frame_(frame), slots_(n_slots) {}
 
@@ -72,6 +75,7 @@ public:
     bool keep_pcm = true;
 
     int add_utterance() { utts_.emplace_back(); return (int)utts_.size() - 1; }
+    void set_open(int utt, bool open) { utts_[utt].open = open; }
     int sentences(int utt) const { return (int)utts_[utt].jobs.size(); }
     // j.utt must come from add_utterance(); an utterance's audio is its jobs' frames in the order they were added
     int add_job(Job j) {
@@ -90,7 +94,8 @@ public:
         return std::max(cap, 0);
     }
 
-    // Runs every queued job to completion. Returns the number of frames produced, or a negative engine error.
+    // Runs every queued job to completion. Returns the number of frames produced, or a negative engine error. Open utterances waiting for
+    // text are not waited for: it returns once nothing is queued or running.
     long long run() { return pump(INT_MAX); }
 
     // Runs the refill -> submit -> collect loop until `max_steps` steps have been collected and at least one frame was produced, and
@@ -247,7 +252,7 @@ public:
     void cancel(int utt) {
         Utt& U = utts_[utt];
         if (U.cancelled || status(utt, nullptr) == kDone) return;
-        U.cancelled = true;
+        U.cancelled = true; U.open = false;
         for (int j : U.jobs) {
             Job& J = jobs_[j];
             std::vector<float>().swap(J.pcm);
@@ -264,12 +269,12 @@ public:
         if (U.cancelled) return kCancelled;
         bool all_done = true, any_started = false;
         for (int j : U.jobs) { all_done = all_done && jobs_[j].done; any_started = any_started || jobs_[j].started || jobs_[j].done; }
-        return all_done ? kDone : any_started ? kRunning : kQueued;
+        return all_done ? (U.open ? kOpen : kDone) : any_started ? kRunning : kQueued;
     }
 
 private:
     struct Slot { int job = -1; long long live_from = 0; };
-    struct Utt { std::vector<int> jobs; size_t next = 0; int next_frame = 0; bool cancelled = false; };   // next / next_frame: pop cursor
+    struct Utt { std::vector<int> jobs; size_t next = 0; int next_frame = 0; bool cancelled = false, open = false; };   // next / next_frame: pop cursor
     int kept(const Job& J) const { return (int)(J.pcm.size() / (size_t)frame_); }
     int busy_slots() const { int b = 0; for (const Slot& S : slots_) b += S.job >= 0; return b; }
     // jobs added since the last admission join the back of the queue, longest processing time (frame cap) first: within one admission the

@@ -403,10 +403,18 @@ int ptts_c_stream_pending(ptts_stream_t* s, int index, char* buf, int buflen) {
     return n;
 }
 
+// Host-only tokenizer + splitter object (ptts_c_text_*); a batch without a context borrows its tokenizer (ptts_c_batch_set_text).
+struct ptts_text_t { SpmUnigram tok; SentenceSplitter sp; };
+
 // ---- continuous batching (host/batch_scheduler.hpp): many utterances over the engine's slots, finished slots refilled ----
 struct ptts_batch_t {
     ptts_context_t* ctx = nullptr;                // null for a scheduler driven through caller-supplied ops (tests)
     BatchScheduler* sched = nullptr;
+    const ptts_text_t* text = nullptr;            // borrowed tokenizer of a batch without a context (ptts_c_batch_set_text)
+    // utterances whose text is still arriving (ptts_c_batch_open .. ptts_c_batch_close), by utterance id
+    struct OpenUtt { SentenceSplitter sp; int voice = 0; float temp = 0.7f; b200_sampling sampling{1, 0.f, -4.f}; };
+    std::map<int, OpenUtt> open;
+    const SpmUnigram* tokenizer() const { return ctx ? &ctx->tokenizer : text ? &text->tok : nullptr; }
 };
 static int batch_begin_engine(void* u, int n, const int32_t* sl, const int32_t* vo, const int32_t* toks, const int32_t* off, const int32_t* mg,
                               const int32_t* fae, const float* tp, const uint32_t* rs, const b200_sampling* sa) {
@@ -456,8 +464,37 @@ int ptts_c_batch_configure(ptts_batch_t* b, int refill_min, int refill_every, in
     if (keep_pcm >= 0) b->sched->keep_pcm = keep_pcm != 0;
     return B200_OK;
 }
+// The scheduler's copy of the engine's KV-capacity clamp for voice `vid` (BatchScheduler::effective_cap). B200_EINVAL for an unknown voice.
+static int batch_use_voice(ptts_batch_t* b, int vid) {
+    if (!b->ctx) return B200_OK;
+    const int vl = b200_voice_len(b->ctx->engine, vid);
+    if (vl < 0) return B200_EINVAL;
+    auto& rv = b->sched->room_of_voice;
+    if ((int)rv.size() <= vid) rv.resize(vid + 1, 1 << 30);
+    rv[vid] = b200_kv_capacity(b->ctx->engine) - vl;
+    return B200_OK;
+}
+// One sentence of the splitter -> the next job of utterance `utt`, with the reference's cap and frames_after_eos
+// (src/pocket_tts.cpp:429-430,504-506). The RNG stream id is the job index + 1 at this moment (BatchScheduler::add_job).
+static void batch_add_sentence(ptts_batch_t* b, int utt, int vid, const std::string& sent, float temp, const b200_sampling* sampling) {
+    BatchScheduler::Job j; j.utt = utt; j.index = b->sched->sentences(utt); j.voice = vid; j.temp = temp;
+    if (sampling) j.sampling = *sampling;
+    const int words = count_words_impl(sent);
+    j.fae = (words <= 4 ? 3 : 1) + 2; j.max_gen = (int)((words + 2.0f) * 12.5f);
+    std::vector<int> ids = b->tokenizer()->encode(sent);
+    j.ids.assign(ids.begin(), ids.end());
+    b->sched->add_job(std::move(j));
+}
+// Every sentence the splitter has completed becomes a job of the utterance, in order; returns their number.
+static int batch_take_sentences(ptts_batch_t* b, int utt, ptts_batch_t::OpenUtt& o) {
+    const int n = (int)o.sp.sentences.size();
+    for (const std::string& sent : o.sp.sentences) batch_add_sentence(b, utt, o.voice, sent, o.temp, &o.sampling);
+    o.sp.sentences.clear();
+    return n;
+}
+
 // One utterance = text in the reference's streaming sense: split into sentences (str_processor, conditioners/text.h:181-251), each
-// sentence is one job with the reference's cap and frames_after_eos (src/pocket_tts.cpp:429-430,504-506).
+// sentence is one job.
 int ptts_c_batch_add(ptts_batch_t* b, const char* voice, const char* text, float temp) {
     return ptts_c_batch_add_sampling(b, voice, text, temp, nullptr);
 }
@@ -465,35 +502,58 @@ int ptts_c_batch_add_sampling(ptts_batch_t* b, const char* voice, const char* te
     if (!b || !b->ctx || !voice || !text) return B200_EINVAL;
     if (sampling && b200_sampling_check(sampling) != B200_OK) return B200_EINVAL;
     const int vid = resolve_voice(b->ctx, voice);
-    auto& rv = b->sched->room_of_voice;
-    if ((int)rv.size() <= vid) rv.resize(vid + 1, 1 << 30);
-    rv[vid] = b200_kv_capacity(b->ctx->engine) - b200_voice_len(b->ctx->engine, vid);
+    batch_use_voice(b, vid);
     SentenceSplitter sp; sp.reset(); sp.ingest(text); sp.flush();
     const int utt = b->sched->add_utterance();
-    int idx = 0;
-    for (const std::string& sent : sp.sentences) {
-        BatchScheduler::Job j; j.utt = utt; j.index = idx++; j.voice = vid; j.temp = temp;
-        if (sampling) j.sampling = *sampling;
-        const int words = count_words_impl(sent);
-        j.fae = (words <= 4 ? 3 : 1) + 2; j.max_gen = (int)((words + 2.0f) * 12.5f);
-        std::vector<int> ids = b->ctx->tokenizer.encode(sent);
-        j.ids.assign(ids.begin(), ids.end());
-        b->sched->add_job(std::move(j));
-    }
+    for (const std::string& sent : sp.sentences) batch_add_sentence(b, utt, vid, sent, temp, sampling);
     return utt;
+}
+
+// Streamed text: the batched counterpart of ptts_stream_send / ptts_stream_flush. The utterance owns a splitter until close or cancel.
+int ptts_c_batch_open_id(ptts_batch_t* b, int voice_id, float temp, const b200_sampling* sampling) {
+    if (!b || !b->tokenizer() || voice_id < 0) return B200_EINVAL;
+    if (sampling && b200_sampling_check(sampling) != B200_OK) return B200_EINVAL;
+    if (batch_use_voice(b, voice_id) != B200_OK) return B200_EINVAL;
+    const int utt = b->sched->add_utterance();
+    ptts_batch_t::OpenUtt& o = b->open[utt];
+    o.sp.reset(); o.voice = voice_id; o.temp = temp;
+    if (sampling) o.sampling = *sampling;
+    b->sched->set_open(utt, true);
+    return utt;
+}
+int ptts_c_batch_open(ptts_batch_t* b, const char* voice, float temp, const b200_sampling* sampling) {
+    if (!b || !b->ctx || !voice) return B200_EINVAL;
+    if (sampling && b200_sampling_check(sampling) != B200_OK) return B200_EINVAL;
+    return ptts_c_batch_open_id(b, resolve_voice(b->ctx, voice), temp, sampling);
+}
+int ptts_c_batch_send(ptts_batch_t* b, int utt, const char* chunk) {
+    if (!b || !chunk) return B200_EINVAL;
+    auto it = b->open.find(utt);
+    if (it == b->open.end()) return B200_EINVAL;
+    it->second.sp.ingest(chunk);
+    return batch_take_sentences(b, utt, it->second);
+}
+int ptts_c_batch_close(ptts_batch_t* b, int utt) {
+    if (!b) return B200_EINVAL;
+    auto it = b->open.find(utt);
+    if (it == b->open.end()) return B200_EINVAL;
+    it->second.sp.flush();
+    const int n = batch_take_sentences(b, utt, it->second);
+    b->open.erase(it);
+    b->sched->set_open(utt, false);
+    return n;
+}
+int ptts_c_batch_set_text(ptts_batch_t* b, const ptts_text_t* text) {
+    if (!b || b->ctx) return B200_EINVAL;           // a batch over a context tokenizes with the context's tokenizer
+    b->text = text;
+    return B200_OK;
 }
 // One sentence given as token ids, appended to utterance `utt`.
 static int batch_add_token_job(ptts_batch_t* b, int utt, int voice_id, const int32_t* ids, int n_ids, int max_gen_len, int frames_after_eos, float temp,
                                uint32_t rng_stream, const b200_sampling* sampling) {
     if (n_ids < 0 || (n_ids > 0 && !ids)) return B200_EINVAL;
     if (sampling && b200_sampling_check(sampling) != B200_OK) return B200_EINVAL;
-    if (b->ctx) {
-        auto& rv = b->sched->room_of_voice;
-        const int vl = b200_voice_len(b->ctx->engine, voice_id);
-        if (vl < 0) return B200_EINVAL;
-        if ((int)rv.size() <= voice_id) rv.resize(voice_id + 1, 1 << 30);
-        rv[voice_id] = b200_kv_capacity(b->ctx->engine) - vl;
-    }
+    if (batch_use_voice(b, voice_id) != B200_OK) return B200_EINVAL;
     if (utt < 0) utt = b->sched->add_utterance();
     BatchScheduler::Job j; j.utt = utt; j.index = b->sched->sentences(utt); j.voice = voice_id; j.temp = temp; j.max_gen = max_gen_len; j.fae = frames_after_eos;
     j.rng_stream = rng_stream; j.ids.assign(ids, ids + n_ids);
@@ -536,6 +596,7 @@ int ptts_c_batch_pop(ptts_batch_t* b, int utt, float* pcm, int max_frames) {
 }
 int ptts_c_batch_cancel(ptts_batch_t* b, int utt) {
     if (!b || !b->sched->valid_utt(utt)) return B200_EINVAL;
+    b->open.erase(utt);                           // an open utterance is closed by its cancel: no more text
     b->sched->cancel(utt);
     return B200_OK;
 }
@@ -550,7 +611,6 @@ void ptts_c_batch_stats(ptts_batch_t* b, ptts_batch_stats* out) {
 }
 
 // Host-only helpers (no GPU needed): tokenizer / splitter objects for CPU-side tests and FFI users.
-struct ptts_text_t { SpmUnigram tok; SentenceSplitter sp; };
 B200_API ptts_text_t* ptts_c_text_create(const char* tokenizer_model) {
     auto* t = new ptts_text_t;
     if (!t->tok.load(tokenizer_model)) { delete t; return nullptr; }
